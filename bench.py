@@ -3,7 +3,7 @@
 BASELINE.json configs.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
-                    [--workload c1|c2|c3|c4|c5] [--scaling weak|strong]
+                    [--workload c1|c2|c3|c4|c5] [--scaling weak|strong] [--dump-outputs DIR]
 
 Default = config 4, the one the metric is quoted on: 15-branch tree, T=50, K=10, G=20 000,
 sample_density, 1M cells per GPU ("weak"; every rank samples its own slab with globally numbered
@@ -23,6 +23,15 @@ index map -> library sizes -> NB draw of cells x genes counts into HBM.  Prints 
 --impl reference times the reference's CPU algorithm (the oracle port: NumPy gather + get_pr_umi +
 legacy RandomState.negative_binomial, i.e. what scipy's nbinom.rvs executes at
 prosstt/simulation.py:647-648) on all host cores, on a bounded cell sample of the same workload.
+
+--dump-outputs DIR writes what the last timed step computed (rank 0's cells), so that two builds can be
+compared output for output; the inputs depend only on the arguments (fixed seeds):
+  X.npy          float32 (k, G): counts of k cells, all of them if they fit 30 MB, else a fixed seeded sample
+  cell.npy       float64 (k,): global index of each of those cells
+  pseudotime.npy, branch.npy, scalings.npy   float64: per cell, for every cell of the step if the three fit
+                 30 MB, else for the k cells of X.npy
+(at most 60 MB in all; counts are exact in float32 up to 2^24).
+c5 keeps only the last chunk of a step resident: its files describe that chunk.
 """
 import argparse
 import json
@@ -77,7 +86,13 @@ def parse_args():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed step to DIR/<name>.npy (at most 60 MB)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours (the reference arm keeps only checksums)")
     w = dict(WORKLOADS[a.workload])
     if a.genes:
         w["G"] = a.genes
@@ -260,11 +275,35 @@ def cpu_baseline(a, sample_cells):
                       % (X.shape[0], a.w["G"], dt)}
 
 
+DUMP_HALF_BYTES = 30 * 10 ** 6         # two halves: 60 MB of arrays in all
+
+
+def dump_outputs(path, result, names, first):
+    """Write one step's (X, pseudotime, branch codes, scalings) device tensors as DIR/<name>.npy (see the module
+    docstring).  `names` maps branch codes to the branch names the caller receives; `first` is the global index
+    of the step's first cell."""
+    import torch
+    X, pt, codes, s64 = result
+    n, G = X.shape
+    k = min(n, DUMP_HALF_BYTES // (4 * G + 32))        # a row of X and the cell's four float64 values
+    cells = np.arange(n) if k == n else np.sort(np.random.RandomState(SEEDS["sampling"]).choice(n, k, replace=False))
+    sel = torch.from_numpy(cells).to(X.device)
+    per_cell = (lambda v: v) if 3 * 8 * n <= DUMP_HALF_BYTES else (lambda v: v.index_select(0, sel))
+    arrays = {"X": X.index_select(0, sel).cpu().numpy().astype(np.float32),
+              "cell": (first + cells).astype(np.float64),
+              "pseudotime": per_cell(pt).cpu().numpy().astype(np.float64),
+              "branch": np.asarray(names, dtype=np.float64)[per_cell(codes).cpu().numpy().astype(np.int64)],
+              "scalings": per_cell(s64).cpu().numpy().astype(np.float64)}
+    os.makedirs(path, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), arr)
+
+
 def run_ours(a):
     import torch
     import torch.distributed as dist
     from prosstt_b200 import _native as nat
-    from prosstt_b200.device import CountEngine
+    from prosstt_b200.device import CountEngine, tree_tables
     from prosstt_b200.session import DensitySession
     from prosstt_b200 import simulation as sim
 
@@ -303,7 +342,8 @@ def run_ours(a):
 
     # ---- the step of this workload ----------------------------------------------------------------------
     def make_stepper(total_cells, scaling):
-        """Returns (step(seed), cells sampled by this rank per step, whole-job cells per step)."""
+        """Returns (step(seed), cells sampled by this rank per step, whole-job cells per step).  step(seed) returns
+        the device tensors (X, pseudotime, branch codes, scalings) of this rank's cells (c5: of the last chunk)."""
         if scaling == "weak":
             mine, first, job = total_cells, rank * total_cells, total_cells * world
         else:
@@ -317,7 +357,8 @@ def run_ours(a):
             def step(seed):
                 for lo in range(0, mine, chunk):          # c5: chunk after chunk into one reused buffer
                     sess.set_range(first + lo, min(chunk, mine - lo))
-                    sess.step(seed)
+                    X = sess.step(seed)
+                return X, sess.pt[:sess.n], sess.codes[:sess.n], sess.s64[:sess.n]
             return step, mine, job, sess
         if w["fn"] == "whole_tree":
             P = sum(time_.values())
@@ -356,7 +397,8 @@ def run_ours(a):
         w0 = time.time()
         ev0.record()
         for i in range(steps):
-            step(seed + 100 + i)
+            last = None                           # free the previous step's outputs before the next one allocates
+            last = step(seed + 100 + i)
         ev1.record()
         barrier()
         w1 = time.time()
@@ -364,12 +406,15 @@ def run_ours(a):
         draws = [e0.elapsed_time(e1) for e0, e1 in CountEngine.timers]
         CountEngine.timers = None
         ms = max_over_ranks(ev0.elapsed_time(ev1))
-        return ms, draws, launches, (clocks.stop(w0, w1) if clocks else None)
+        return ms, draws, launches, (clocks.stop(w0, w1) if clocks else None), last
 
     step, mine, job, sess = make_stepper(w["cells"], a.scaling)
-    ms, draws, launches, clock_rec = timed(step, a.steps, a.warmup, sample_clocks=True)
+    ms, draws, launches, clock_rec, last = timed(step, a.steps, a.warmup, sample_clocks=True)
     if sess is not None:
         sess.engine.check()
+    if a.dump_outputs and rank == 0:
+        dump_outputs(a.dump_outputs, last, tree_tables(tree, dev).names, sess.first if sess is not None else 0)
+    del last
     value = float(job) * G * a.steps / (ms / 1e3)
     kernel_ms = float(np.sum(draws)) / a.steps            # all draw launches of one step (c5: one per chunk)
 
@@ -384,7 +429,7 @@ def run_ours(a):
             del sess, step
             torch.cuda.empty_cache()
             s_step, s_mine, s_job, s_sess = make_stepper(w["cells"], "strong")
-            s_ms, s_draws, s_launch, _ = timed(s_step, a.steps, a.warmup)
+            s_ms, s_draws, s_launch = timed(s_step, a.steps, a.warmup)[:3]
             s_sess.engine.check()
             d = float(np.sum(s_draws)) / a.steps
             strong = {"value": float(s_job) * G * a.steps / (s_ms / 1e3), "unit": UNIT, "cells_total": s_job,

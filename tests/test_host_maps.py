@@ -2,6 +2,8 @@
 produced by running the reference: integer maps are bit-exact.  CPU only."""
 import re
 import os
+import subprocess
+import sys
 
 import numpy as np
 import pytest
@@ -163,7 +165,12 @@ def test_library_loads_and_exports_every_declared_symbol():
     for name in declared:
         assert getattr(lib, name) is not None
     assert lib.pst_abi_version() == 2
-    assert lib.pst_launch_count() == 0
+    # loading launches nothing; asked of a fresh process, since earlier tests in this one may have launched kernels
+    code = "import sys; sys.path.insert(0, %r); from prosstt_b200 import _native as nat; " \
+           "print(nat.load().pst_launch_count())" % ROOT
+    fresh = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True)
+    assert fresh.returncode == 0, fresh.stderr
+    assert fresh.stdout.strip() == "0"
 
 
 def test_no_cpu_fallback():
