@@ -251,6 +251,28 @@ int pst_transform_counts(const int32_t *X, int64_t n, int64_t G, int64_t ldx, co
  * row's end).  Replaces the dense text dump of tree_utils.py:111-121 as the exchange format. */
 int pst_csr_fill(const int32_t *X, int64_t n, int64_t G, int64_t ldx, const int64_t *indptr,
                  int32_t *indices, int32_t *data, uint32_t *flags, void *stream);
+/* Sizes of the CSR form of X[n][ldx] (first G columns), pass 1 of the samplers' out="csr" path:
+ * row_nnz[i] = number of nonzeros of row i (written), *sat_count += number of elements >= 65535,
+ * the uint16 saturation value of pst_csr_pack (ADDED to: the caller zeroes it; may be NULL).
+ * One streaming read of X, HBM-read bound, 4 B per count. */
+int pst_csr_row_counts(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int32_t *row_nnz,
+                       uint64_t *sat_count, void *stream);
+/* Row pointer from the row sizes: indptr[0] = 0, indptr[i+1] = row_nnz[0] + ... + row_nnz[i]
+ * (n+1 int64 entries).  One CTA; n is one shard's cells. */
+int pst_csr_row_offsets(const int32_t *row_nnz, int64_t n, int64_t *indptr, void *stream);
+/* Pass 2 of out="csr": pst_csr_fill for a chunk of rows, writing narrow streams into a window.
+ * indptr holds the chunk's n+1 GLOBAL row offsets (from pst_csr_row_offsets); nonzero number p
+ * (indptr[0] <= p < indptr[n]) goes to indices[p - base] and data[p - base], columns ascending in
+ * each row.  index_bits 16 (uint16, needs G <= 65536) or 32 (int32).  data_bits 32: exact int32
+ * values; data_bits 16: uint16 min(v, 65535), and every v >= 65535 is also listed as
+ * (ovf_pos = p, ovf_value = v), appended at atomicAdd(ovf_count, 1) when that slot is < ovf_cap
+ * (ovf_count keeps counting past the cap; pst_csr_row_counts' sat_count is the exact size needed).
+ * Sets PST_FLAG_ROW in flags[0] if a row's nonzeros do not match indptr (nothing is written past
+ * a row's end). */
+int pst_csr_pack(const int32_t *X, int64_t n, int64_t G, int64_t ldx, const int64_t *indptr,
+                 int64_t base, void *indices, int32_t index_bits, void *data, int32_t data_bits,
+                 int64_t *ovf_pos, int32_t *ovf_value, int64_t ovf_cap, uint64_t *ovf_count,
+                 uint32_t *flags, void *stream);
 
 /* Narrow transfer formats for the device->host path (PCIe is the bound at 4 B per count):
  * out[i][g] = min(X[i][g], SAT) as uint8 (out_bits 8, SAT 255) or uint16 (out_bits 16, SAT 65535),

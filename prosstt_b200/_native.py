@@ -52,6 +52,9 @@ _SIGNATURES = {
     "pst_count_stats": (C.c_int, [_p, _i64, _i64, _i64, _p, _p, _p, _p, _p, _p]),
     "pst_transform_counts": (C.c_int, [_p, _i64, _i64, _i64, _p, _i32, _p, _i64, _p]),
     "pst_csr_fill": (C.c_int, [_p, _i64, _i64, _i64, _p, _p, _p, _p, _p]),
+    "pst_csr_row_counts": (C.c_int, [_p, _i64, _i64, _i64, _p, _p, _p]),
+    "pst_csr_row_offsets": (C.c_int, [_p, _i64, _p, _p]),
+    "pst_csr_pack": (C.c_int, [_p, _i64, _i64, _i64, _p, _i64, _p, _i32, _p, _i32, _p, _p, _i64, _p, _p, _p]),
     "pst_store_fill": (C.c_int, [_p, _i64, _i32, _p]),
     "pst_host_widen": (C.c_int, [_p, _i32, _p, _i32, _i64, _i32]),
     "pst_host_widen_stream": (C.c_int, [_p, _i32, _p, _i32, _i64, _i32]),

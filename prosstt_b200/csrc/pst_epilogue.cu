@@ -44,15 +44,40 @@ transform_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ld
   }
 }
 
+// one gene quad of row `src` (zeros past G)
+template <bool VEC>
+__device__ __forceinline__ int4 load_quad(const int32_t *__restrict__ src, int64_t q, int64_t Q, int64_t G) {
+  int4 v = make_int4(0, 0, 0, 0);
+  if (q < Q) {
+    if (VEC) {
+      v = __ldcs(reinterpret_cast<const int4 *>(src + q * 4));
+    } else {
+      const int64_t g = q * 4;
+      v.x = src[g];
+      if (g + 1 < G) v.y = src[g + 1];
+      if (g + 2 < G) v.z = src[g + 2];
+      if (g + 3 < G) v.w = src[g + 3];
+    }
+  }
+  return v;
+}
+
 // ---------------------------------------------------------------------------------------------
 // CSR fill: one warp per row, 128 genes per step; a lane owns a gene quad, so column order inside
-// the row is preserved by an exclusive warp prefix of the lanes' nonzero counts
+// the row is preserved by an exclusive warp prefix of the lanes' nonzero counts.
+// Nonzero number p of the matrix (indptr[0] <= p < indptr[n]) goes to indices/data[p - base]: a
+// chunk of rows fills its own window of the streams.  IDX / VAL are the stored widths; SAT: values
+// are stored as min(v, 65535) and every v >= 65535 is also listed exactly as (p, v) in the overflow
+// list (slot from atomicAdd(ovf_count), written when below ovf_cap).
 // ---------------------------------------------------------------------------------------------
-template <bool VEC>
+constexpr int32_t kCsrSat = 65535;
+
+template <typename IDX, typename VAL, bool SAT, bool VEC>
 __global__ void __launch_bounds__(256)
 csr_fill_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx,
-                const int64_t *__restrict__ indptr, int32_t *__restrict__ indices,
-                int32_t *__restrict__ data, uint32_t *__restrict__ flags) {
+                const int64_t *__restrict__ indptr, int64_t base, IDX *__restrict__ indices,
+                VAL *__restrict__ data, int64_t *__restrict__ ovf_pos, int32_t *__restrict__ ovf_value,
+                int64_t ovf_cap, unsigned long long *__restrict__ ovf_count, uint32_t *__restrict__ flags) {
   const int lane = threadIdx.x & 31;
   const unsigned lt = (1u << lane) - 1u;
   const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
@@ -65,18 +90,7 @@ csr_fill_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx
 #pragma unroll 4
     for (int64_t q0 = 0; q0 < Q; q0 += 32) {
       const int64_t q = q0 + lane;
-      int4 v = make_int4(0, 0, 0, 0);
-      if (q < Q) {
-        if (VEC) {
-          v = __ldcs(reinterpret_cast<const int4 *>(src + q * 4));
-        } else {
-          const int64_t g = q * 4;
-          v.x = src[g];
-          if (g + 1 < G) v.y = src[g + 1];
-          if (g + 2 < G) v.z = src[g + 2];
-          if (g + 3 < G) v.w = src[g + 3];
-        }
-      }
+      const int4 v = load_quad<VEC>(src, q, Q, G);
       // exclusive prefix of the lanes' nonzero counts (0..4) from three ballots of the count's bits
       const int c = (v.x != 0) + (v.y != 0) + (v.z != 0) + (v.w != 0);
       const unsigned b0 = __ballot_sync(0xffffffffu, c & 1), b1 = __ballot_sync(0xffffffffu, c & 2),
@@ -86,14 +100,114 @@ csr_fill_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx
       int64_t w = pos + excl;
       if (pos + total <= end) {                   // indptr is consistent with the matrix
         const int32_t g = (int32_t)(q * 4);
-        if (v.x != 0) { indices[w] = g;     data[w] = v.x; ++w; }
-        if (v.y != 0) { indices[w] = g + 1; data[w] = v.y; ++w; }
-        if (v.z != 0) { indices[w] = g + 2; data[w] = v.z; ++w; }
-        if (v.w != 0) { indices[w] = g + 3; data[w] = v.w; ++w; }
+        const int32_t vv[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+          if (vv[j] != 0) {
+            indices[w - base] = (IDX)(g + j);
+            if (SAT && vv[j] >= kCsrSat) {        // rare: one atomic per listed count
+              const unsigned long long slot = atomicAdd(ovf_count, 1ull);
+              if ((int64_t)slot < ovf_cap) { ovf_pos[slot] = w; ovf_value[slot] = vv[j]; }
+              data[w - base] = (VAL)kCsrSat;
+            } else {
+              data[w - base] = (VAL)vv[j];
+            }
+            ++w;
+          }
+        }
       }
       pos += total;
     }
     if (lane == 0 && pos != end) atomicOr(flags, (uint32_t)PST_FLAG_ROW);   // indptr does not match X
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// Row sizes of the CSR form: row_nnz[i] = nonzeros of row i; *sat_count += elements >= 65535.  One
+// warp per row, four 128-bit streaming loads in flight per lane; a lane keeps its own counts and the
+// warp sums them once per row (one REDUX instead of ballots per step: only the total is needed here),
+// the saturated elements once per warp with a single atomic.
+// ---------------------------------------------------------------------------------------------
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+csr_row_count_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx,
+                     int32_t *__restrict__ row_nnz, unsigned long long *__restrict__ sat_count) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  const int64_t Q = (G + 3) / 4;
+  unsigned sat = 0;
+  for (int64_t row = warp0; row < n; row += n_warps) {
+    const int32_t *src = X + row * ldx;
+    unsigned c = 0;
+    for (int64_t q0 = 0; q0 < Q; q0 += 128) {
+      int4 v[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) v[j] = load_quad<VEC>(src, q0 + 32 * j + lane, Q, G);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        c += (v[j].x != 0) + (v[j].y != 0) + (v[j].z != 0) + (v[j].w != 0);
+        sat += (v[j].x >= kCsrSat) + (v[j].y >= kCsrSat) + (v[j].z >= kCsrSat) + (v[j].w >= kCsrSat);
+      }
+    }
+    c = __reduce_add_sync(0xffffffffu, c);
+    if (lane == 0) row_nnz[row] = (int32_t)c;
+  }
+  sat = __reduce_add_sync(0xffffffffu, sat);
+  if (lane == 0 && sat != 0 && sat_count != nullptr) atomicAdd(sat_count, (unsigned long long)sat);
+}
+
+// ---------------------------------------------------------------------------------------------
+// indptr[0] = 0, indptr[i + 1] = row_nnz[0] + ... + row_nnz[i]: one CTA walks the rows in tiles of
+// 1024 x 8; each thread sums its 8 rows, the block scans the thread sums (warp shuffles + one word per
+// warp in shared memory) and carries the tile total into the next tile.  n is one shard's cells (a
+// few million at most: a few hundred microseconds), so no grid-wide scan is needed.
+// ---------------------------------------------------------------------------------------------
+constexpr int kScanThreads = 1024, kScanItems = 8;
+
+__global__ void __launch_bounds__(kScanThreads)
+csr_row_offsets_kernel(const int32_t *__restrict__ row_nnz, int64_t n, int64_t *__restrict__ indptr) {
+  __shared__ long long warp_sum[kScanThreads / 32];
+  __shared__ long long carry_s;
+  const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
+  long long carry = 0;
+  if (t == 0) indptr[0] = 0;
+  for (int64_t tile = 0; tile < n; tile += (int64_t)kScanThreads * kScanItems) {
+    const int64_t i0 = tile + (int64_t)t * kScanItems;
+    int32_t v[kScanItems];
+    long long s = 0;
+#pragma unroll
+    for (int j = 0; j < kScanItems; ++j) {
+      v[j] = (i0 + j < n) ? row_nnz[i0 + j] : 0;
+      s += v[j];
+    }
+    long long incl = s;                                         // inclusive scan of the thread sums
+#pragma unroll
+    for (int d = 1; d < 32; d <<= 1) {
+      const long long o = __shfl_up_sync(0xffffffffu, incl, d);
+      if (lane >= d) incl += o;
+    }
+    if (lane == 31) warp_sum[wid] = incl;
+    __syncthreads();
+    if (wid == 0) {
+      long long ws = warp_sum[lane];
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const long long o = __shfl_up_sync(0xffffffffu, ws, d);
+        if (lane >= d) ws += o;
+      }
+      warp_sum[lane] = ws;                                      // inclusive over warps
+      if (lane == 31) carry_s = carry + ws;
+    }
+    __syncthreads();
+    long long run = carry + (wid ? warp_sum[wid - 1] : 0) + incl - s;
+#pragma unroll
+    for (int j = 0; j < kScanItems; ++j) {
+      run += v[j];
+      if (i0 + j < n) indptr[i0 + j + 1] = run;
+    }
+    carry = carry_s;
+    __syncthreads();                                            // warp_sum / carry_s are rewritten next tile
   }
 }
 
@@ -207,8 +321,71 @@ extern "C" int pst_csr_fill(const int32_t *X, int64_t n, int64_t G, int64_t ldx,
   PST_REQUIRE(X && indptr && indices && data && flags, fn, "null pointer");
   const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
   const unsigned grid = stream_grid(n * 32);
-  if (vec) csr_fill_kernel<true><<<grid, 256, 0, (cudaStream_t)stream>>>(X, n, G, ldx, indptr, indices, data, flags);
-  else csr_fill_kernel<false><<<grid, 256, 0, (cudaStream_t)stream>>>(X, n, G, ldx, indptr, indices, data, flags);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec) csr_fill_kernel<int32_t, int32_t, false, true><<<grid, 256, 0, st>>>(
+      X, n, G, ldx, indptr, 0, indices, data, nullptr, nullptr, 0, nullptr, flags);
+  else csr_fill_kernel<int32_t, int32_t, false, false><<<grid, 256, 0, st>>>(
+      X, n, G, ldx, indptr, 0, indices, data, nullptr, nullptr, 0, nullptr, flags);
+  return check_launch(fn);
+}
+
+extern "C" int pst_csr_row_counts(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int32_t *row_nnz,
+                                  uint64_t *sat_count, void *stream) {
+  const char *fn = "pst_csr_row_counts";
+  PST_REQUIRE(n >= 0 && G >= 0 && ldx >= G, fn, "need n, G >= 0 and ldx >= G");
+  PST_REQUIRE(G < ((int64_t)1 << 31), fn, "a row's count does not fit int32");
+  if (n == 0) return 0;
+  PST_REQUIRE(X && row_nnz, fn, "null pointer");
+  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
+  const unsigned grid = stream_grid(n * 32);
+  cudaStream_t st = (cudaStream_t)stream;
+  unsigned long long *sat = (unsigned long long *)sat_count;
+  if (vec) csr_row_count_kernel<true><<<grid, 256, 0, st>>>(X, n, G, ldx, row_nnz, sat);
+  else csr_row_count_kernel<false><<<grid, 256, 0, st>>>(X, n, G, ldx, row_nnz, sat);
+  return check_launch(fn);
+}
+
+extern "C" int pst_csr_row_offsets(const int32_t *row_nnz, int64_t n, int64_t *indptr, void *stream) {
+  const char *fn = "pst_csr_row_offsets";
+  PST_REQUIRE(n >= 0, fn, "need n >= 0");
+  PST_REQUIRE(indptr && (n == 0 || row_nnz), fn, "null pointer");
+  csr_row_offsets_kernel<<<1, kScanThreads, 0, (cudaStream_t)stream>>>(row_nnz, n, indptr);
+  return check_launch(fn);
+}
+
+extern "C" int pst_csr_pack(const int32_t *X, int64_t n, int64_t G, int64_t ldx, const int64_t *indptr,
+                            int64_t base, void *indices, int32_t index_bits, void *data, int32_t data_bits,
+                            int64_t *ovf_pos, int32_t *ovf_value, int64_t ovf_cap, uint64_t *ovf_count,
+                            uint32_t *flags, void *stream) {
+  const char *fn = "pst_csr_pack";
+  PST_REQUIRE(n >= 0 && G >= 0 && ldx >= G && base >= 0 && ovf_cap >= 0, fn,
+              "need n, G, base, ovf_cap >= 0 and ldx >= G");
+  PST_REQUIRE(index_bits == 16 || index_bits == 32, fn, "index_bits must be 16 or 32");
+  PST_REQUIRE(data_bits == 16 || data_bits == 32, fn, "data_bits must be 16 or 32");
+  PST_REQUIRE(index_bits == 32 || G <= 65536, fn, "16-bit column indices need G <= 65536");
+  PST_REQUIRE(G < ((int64_t)1 << 31), fn, "column index does not fit int32");
+  if (n == 0 || G == 0) return 0;
+  PST_REQUIRE(X && indptr && indices && data && flags, fn, "null pointer");
+  PST_REQUIRE(data_bits == 32 || (ovf_count && (ovf_cap == 0 || (ovf_pos && ovf_value))), fn,
+              "16-bit values need the overflow list");
+  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
+  const unsigned grid = stream_grid(n * 32);
+  cudaStream_t st = (cudaStream_t)stream;
+  unsigned long long *cnt = (unsigned long long *)ovf_count;
+#define PST_LAUNCH_PACK(I, V, S)                                                                             \
+  do {                                                                                                       \
+    if (vec) csr_fill_kernel<I, V, S, true><<<grid, 256, 0, st>>>(X, n, G, ldx, indptr, base, (I *)indices,  \
+                                                                  (V *)data, ovf_pos, ovf_value, ovf_cap,    \
+                                                                  cnt, flags);                               \
+    else csr_fill_kernel<I, V, S, false><<<grid, 256, 0, st>>>(X, n, G, ldx, indptr, base, (I *)indices,     \
+                                                               (V *)data, ovf_pos, ovf_value, ovf_cap, cnt,  \
+                                                               flags);                                       \
+  } while (0)
+  if (index_bits == 16 && data_bits == 16) PST_LAUNCH_PACK(uint16_t, uint16_t, true);
+  else if (index_bits == 32 && data_bits == 16) PST_LAUNCH_PACK(int32_t, uint16_t, true);
+  else if (index_bits == 16) PST_LAUNCH_PACK(uint16_t, int32_t, false);
+  else PST_LAUNCH_PACK(int32_t, int32_t, false);
+#undef PST_LAUNCH_PACK
   return check_launch(fn);
 }
 

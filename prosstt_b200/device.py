@@ -10,6 +10,7 @@ import numpy as np
 import torch
 
 from prosstt_b200 import _native as nat
+from prosstt_b200 import hostpool
 
 
 def tree_tables(tree, dev):
@@ -264,6 +265,7 @@ class CountEngine(object):
     """draw_counts on one GPU: replicated small state + a cell range to sample."""
 
     timers = None     # set to a list to collect (start, end) CUDA events around every draw (bench.py)
+    csr_timers = None  # set to a list to collect (start, end of pass 1, end of pass 2) events of draw_to_csr
 
     def __init__(self, tree, tables, alpha, beta, dev, sampler="gamma_poisson"):
         self.dev = dev
@@ -452,6 +454,139 @@ class CountEngine(object):
                                 "list holds %d: use a wider transport or a larger overflow_cap"
                                 % (count, transport, overflow_cap))
         return ovf_index[:count].cpu(), ovf_value[:count].cpu()
+
+    def draw_to_csr(self, rows, scaling32, seed, cell0, data_dtype=np.int64, chunk_cells=None, threads=0):
+        """Sample the cells as CSR arrays on the host: (indptr, indices, data) NumPy arrays, columns ascending
+        in every row, no explicit zeros; the same counts as draw().  The dense matrix exists only one chunk at
+        a time in HBM.
+
+        Pass 1 draws each chunk and counts its nonzeros per row (pst_csr_row_counts) and the counts >= 65535;
+        one scan (pst_csr_row_offsets) gives the row pointer, which is the only thing read back.  So nnz is
+        known before any result memory exists: indices and data are allocated once at their final size, with
+        int32 indptr/indices when nnz < 2^31 and int64 otherwise (scipy wants the two of one dtype).
+        Pass 2 draws each chunk again (a pure function of (seed, cell, gene)), packs it into a uint16 (G <=
+        65536) or int32 column stream and a uint16 value stream (pst_csr_pack), copies both into pinned
+        staging and host threads widen them into indices[p0:p1] / data[p0:p1] while the next chunk is
+        sampled; the values that saturated uint16 are written from the exact overflow list at the end.
+        data_dtype: np.int64 or np.int32."""
+        import concurrent.futures
+        data_dtype = np.dtype(data_dtype)
+        if data_dtype not in (np.dtype(np.int32), np.dtype(np.int64)):
+            raise ValueError("CSR data must be int32 or int64, not %s" % data_dtype)
+        n, G, dev = int(rows.numel()), self.G, self.dev
+        if not threads:
+            threads = _host_threads()
+        if n == 0 or G == 0:
+            return np.zeros(n + 1, np.int32), np.zeros(0, np.int32), np.zeros(0, data_dtype)
+        ibits = 16 if G <= 65536 else 32                 # width of the column stream
+        ramp_up = chunk_cells is None
+        if chunk_cells is None:
+            chunk_cells = _STAGE_BYTES // max(1, (ibits // 8 + 2) * G)
+        chunk_cells = max(1, min(n, int(chunk_cells)))
+        bounds, lo = [], 0
+        # the first chunks are smaller so that the copy and the host threads start almost immediately
+        ramp = [max(1, chunk_cells // 8), max(1, chunk_cells // 4), max(1, chunk_cells // 2)] if ramp_up else []
+        while lo < n:
+            size = ramp.pop(0) if ramp else chunk_cells
+            bounds.append((lo, min(n, lo + size)))
+            lo = bounds[-1][1]
+        st = nat.stream_ptr(dev)
+        main = torch.cuda.current_stream(dev)
+        events = CountEngine.csr_timers
+        if events is not None:
+            ev = [torch.cuda.Event(enable_timing=True) for _ in range(3)]
+            ev[0].record(main)
+        # ---- pass 1: row sizes and the number of saturated values
+        work = torch.empty((chunk_cells, G), dtype=torch.int32, device=dev)
+        row_nnz = torch.empty(n, dtype=torch.int32, device=dev)
+        sat = torch.zeros(1, dtype=torch.int64, device=dev)
+        for lo, hi in bounds:
+            self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[:hi - lo])
+            nat.call("pst_csr_row_counts", work.data_ptr(), hi - lo, G, G, row_nnz[lo:hi], sat, st)
+        indptr_d = torch.empty(n + 1, dtype=torch.int64, device=dev)
+        nat.call("pst_csr_row_offsets", row_nnz, n, indptr_d, st)
+        if events is not None:
+            ev[1].record(main)
+        indptr64 = indptr_d.cpu().numpy()
+        n_sat = int(sat.item())
+        self.check()                                     # domain / range errors before any result memory
+        # ---- allocate once, at the final size
+        nnz = int(indptr64[-1])
+        idx_dtype = np.dtype(np.int32) if nnz < (1 << 31) else np.dtype(np.int64)
+        indptr = indptr64.astype(np.int32) if idx_dtype == np.int32 else indptr64
+        indices, fresh_i = hostpool.result_array((nnz,), idx_dtype)
+        data, fresh_d = hostpool.result_array((nnz,), data_dtype)
+        lib = nat.load()
+        widen_i = lib.pst_host_widen if fresh_i else lib.pst_host_widen_stream
+        widen_d = lib.pst_host_widen if fresh_d else lib.pst_host_widen_stream
+        ibytes, ibits_out, dbits_out = ibits // 8, 8 * idx_dtype.itemsize, 8 * data_dtype.itemsize
+
+        def value_offset(m):                            # the value stream starts on a 64-byte boundary
+            return (m * ibytes + 63) // 64 * 64
+
+        stage_bytes = max(value_offset(int(indptr64[hi] - indptr64[lo])) + 2 * int(indptr64[hi] - indptr64[lo])
+                          for lo, hi in bounds)
+        stage_dev = [torch.empty(max(1, stage_bytes), dtype=torch.uint8, device=dev) for _ in range(2)]
+        stage_host = _pinned_staging(dev, stage_bytes)
+        ovf_pos = torch.empty(max(1, n_sat), dtype=torch.int64, device=dev)
+        ovf_value = torch.empty(max(1, n_sat), dtype=torch.int32, device=dev)
+        ovf_count = torch.zeros(1, dtype=torch.int64, device=dev)
+        pack_flags = torch.zeros(1, dtype=torch.int32, device=dev)
+        copy_stream = torch.cuda.Stream(device=dev)
+        pool = concurrent.futures.ThreadPoolExecutor(max_workers=1)
+        pending = [None, None]                          # host threads still reading stage_host[k]
+
+        def landed(k, p0, m, event):
+            event.synchronize()                         # both streams of the chunk are in stage_host[k]
+            src = stage_host[k].data_ptr()
+            rc = widen_i(src, ibits, indices.ctypes.data + p0 * idx_dtype.itemsize, ibits_out, m, int(threads))
+            rc |= widen_d(src + value_offset(m), 16, data.ctypes.data + p0 * data_dtype.itemsize, dbits_out, m,
+                          int(threads))
+            if rc != 0:
+                raise nat.NativeError("pst_host_widen failed")
+
+        # ---- pass 2: redraw, pack, stream
+        try:
+            for i, (lo, hi) in enumerate(bounds):
+                p0, p1 = int(indptr64[lo]), int(indptr64[hi])
+                m = p1 - p0
+                if m == 0:
+                    continue                            # nothing to pack: the redraw has no nonzero either
+                k = i & 1
+                if pending[k] is not None:
+                    pending[k].result()                 # stage_host[k] (and so stage_dev[k]) is free again
+                self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[:hi - lo])
+                buf = stage_dev[k]
+                nat.call("pst_csr_pack", work.data_ptr(), hi - lo, G, G, indptr_d[lo:hi + 1], p0, buf.data_ptr(),
+                         ibits, buf.data_ptr() + value_offset(m), 16, ovf_pos, ovf_value, n_sat, ovf_count,
+                         pack_flags, st)
+                used = value_offset(m) + 2 * m
+                done = torch.cuda.Event()
+                done.record(main)
+                with torch.cuda.stream(copy_stream):
+                    copy_stream.wait_event(done)
+                    stage_host[k][:used].copy_(buf[:used], non_blocking=True)
+                    copied = torch.cuda.Event()
+                    copied.record(copy_stream)
+                pending[k] = pool.submit(landed, k, p0, m, copied)
+            if events is not None:
+                ev[2].record(main)
+                events.append(tuple(ev))
+            for f in pending:
+                if f is not None:
+                    f.result()
+        finally:
+            pool.shutdown(wait=True)
+        self.check()
+        if int(pack_flags.item()) != 0:
+            raise RuntimeError("the redrawn counts do not match the row sizes of the first pass")
+        listed = int(ovf_count.item())
+        if listed != n_sat:
+            raise RuntimeError("%d counts >= 65535 in the second pass, %d in the first" % (listed, n_sat))
+        if n_sat:
+            pos, value = ovf_pos[:n_sat].cpu(), ovf_value[:n_sat].cpu()
+            lib.pst_host_apply_overflow(data.ctypes.data, dbits_out, 0, nnz, pos.data_ptr(), value.data_ptr(), n_sat)
+        return indptr, indices, data
 
     def _draw_to_host_staged(self, rows, scaling32, seed, cell0, host_out, hdt, chunk_cells, overflow_cap,
                              transport, threads, fresh=False):

@@ -11,8 +11,12 @@ Extra keyword-only arguments (never required):
   shard    (rank, world): sample only this rank's contiguous slice of the cells; every
            random quantity is keyed by the GLOBAL cell index, so the union over ranks is
            bit-identical to the unsharded call
-  dtype    dtype of the returned count matrix (reference: int64; int32 avoids a host pass)
-  out      "numpy" (reference behaviour) or "torch" (leave everything on the GPU)
+  dtype    dtype of the returned count matrix (reference: int64; int32 avoids a host pass); with
+           out="csr" the dtype of its data, int64 or int32
+  out      "numpy" (reference behaviour), "torch" (leave everything on the GPU) or "csr": X is a
+           scipy.sparse.csr_matrix (canonical: columns ascending, no explicit zeros; int32 indptr/indices,
+           int64 when it has 2^31 nonzeros or more) with the same counts as "numpy".  The GPU compacts
+           each chunk and only the nonzeros cross PCIe (CountEngine.draw_to_csr); not with host_out
   sampler  "hybrid" (default): direct inversion of the NB cdf for mean <= 32, sd <= 20, gamma scale <= 32 and
            shape <= 48 - in fp32 below the 1 - 2^-14 quantile of its uniform, with a 64-bit uniform against an
            fp64-accumulated cdf above it, so body and far tail match the exact pmf (checked at 1e9 draws per
@@ -410,15 +414,45 @@ def _shard_range(n, shard):
     return shard_range(n, rank, world)
 
 
+def _check_csr_request(out, dtype, host_out=None):
+    """out="csr" takes int64 (default) or int32 data and no preallocated host_out."""
+    if out != "csr":
+        return
+    if host_out is not None:
+        raise ValueError("host_out cannot be combined with out='csr'")
+    if np.dtype(dtype) not in (np.dtype(np.int64), np.dtype(np.int32)):
+        raise ValueError("out='csr' stores int64 or int32 counts, not %s" % np.dtype(dtype))
+
+
+def _csr_matrix(indptr, indices, data, shape):
+    """scipy.sparse.csr_matrix over the given arrays without a copy or a scan: the constructor would check
+    every column index and copy int64 index arrays whose contents fit int32.  The arrays are already in
+    canonical form (columns ascending in every row, no explicit zeros, no duplicates)."""
+    import scipy.sparse as sp
+    m = sp.csr_matrix(shape, dtype=data.dtype)
+    m.indptr, m.indices, m.data = indptr, indices, data
+    m.has_sorted_indices = True
+    m.has_canonical_format = True
+    return m
+
+
 def _sample_counts(engine, rows, s32, seed, first, dtype, out):
-    """The count matrix of the cells described by rows/s32: a device int32 tensor (out="torch") or a
-    fresh host array of `dtype` (reference: int64, simulation.py:651).  The host form never holds the
-    whole matrix on the GPU: chunks are sampled, copied as int32 into pinned staging and expanded into
-    the result by host threads while the next chunk is sampled (CountEngine.draw_to_host)."""
+    """The count matrix of the cells described by rows/s32: a device int32 tensor (out="torch"), a
+    scipy.sparse.csr_matrix with `dtype` data (out="csr", CountEngine.draw_to_csr: only the nonzeros cross
+    PCIe) or a fresh host array of `dtype` (reference: int64, simulation.py:651).  The host forms never hold
+    the whole matrix on the GPU: chunks are sampled, copied into pinned staging and expanded into the result
+    by host threads while the next chunk is sampled (CountEngine.draw_to_host)."""
     if out == "torch":
         X = engine.draw(rows, s32, seed, first)
         engine.check()
         return X
+    if out == "csr":
+        _check_csr_request(out, dtype)
+        n = int(rows.numel())
+        indptr, indices, data = engine.draw_to_csr(rows, s32, seed, first, data_dtype=dtype)
+        torch.cuda.current_stream(engine.dev).synchronize()
+        engine.check()
+        return _csr_matrix(indptr, indices, data, (n, engine.G))
     want = np.dtype(dtype)
     n = int(rows.numel())
     direct = want in (np.dtype(np.int32), np.dtype(np.int64))
@@ -442,6 +476,7 @@ def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mea
     and a fifth entry of host_out, a dict, receives the exact values of the saturated elements as
     "index" (flat, into X) and "value" arrays (formats.widen rebuilds the int32 matrix); without
     the dict a saturated element raises OverflowError instead of passing silently."""
+    _check_csr_request(out, dtype, host_out)
     n = int(rows.numel())
     s64, s32 = sut.calc_scalings(n, scale, scale_mean, scale_v, seed=nat.derive_seed(seed, 1),
                                  first=first, device=dev, return_device=True)
@@ -645,6 +680,7 @@ def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, de
     (simulation.py:602-651): X[n,g] ~ NB(mean = means[branch_n][t_n - start, g]*scaling_n,
     variance = alpha_g mean^2 + beta_g mean)."""
     dev = nat.device(device)
+    _check_csr_request(out, dtype)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
     pt = pseudotime if isinstance(pseudotime, torch.Tensor) else \
