@@ -4,6 +4,7 @@ Layout (include/prosstt_b200.h): branches in `tree.branches` order, branch b own
 rows [row_base[b], row_base[b]+T_b); P = sum T_b.  Everything here is small and
 replicated on every GPU (a few MB; the means table is P x G fp32); only cells shard.
 """
+import concurrent.futures
 import os
 
 import numpy as np
@@ -261,6 +262,76 @@ def _pinned_staging(dev, nbytes):
     return have
 
 
+def _plan_chunks(n, chunk_cells, cell_bytes, budget):
+    """The cell chunks of a chunked device->host call: (chunk, [(lo, hi), ...]) covering [0, n) in order, where
+    chunk is the largest chunk (the size of the buffers).  Owns the chunk size and the ramp-up.
+    chunk_cells=None: chunks of `budget` bytes at `cell_bytes` per cell, and the first chunks are 1/8, 1/4 and 1/2
+    of that so that the copy (and the host threads) start almost immediately.  An explicit chunk_cells (at least
+    1, at most n) has no ramp."""
+    ramp_up = chunk_cells is None
+    if ramp_up:
+        chunk_cells = budget // max(1, cell_bytes)
+    chunk = max(1, min(n, int(chunk_cells)))
+    ramp = [max(1, chunk // 8), max(1, chunk // 4), max(1, chunk // 2)] if ramp_up else []
+    bounds, lo = [], 0
+    while lo < n:
+        size = ramp.pop(0) if ramp else chunk
+        bounds.append((lo, min(n, lo + size)))
+        lo = bounds[-1][1]
+    return chunk, bounds
+
+
+_TRANSPORTS = {"i32": torch.int32, "u16": torch.uint16, "u8": torch.uint8}
+
+
+def _host_route(is_np, hdt, pinned, transport, threads):
+    """How draw_to_host moves the counts into a host matrix of dtype `hdt` (the table in its docstring):
+    returns (route, retry).  route is "direct" (the copy engine writes the matrix) or the staged transport
+    "i32" / "u16" / "u8"; retry is the route to sample again through when an automatically chosen "u8"
+    overflows its list, else None.  Raises ValueError for a combination that has no route."""
+    if hdt in (torch.uint16, torch.uint8):
+        if is_np or transport not in (None, "direct"):
+            raise ValueError("a uint16 / uint8 host matrix must be a CPU tensor and takes transport 'direct'")
+        return "direct", None
+    if transport is None:
+        # nothing asked for: the copy engine writes a pinned int32 matrix itself ("direct"), every other
+        # target is filled by host threads from int32 staging ("i32") - or, where this rank's share of
+        # the host cores expands uint8 well above the PCIe rate, from uint8 staging ("u8")
+        wide = "direct" if (not is_np and hdt == torch.int32 and pinned) else "i32"
+        if not _AUTO_STATE["narrow_overflowed"] and _shared_host_transport(threads) == "u8":
+            return "u8", wide
+        return wide, None
+    if transport == "direct":
+        if is_np or hdt != torch.int32:
+            raise ValueError("transport 'direct' needs an int32, uint16 or uint8 CPU tensor")
+        return "direct", None
+    if transport not in _TRANSPORTS:
+        raise ValueError("transport must be 'direct', 'i32', 'u16' or 'u8'")
+    return transport, None
+
+
+class _OverflowList(object):
+    """The exact list of the counts a narrow format cannot hold, on the device: int64 positions, int32 values,
+    an int64 count and the capacity.  Owns the check that the list held every such count."""
+
+    def __init__(self, capacity, dev):
+        self.capacity = int(capacity)
+        self.pos = torch.empty(max(1, self.capacity), dtype=torch.int64, device=dev)
+        self.value = torch.empty(max(1, self.capacity), dtype=torch.int32, device=dev)
+        self.count = torch.zeros(1, dtype=torch.int64, device=dev)
+        # in the order pst_narrow_counts and pst_csr_pack take them
+        self.kernel_args = (self.pos, self.value, self.capacity, self.count)
+
+    def read(self, fmt):
+        """(positions, values) device tensors of the listed counts, in the order the kernels appended them."""
+        count = int(self.count.item())
+        if count > self.capacity:
+            raise OverflowError("%d counts reach the saturation value of %s but the overflow list holds %d: "
+                                "use a wider format or a larger overflow_cap"
+                                % (count, str(fmt).replace("torch.", ""), self.capacity))
+        return self.pos[:count], self.value[:count]
+
+
 class CountEngine(object):
     """draw_counts on one GPU: replicated small state + a cell range to sample."""
 
@@ -314,23 +385,34 @@ class CountEngine(object):
         """Sample in cell chunks and stream them into `host_out`, an (n, G) CPU tensor or C-contiguous
         NumPy array: sampling of chunk i+1 overlaps the transfer (and host-side expansion) of chunk i.
 
-        host_out int32, pinned, transport None/"direct": the counts as sampled are copied straight into
-          it (4 B per count over PCIe).
-        host_out uint16 / uint8 (pinned): the narrow formats themselves (2 / 1 B per count):
-          min(count, SAT) with SAT = 65535 / 255, and every element that reads SAT is listed exactly in
-          `self.overflow` = (flat index into host_out, int32 value) NumPy arrays sorted by index
-          (formats.widen rebuilds int32).  At default depth about 2 in 10^4 counts reach 255 and none
-          reaches 65535.
-        host_out int32 or int64, pageable or pinned, transport "u8" / "u16" / "i32": the chunk crosses
-          PCIe in the transport format into pinned staging buffers (cached per device) and host threads
-          (pst_host_widen) expand it into host_out, the overflow list is applied at the end: the caller
-          receives exact int32 / int64 counts.  This is the path of the reference-shaped call, which
-          returns a fresh (pageable) int64 array.  Default transport: the wide one ("direct" for a pinned
-          int32 tensor, "i32" otherwise) or "u8", whichever is faster on this host (_shared_host_transport);
-          an automatically chosen "u8" whose overflow list does not fit (deep regimes) is sampled again
-          through the wide transport - the counts are the same either way.
-          The expansion uses streaming stores (pst_host_widen_stream) unless `fresh` says that host_out was
-          just allocated and never touched (its pages are zeroed into the cache by the first-touch faults)."""
+        Direct: the counts are copied in the dtype of host_out straight into it (4 / 2 / 1 B per count over
+          PCIe).  For uint16 / uint8 that is min(count, SAT) with SAT = 65535 / 255, and every element that
+          reads SAT is listed exactly in `self.overflow` = (flat index into host_out, int32 value) NumPy arrays
+          sorted by index (formats.widen rebuilds int32); on every other route self.overflow is None.  At
+          default depth about 2 in 10^4 counts reach 255 and none reaches 65535.
+        Staged through transport "u8" / "u16" / "i32": the chunk crosses PCIe in the transport format into
+          pinned staging buffers (cached per device) and host threads (pst_host_widen) expand it into host_out,
+          the overflow list is applied at the end: the caller receives exact int32 / int64 counts.  This is the
+          path of the reference-shaped call, which returns a fresh (pageable) int64 array.  The expansion uses
+          streaming stores (pst_host_widen_stream) unless `fresh` says that host_out was just allocated and
+          never touched (its pages are zeroed into the cache by the first-touch faults).
+
+        | host_out                                | transport            | route                      |
+        |-----------------------------------------|----------------------|----------------------------|
+        | pinned int32 tensor                     | None                 | "u8" (*), else direct      |
+        | int32 tensor, not pinned                | None                 | "u8" (*), else "i32"       |
+        | int32 tensor, pinned or not             | "direct"             | direct                     |
+        | uint16 / uint8 tensor                   | None or "direct"     | direct, narrow             |
+        | uint16 / uint8 tensor                   | anything else        | ValueError                 |
+        | uint16 / uint8 NumPy array              | any                  | ValueError                 |
+        | int64 tensor, int32 / int64 NumPy array | None                 | "u8" (*), else "i32"       |
+        | int64 tensor, int32 / int64 NumPy array | "direct"             | ValueError                 |
+        | int32 / int64 tensor or NumPy array     | "i32" / "u16" / "u8" | staged with that transport |
+        | wrong shape or dtype                    | any                  | ValueError                 |
+
+        (*) "u8" where _shared_host_transport says it is faster on this host and no automatically chosen "u8"
+        has overflowed in this process: its overflow list does not fit in deep regimes, and then the call is
+        sampled again through the wide route and the process keeps to it - the counts are the same either way."""
         n = int(rows.numel())
         is_np = isinstance(host_out, np.ndarray)
         if is_np:
@@ -344,38 +426,49 @@ class CountEngine(object):
         if hdt not in (torch.int32, torch.int64, torch.uint16, torch.uint8) or tuple(host_out.shape) != (n, self.G):
             raise ValueError("host_out must be an int32, int64, uint16 or uint8 CPU matrix of shape (%d, %d)"
                              % (n, self.G))
-        narrow_dst = hdt in (torch.uint16, torch.uint8)
         if not threads:
             threads = _host_threads()
-        auto = transport is None
-        wide = None
-        if auto and not narrow_dst:
-            # nothing asked for: the copy engine writes a pinned int32 matrix itself ("direct"), every other
-            # target is filled by host threads from int32 staging ("i32") - or, where this rank's share of
-            # the host cores expands uint8 well above the PCIe rate, from uint8 staging ("u8")
-            wide = "direct" if (not is_np and hdt == torch.int32 and pinned) else "i32"
-            transport = wide
-            if not _AUTO_STATE["narrow_overflowed"] and _shared_host_transport(threads) == "u8":
-                transport = "u8"
-        if transport in (None, "direct") and not is_np and hdt != torch.int64 and \
-                (pinned or narrow_dst or transport == "direct"):
-            return self._draw_to_host_direct(rows, scaling32, seed, cell0, host_out, chunk_cells, overflow_cap)
-        if narrow_dst:
-            raise ValueError("a uint16 / uint8 host matrix must be a CPU tensor and takes transport 'direct'")
+        route, retry = _host_route(is_np, hdt, pinned, transport, threads)
+        self.overflow = None
+
+        def fill(route, overflow_cap, fresh):
+            if route == "direct":
+                ovf = self._dense_chunks(rows, scaling32, seed, cell0, hdt, chunk_cells, overflow_cap,
+                                         host_out=host_out)
+                if ovf is not None:
+                    index, value = ovf.read(hdt)
+                    index, order = torch.sort(index)            # appended in no particular order
+                    self.overflow = (index.cpu().numpy(), value[order].cpu().numpy())
+                return host_out
+            G, width = self.G, _TRANSPORTS[route].itemsize
+            dst_bits = 32 if hdt == torch.int32 else 64
+            dst_ptr = host_out.ctypes.data if is_np else host_out.data_ptr()
+            lib = nat.load()
+            widen = lib.pst_host_widen if fresh else lib.pst_host_widen_stream
+
+            def expand(staged, lo, hi):
+                rc = widen(staged.data_ptr(), 8 * width, dst_ptr + lo * G * (dst_bits // 8), dst_bits,
+                           (hi - lo) * G, int(threads))
+                if rc != 0:
+                    raise nat.NativeError("pst_host_widen failed")
+
+            listed = self.stream_chunks(rows, scaling32, seed, cell0, expand, route, chunk_cells, overflow_cap)
+            if listed is not None:
+                index, value = listed
+                lib.pst_host_apply_overflow(dst_ptr, dst_bits, 0, n * G, index.data_ptr(), value.data_ptr(),
+                                            int(index.numel()))
+            return host_out
+
         try:
-            return self._draw_to_host_staged(rows, scaling32, seed, cell0, host_out, hdt, chunk_cells, overflow_cap,
-                                             transport or "i32", threads, fresh)
+            return fill(route, overflow_cap, fresh)
         except OverflowError:
-            if not (auto and transport == "u8"):
+            if retry is None:
                 raise
         # A deep regime (more than 1 % of the counts above 254): the uint8 transport nobody asked for does not
         # pay here.  The draw is a pure function of (seed, cell, gene): sample again through the wide transport,
         # and keep to it for the rest of the process.
         _AUTO_STATE["narrow_overflowed"] = True
-        if wide == "direct":
-            return self._draw_to_host_direct(rows, scaling32, seed, cell0, host_out, chunk_cells, None)
-        return self._draw_to_host_staged(rows, scaling32, seed, cell0, host_out, hdt, chunk_cells, None,
-                                         "i32", threads, False)
+        return fill(retry, None, False)
 
     def stream_chunks(self, rows, scaling32, seed, cell0, consume, transport="i32", chunk_cells=None,
                       overflow_cap=None):
@@ -385,75 +478,14 @@ class CountEngine(object):
         next chunk is sampled and copied.  The matrix is never resident anywhere: this is the streamed
         path for outputs larger than HBM (config 5: 600 GB).  Returns the overflow list of the narrow
         transports as CPU tensors (flat index, exact value), unsorted, or None."""
-        import concurrent.futures
-        n, G = int(rows.numel()), self.G
-        tdt = {"u8": torch.uint8, "u16": torch.uint16, "i32": torch.int32}.get(transport)
+        tdt = _TRANSPORTS.get(transport)
         if tdt is None:
             raise ValueError("transport must be 'i32', 'u16' or 'u8'")
-        width = torch.empty(0, dtype=tdt).element_size()
-        narrow = width < 4
-        ramp_up = chunk_cells is None
-        if chunk_cells is None:
-            chunk_cells = max(1, min(n, _STAGE_BYTES // max(1, width * G)))
-        if narrow and overflow_cap is None:
-            overflow_cap = (1 << 20) if width == 2 else max(1 << 20, n * G // 100)
-        dev = self.dev
-        stage_dev = [torch.empty((chunk_cells, G), dtype=tdt, device=dev) for _ in range(2)]
-        stage_host = _pinned_staging(dev, chunk_cells * G * width)
-        if narrow:
-            work = torch.empty((chunk_cells, G), dtype=torch.int32, device=dev)
-            ovf_index = torch.empty(max(1, overflow_cap), dtype=torch.int64, device=dev)
-            ovf_value = torch.empty(max(1, overflow_cap), dtype=torch.int32, device=dev)
-            ovf_count = torch.zeros(1, dtype=torch.int64, device=dev)
-        copy_stream = torch.cuda.Stream(device=dev)
-        main = torch.cuda.current_stream(dev)
-        pool = concurrent.futures.ThreadPoolExecutor(max_workers=1)
-        pending = [None, None]                      # consumer still reading stage_host[k]
-
-        def landed(k, lo, hi, event):
-            event.synchronize()                     # the chunk is in stage_host[k]
-            consume(stage_host[k][:(hi - lo) * G * width], lo, hi)
-
-        # the first chunks are smaller so that the copy and the consumer start almost immediately
-        bounds, lo = [], 0
-        ramp = [max(1, chunk_cells // 8), max(1, chunk_cells // 4), max(1, chunk_cells // 2)] if ramp_up else []
-        while lo < n:
-            size = ramp.pop(0) if ramp else chunk_cells
-            bounds.append((lo, min(n, lo + size)))
-            lo = bounds[-1][1]
-        try:
-            for i, (lo, hi) in enumerate(bounds):
-                k = i & 1
-                if pending[k] is not None:
-                    pending[k].result()             # stage_host[k] (and so stage_dev[k]) is free again
-                buf = stage_dev[k][:hi - lo]
-                if narrow:
-                    self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[:hi - lo])
-                    nat.call("pst_narrow_counts", work.data_ptr(), hi - lo, G, G, buf.data_ptr(), G, 8 * width, lo,
-                             ovf_index, ovf_value, int(overflow_cap), ovf_count, nat.stream_ptr(dev))
-                else:
-                    self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=buf)
-                done = torch.cuda.Event()
-                done.record(main)
-                with torch.cuda.stream(copy_stream):
-                    copy_stream.wait_event(done)
-                    stage_host[k][:(hi - lo) * G * width].copy_(buf.view(torch.uint8).view(-1), non_blocking=True)
-                    copied = torch.cuda.Event()
-                    copied.record(copy_stream)
-                pending[k] = pool.submit(landed, k, lo, hi, copied)
-            for f in pending:
-                if f is not None:
-                    f.result()
-        finally:
-            pool.shutdown(wait=True)
-        if not narrow:
+        ovf = self._dense_chunks(rows, scaling32, seed, cell0, tdt, chunk_cells, overflow_cap, consume=consume)
+        if ovf is None:
             return None
-        count = int(ovf_count.item())
-        if count > overflow_cap:
-            raise OverflowError("%d counts reach the saturation value of the %s transport but the overflow "
-                                "list holds %d: use a wider transport or a larger overflow_cap"
-                                % (count, transport, overflow_cap))
-        return ovf_index[:count].cpu(), ovf_value[:count].cpu()
+        index, value = ovf.read(tdt)
+        return index.cpu(), value.cpu()
 
     def draw_to_csr(self, rows, scaling32, seed, cell0, data_dtype=np.int64, chunk_cells=None, threads=0):
         """Sample the cells as CSR arrays on the host: (indptr, indices, data) NumPy arrays, columns ascending
@@ -469,7 +501,6 @@ class CountEngine(object):
         staging and host threads widen them into indices[p0:p1] / data[p0:p1] while the next chunk is
         sampled; the values that saturated uint16 are written from the exact overflow list at the end.
         data_dtype: np.int64 or np.int32."""
-        import concurrent.futures
         data_dtype = np.dtype(data_dtype)
         if data_dtype not in (np.dtype(np.int32), np.dtype(np.int64)):
             raise ValueError("CSR data must be int32 or int64, not %s" % data_dtype)
@@ -479,17 +510,7 @@ class CountEngine(object):
         if n == 0 or G == 0:
             return np.zeros(n + 1, np.int32), np.zeros(0, np.int32), np.zeros(0, data_dtype)
         ibits = 16 if G <= 65536 else 32                 # width of the column stream
-        ramp_up = chunk_cells is None
-        if chunk_cells is None:
-            chunk_cells = _STAGE_BYTES // max(1, (ibits // 8 + 2) * G)
-        chunk_cells = max(1, min(n, int(chunk_cells)))
-        bounds, lo = [], 0
-        # the first chunks are smaller so that the copy and the host threads start almost immediately
-        ramp = [max(1, chunk_cells // 8), max(1, chunk_cells // 4), max(1, chunk_cells // 2)] if ramp_up else []
-        while lo < n:
-            size = ramp.pop(0) if ramp else chunk_cells
-            bounds.append((lo, min(n, lo + size)))
-            lo = bounds[-1][1]
+        chunk_cells, bounds = _plan_chunks(n, chunk_cells, (ibits // 8 + 2) * G, _STAGE_BYTES)
         st = nat.stream_ptr(dev)
         main = torch.cuda.current_stream(dev)
         events = CountEngine.csr_timers
@@ -507,6 +528,7 @@ class CountEngine(object):
         nat.call("pst_csr_row_offsets", row_nnz, n, indptr_d, st)
         if events is not None:
             ev[1].record(main)
+            ev[2].record(main)                           # and again behind every pack kernel of pass 2
         indptr64 = indptr_d.cpu().numpy()
         n_sat = int(sat.item())
         self.check()                                     # domain / range errors before any result memory
@@ -524,153 +546,132 @@ class CountEngine(object):
         def value_offset(m):                            # the value stream starts on a 64-byte boundary
             return (m * ibytes + 63) // 64 * 64
 
-        stage_bytes = max(value_offset(int(indptr64[hi] - indptr64[lo])) + 2 * int(indptr64[hi] - indptr64[lo])
-                          for lo, hi in bounds)
+        def window(lo, hi):                             # first nonzero, nonzeros and packed bytes of cells [lo, hi)
+            p0, m = int(indptr64[lo]), int(indptr64[hi] - indptr64[lo])
+            return p0, m, value_offset(m) + 2 * m
+
+        stage_bytes = max(window(lo, hi)[2] for lo, hi in bounds)
         stage_dev = [torch.empty(max(1, stage_bytes), dtype=torch.uint8, device=dev) for _ in range(2)]
         stage_host = _pinned_staging(dev, stage_bytes)
-        ovf_pos = torch.empty(max(1, n_sat), dtype=torch.int64, device=dev)
-        ovf_value = torch.empty(max(1, n_sat), dtype=torch.int32, device=dev)
-        ovf_count = torch.zeros(1, dtype=torch.int64, device=dev)
+        ovf = _OverflowList(n_sat, dev)
         pack_flags = torch.zeros(1, dtype=torch.int32, device=dev)
-        copy_stream = torch.cuda.Stream(device=dev)
-        pool = concurrent.futures.ThreadPoolExecutor(max_workers=1)
-        pending = [None, None]                          # host threads still reading stage_host[k]
 
-        def landed(k, p0, m, event):
-            event.synchronize()                         # both streams of the chunk are in stage_host[k]
-            src = stage_host[k].data_ptr()
+        # ---- pass 2: redraw, pack, stream
+        def produce(k, lo, hi):
+            p0, m, used = window(lo, hi)
+            self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[:hi - lo])
+            buf = stage_dev[k]
+            nat.call("pst_csr_pack", work.data_ptr(), hi - lo, G, G, indptr_d[lo:hi + 1], p0, buf.data_ptr(),
+                     ibits, buf.data_ptr() + value_offset(m), 16, *ovf.kernel_args, pack_flags, st)
+            if events is not None:
+                ev[2].record(main)
+            return buf[:used], stage_host[k][:used]
+
+        def consume(staged, lo, hi):
+            p0, m, _ = window(lo, hi)
+            src = staged.data_ptr()
             rc = widen_i(src, ibits, indices.ctypes.data + p0 * idx_dtype.itemsize, ibits_out, m, int(threads))
             rc |= widen_d(src + value_offset(m), 16, data.ctypes.data + p0 * data_dtype.itemsize, dbits_out, m,
                           int(threads))
             if rc != 0:
                 raise nat.NativeError("pst_host_widen failed")
 
-        # ---- pass 2: redraw, pack, stream
+        # a chunk without nonzeros has nothing to pack: the redraw would have no nonzero either
+        self._copy_chunks([(lo, hi) for lo, hi in bounds if window(lo, hi)[1]], produce, consume)
+        if events is not None:
+            events.append(tuple(ev))
+        self.check()
+        if int(pack_flags.item()) != 0:
+            raise RuntimeError("the redrawn counts do not match the row sizes of the first pass")
+        listed = int(ovf.count.item())
+        if listed != n_sat:
+            raise RuntimeError("%d counts >= 65535 in the second pass, %d in the first" % (listed, n_sat))
+        if n_sat:
+            pos, value = ovf.pos[:n_sat].cpu(), ovf.value[:n_sat].cpu()
+            lib.pst_host_apply_overflow(data.ctypes.data, dbits_out, 0, nnz, pos.data_ptr(), value.data_ptr(), n_sat)
+        return indptr, indices, data
+
+    def _dense_chunks(self, rows, scaling32, seed, cell0, tdt, chunk_cells, overflow_cap, host_out=None,
+                      consume=None):
+        """The counts of the cells in the transfer dtype `tdt` through _copy_chunks: straight into `host_out`
+        (a CPU tensor of dtype tdt) or through pinned staging into `consume`.  Owns the dense chunk sizes and
+        the narrowing: int32 is drawn into the copy buffer itself; uint16 / uint8 are drawn into an int32 work
+        buffer and pst_narrow_counts writes min(count, SAT) into the copy buffer and lists the saturated counts.
+        Returns that _OverflowList, or None for int32."""
+        n, G, dev = int(rows.numel()), self.G, self.dev
+        width = tdt.itemsize
+        # ~1 GiB copies keep the copy engine at its large-transfer rate; staged chunks fit the pinned staging
+        chunk, bounds = _plan_chunks(n, chunk_cells, width * G, (1 << 30) if host_out is not None else _STAGE_BYTES)
+        stage = [torch.empty((chunk, G), dtype=tdt, device=dev) for _ in range(2)]
+        ovf = None
+        if width < 4:
+            # the int32 chunk is consumed by the narrowing kernel on the sampling stream, so one is enough
+            work = torch.empty((chunk, G), dtype=torch.int32, device=dev)
+            if overflow_cap is None:
+                # uint8 lists every count >= 255 (2e-4 of them at default depth; allow 50x that)
+                overflow_cap = (1 << 20) if width == 2 else max(1 << 20, n * G // 100)
+            ovf = _OverflowList(overflow_cap, dev)
+        if host_out is None:
+            stage_host = _pinned_staging(dev, chunk * G * width)
+
+        def produce(k, lo, hi):
+            buf = stage[k][:hi - lo]
+            if ovf is None:
+                self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=buf)
+            else:
+                self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[:hi - lo])
+                nat.call("pst_narrow_counts", work.data_ptr(), hi - lo, G, G, buf.data_ptr(), G, 8 * width, lo,
+                         *ovf.kernel_args, nat.stream_ptr(dev))
+            if host_out is not None:
+                return buf, host_out[lo:hi]
+            return buf.view(torch.uint8).view(-1), stage_host[k][:(hi - lo) * G * width]
+
+        self._copy_chunks(bounds, produce, consume)
+        return ovf
+
+    def _copy_chunks(self, bounds, produce, consume=None):
+        """The double-buffered device->host loop behind every chunked result.  For chunk i, with buffer
+        k = i & 1, produce(k, lo, hi) queues the device work that fills device buffer k on the current stream
+        and returns (src, dst): the device bytes and their host destination.  One side stream copies src into
+        dst while the next chunk is produced.  Before buffer k is produced again, the current stream waits on
+        the device for its copy, so without `consume` the host never waits per chunk.  With `consume`, one
+        worker thread calls consume(dst, lo, hi) once the copy has landed, and the host waits for it before
+        buffer k is produced again (dst is pinned staging that the next use of k overwrites).  Owns the
+        overlap and its teardown: whatever ends the loop, the side stream and the worker are drained before
+        the buffers can go back to the allocator."""
+        main = torch.cuda.current_stream(self.dev)
+        copy_stream = torch.cuda.Stream(device=self.dev)
+        pool = concurrent.futures.ThreadPoolExecutor(max_workers=1)
+        copied = [None, None]                           # the copy out of buffer k has finished
+        pending = [None, None]                          # consume still reading the host side of buffer k
+
+        def landed(event, dst, lo, hi):
+            event.synchronize()                         # the chunk is in dst
+            consume(dst, lo, hi)
+
         try:
             for i, (lo, hi) in enumerate(bounds):
-                p0, p1 = int(indptr64[lo]), int(indptr64[hi])
-                m = p1 - p0
-                if m == 0:
-                    continue                            # nothing to pack: the redraw has no nonzero either
                 k = i & 1
                 if pending[k] is not None:
-                    pending[k].result()                 # stage_host[k] (and so stage_dev[k]) is free again
-                self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[:hi - lo])
-                buf = stage_dev[k]
-                nat.call("pst_csr_pack", work.data_ptr(), hi - lo, G, G, indptr_d[lo:hi + 1], p0, buf.data_ptr(),
-                         ibits, buf.data_ptr() + value_offset(m), 16, ovf_pos, ovf_value, n_sat, ovf_count,
-                         pack_flags, st)
-                used = value_offset(m) + 2 * m
+                    pending[k].result()
+                if copied[k] is not None:
+                    main.wait_event(copied[k])
+                src, dst = produce(k, lo, hi)
                 done = torch.cuda.Event()
                 done.record(main)
                 with torch.cuda.stream(copy_stream):
                     copy_stream.wait_event(done)
-                    stage_host[k][:used].copy_(buf[:used], non_blocking=True)
-                    copied = torch.cuda.Event()
-                    copied.record(copy_stream)
-                pending[k] = pool.submit(landed, k, p0, m, copied)
-            if events is not None:
-                ev[2].record(main)
-                events.append(tuple(ev))
+                    dst.copy_(src, non_blocking=True)
+                    copied[k] = torch.cuda.Event()
+                    copied[k].record(copy_stream)
+                if consume is not None:
+                    pending[k] = pool.submit(landed, copied[k], dst, lo, hi)
             for f in pending:
                 if f is not None:
                     f.result()
         finally:
+            copy_stream.synchronize()
             pool.shutdown(wait=True)
-        self.check()
-        if int(pack_flags.item()) != 0:
-            raise RuntimeError("the redrawn counts do not match the row sizes of the first pass")
-        listed = int(ovf_count.item())
-        if listed != n_sat:
-            raise RuntimeError("%d counts >= 65535 in the second pass, %d in the first" % (listed, n_sat))
-        if n_sat:
-            pos, value = ovf_pos[:n_sat].cpu(), ovf_value[:n_sat].cpu()
-            lib.pst_host_apply_overflow(data.ctypes.data, dbits_out, 0, nnz, pos.data_ptr(), value.data_ptr(), n_sat)
-        return indptr, indices, data
-
-    def _draw_to_host_staged(self, rows, scaling32, seed, cell0, host_out, hdt, chunk_cells, overflow_cap,
-                             transport, threads, fresh=False):
-        n, G = int(rows.numel()), self.G
-        width = {"u8": 1, "u16": 2, "i32": 4}.get(transport)
-        if width is None:
-            raise ValueError("transport must be 'direct', 'i32', 'u16' or 'u8'")
-        dst_bits = 32 if hdt == torch.int32 else 64
-        dst_ptr = host_out.ctypes.data if isinstance(host_out, np.ndarray) else host_out.data_ptr()
-        lib = nat.load()
-        widen = lib.pst_host_widen if fresh else lib.pst_host_widen_stream
-        self.overflow = None
-
-        def expand(staged, lo, hi):
-            rc = widen(staged.data_ptr(), 8 * width, dst_ptr + lo * G * (dst_bits // 8), dst_bits,
-                                    (hi - lo) * G, int(threads))
-            if rc != 0:
-                raise nat.NativeError("pst_host_widen failed")
-
-        listed = self.stream_chunks(rows, scaling32, seed, cell0, expand, transport, chunk_cells, overflow_cap)
-        if listed is not None:
-            index, value = listed
-            lib.pst_host_apply_overflow(dst_ptr, dst_bits, 0, n * G, index.data_ptr(), value.data_ptr(),
-                                        int(index.numel()))
-        return host_out
-
-    def _draw_to_host_direct(self, rows, scaling32, seed, cell0, host_out, chunk_cells=None, overflow_cap=None):
-        """Chunks copied straight into a pinned CPU tensor of the transfer dtype (see draw_to_host)."""
-        n = int(rows.numel())
-        narrow = host_out.dtype in (torch.uint16, torch.uint8)
-        width = host_out.element_size()
-        if narrow and overflow_cap is None:
-            # uint8 lists every count >= 255 (2e-4 of them at default depth; allow 50x that)
-            overflow_cap = (1 << 20) if width == 2 else max(1 << 20, n * self.G // 100)
-        if chunk_cells is None:
-            # ~1 GiB copies keep the copy engine at its large-transfer rate; the first chunks are
-            # smaller so that the device->host stream starts almost immediately
-            chunk_cells = max(1, min(n, (1 << 30) // max(1, width * self.G)))
-            ramp = [max(1, chunk_cells // 8), max(1, chunk_cells // 4), max(1, chunk_cells // 2)]
-        else:
-            ramp = []
-        bounds, lo = [], 0
-        while lo < n:
-            size = ramp.pop(0) if ramp else chunk_cells
-            bounds.append((lo, min(n, lo + size)))
-            lo = bounds[-1][1]
-        # staging buffers (what the copy engine reads) are double-buffered; in the narrow format the
-        # int32 chunk is consumed by the narrowing kernel on the sampling stream, so one is enough
-        stage = [torch.empty((chunk_cells, self.G), dtype=host_out.dtype, device=self.dev) for _ in range(2)]
-        self.overflow = None
-        if narrow:
-            work = torch.empty((chunk_cells, self.G), dtype=torch.int32, device=self.dev)
-            ovf_index = torch.empty(max(1, overflow_cap), dtype=torch.int64, device=self.dev)
-            ovf_value = torch.empty(max(1, overflow_cap), dtype=torch.int32, device=self.dev)
-            ovf_count = torch.zeros(1, dtype=torch.int64, device=self.dev)
-        copy_stream = torch.cuda.Stream(device=self.dev)
-        main = torch.cuda.current_stream(self.dev)
-        free = [torch.cuda.Event(), torch.cuda.Event()]
-        for i, (lo, hi) in enumerate(bounds):
-            buf = stage[i & 1][:hi - lo]
-            if i >= 2:
-                main.wait_event(free[i & 1])
-            if narrow:
-                self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[:hi - lo])
-                nat.call("pst_narrow_counts", work.data_ptr(), hi - lo, self.G, self.G, buf.data_ptr(), self.G,
-                         8 * width, lo, ovf_index, ovf_value, int(overflow_cap), ovf_count, nat.stream_ptr(self.dev))
-            else:
-                self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=buf)
-            done = torch.cuda.Event()
-            done.record(main)
-            with torch.cuda.stream(copy_stream):
-                copy_stream.wait_event(done)
-                host_out[lo:hi].copy_(buf, non_blocking=True)
-                free[i & 1].record(copy_stream)
-        copy_stream.synchronize()
-        if narrow:
-            count = int(ovf_count.item())
-            if count > overflow_cap:
-                raise OverflowError("%d counts reach the saturation value of %s but the overflow list holds %d: "
-                                    "use a wider host buffer or a larger overflow_cap"
-                                    % (count, str(host_out.dtype).replace("torch.", ""), overflow_cap))
-            index, order = torch.sort(ovf_index[:count])            # appended in no particular order
-            self.overflow = (index.cpu().numpy(), ovf_value[:count][order].cpu().numpy())
-        return host_out
 
     def check(self):
         """One device->host read of the status word; raises like the reference would."""

@@ -340,6 +340,29 @@ def test_host_side_helpers_of_the_device_to_host_path():
     assert lay[1] == 4 + 4 * lay[0] and lay[2] == lay[1] + 1000 and lay[3] == lay[2] + 38
 
 
+def test_chunk_plan_covers_every_cell_once_in_order():
+    """device._plan_chunks: the chunks of every chunked device->host call.  A budget gives chunks of
+    budget // cell_bytes cells after a ramp of 1/8, 1/4 and 1/2 of that; an explicit chunk size has no ramp."""
+    from prosstt_b200.device import _plan_chunks
+    assert _plan_chunks(1000, None, 40, 40 * 80) == (80, [(0, 10), (10, 30), (30, 70)]
+                                                     + [(lo, min(1000, lo + 80)) for lo in range(70, 1000, 80)])
+    assert _plan_chunks(1000, 300, 40, 40 * 80) == (300, [(0, 300), (300, 600), (600, 900), (900, 1000)])
+    assert _plan_chunks(0, None, 40, 1 << 30) == (1, [])
+    assert _plan_chunks(0, 7, 40, 1 << 30) == (1, [])
+    # n smaller than one chunk: the ramp still applies (chunk 5 -> 1, 1, 2, then the rest), an explicit size not
+    assert _plan_chunks(5, None, 40, 1 << 30) == (5, [(0, 1), (1, 2), (2, 4), (4, 5)])
+    assert _plan_chunks(5, 100, 40, 1 << 30) == (5, [(0, 5)])
+    assert _plan_chunks(3, None, 40, 1) == (1, [(0, 1), (1, 2), (2, 3)])        # budget below one cell
+    for n in (1, 2, 7, 100, 1001):
+        for chunk_cells in (None, 1, 3, 97, 5000):
+            for cell_bytes, budget in ((0, 64), (4, 64), (40, 4000), (4, 1 << 30)):
+                chunk, bounds = _plan_chunks(n, chunk_cells, cell_bytes, budget)
+                assert [c for lo, hi in bounds for c in range(lo, hi)] == list(range(n))
+                assert all(1 <= hi - lo <= chunk for lo, hi in bounds) and chunk <= n
+                if chunk_cells is not None:
+                    assert all(hi - lo == min(chunk_cells, n) for lo, hi in bounds[:-1])
+
+
 def test_result_pool_recycles_only_unreachable_matrices():
     """hostpool: the buffer of a result comes back when the array AND every view of it are gone, is handed
     out again for a matrix of similar size, and PST_HOST_POOL_GB=0 turns the pool off."""
