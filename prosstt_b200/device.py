@@ -565,11 +565,11 @@ class CountEngine(object):
                      ibits, buf.data_ptr() + value_offset(m), 16, *ovf.kernel_args, pack_flags, st)
             if events is not None:
                 ev[2].record(main)
-            return buf[:used], stage_host[k][:used]
+            return [(buf[:used], stage_host[k][:used])]
 
-        def consume(staged, lo, hi):
+        def consume(dsts, lo, hi):
             p0, m, _ = window(lo, hi)
-            src = staged.data_ptr()
+            src = dsts[0].data_ptr()
             rc = widen_i(src, ibits, indices.ctypes.data + p0 * idx_dtype.itemsize, ibits_out, m, int(threads))
             rc |= widen_d(src + value_offset(m), 16, data.ctypes.data + p0 * data_dtype.itemsize, dbits_out, m,
                           int(threads))
@@ -590,6 +590,121 @@ class CountEngine(object):
             pos, value = ovf.pos[:n_sat].cpu(), ovf.value[:n_sat].cpu()
             lib.pst_host_apply_overflow(data.ctypes.data, dbits_out, 0, nnz, pos.data_ptr(), value.data_ptr(), n_sat)
         return indptr, indices, data
+
+    def stream_csr(self, rows, scaling32, seed, cell0, consume, index_dtype=np.int64, data_dtype=np.int64,
+                   chunk_cells=None, threads=0, overflow_cap=None):
+        """Sample the cells in chunks and hand each one as CSR to consume(lo, hi, indptr, indices, data), on a
+        worker thread, once per chunk, in cell order.  indptr is chunk-local int64 (hi - lo + 1 entries from 0);
+        indices and data are the chunk's nonzeros in `index_dtype` / `data_dtype` (int32 or int64), columns
+        ascending in every row.  They are reused host buffers, valid during the call only.  Returns the total
+        nnz.  Concatenated over the chunks, the arrays are draw_to_csr's, so the counts are those of draw().
+
+        Nothing is sized by the whole matrix, and every chunk is drawn once.  Chunk i is drawn into int32 work
+        buffer k = i & 1.  pst_csr_row_counts and pst_csr_row_offsets give its chunk-local row pointer and its
+        count of values >= 65535, and pst_csr_pack writes it at once into device staging k: a uint16 column
+        stream (int32 when G > 65536) and, at the fixed offset of chunk x G column entries, a uint16 value
+        stream, plus the saturated values in overflow list k.  The chunk's (saturated, nnz, status word) reach
+        pinned memory by a small async copy, which the host reads one chunk late, once chunk i+1 is queued
+        (_copy_chunks' collect).  Only then are chunk i's copies queued, sized to its nnz: 4 B per nonzero
+        over PCIe while G <= 65536.  A chunk with more saturated values than its list holds (overflow_cap
+        entries at first) grows the list and is packed again from its work buffer, which survives until chunk
+        i+2 is drawn.  An error in the status word raises as draw() would (raise_flags) and ends the stream."""
+        index_dtype, data_dtype = np.dtype(index_dtype), np.dtype(data_dtype)
+        for what, dt in (("indices", index_dtype), ("data", data_dtype)):
+            if dt not in (np.dtype(np.int32), np.dtype(np.int64)):
+                raise ValueError("CSR %s must be int32 or int64, not %s" % (what, dt))
+        n, G, dev = int(rows.numel()), self.G, self.dev
+        if not threads:
+            threads = _host_threads()
+        if n == 0:
+            return 0
+        if G == 0:
+            consume(0, n, np.zeros(n + 1, np.int64), np.zeros(0, index_dtype), np.zeros(0, data_dtype))
+            return 0
+        ibits = 16 if G <= 65536 else 32                 # width of the column stream
+        ibytes = ibits // 8
+        chunk, bounds = _plan_chunks(n, chunk_cells, (ibytes + 2) * G, _STAGE_BYTES)
+        value_at = (chunk * G * ibytes + 63) // 64 * 64  # the value stream, after the worst-case column stream
+        st = nat.stream_ptr(dev)
+        work = [torch.empty((chunk, G), dtype=torch.int32, device=dev) for _ in range(2)]
+        stage = [torch.empty(value_at + 2 * chunk * G, dtype=torch.uint8, device=dev) for _ in range(2)]
+        row_nnz = torch.empty(chunk, dtype=torch.int32, device=dev)      # read by the scan right after the count
+        indptr = [torch.empty(chunk + 1, dtype=torch.int64, device=dev) for _ in range(2)]
+        info = torch.zeros((2, 3), dtype=torch.int64, device=dev)        # saturated, nnz, status word
+        info_host = torch.zeros((2, 3), dtype=torch.int64).pin_memory()
+        sized = [None, None]
+        ovf = [_OverflowList(overflow_cap or (1 << 16), dev) for _ in range(2)]
+        ovf_host = [torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory() for k in range(2)]
+        pack_flags = torch.zeros(1, dtype=torch.int32, device=dev)
+        # host side: the row pointer, then the streams of the nonzeros, values on a 64-byte boundary
+        stage_host = _pinned_staging(dev, 8 * (chunk + 1) + value_at + 64 + 2 * chunk * G)
+        # the widened chunk, reused from chunk to chunk: its pages are touched as the chunks' nnz needs them and
+        # hostpool keeps them mapped for the next call.  Past the first chunk they are mapped and out of cache,
+        # which is what the streaming stores are for.
+        indices_w = hostpool.result_array((chunk * G,), index_dtype)[0]
+        data_w = hostpool.result_array((chunk * G,), data_dtype)[0]
+        lib = nat.load()
+        widen_i = widen_d = lib.pst_host_widen_stream
+        total = [0]
+
+        def pack(k, cells):
+            ovf[k].count.zero_()
+            nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, stage[k].data_ptr(), ibits,
+                     stage[k].data_ptr() + value_at, 16, *ovf[k].kernel_args, pack_flags, st)
+
+        def produce(k, lo, hi):
+            cells = hi - lo
+            self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[k][:cells])
+            info[k].zero_()
+            nat.call("pst_csr_row_counts", work[k].data_ptr(), cells, G, G, row_nnz, info[k, 0], st)
+            nat.call("pst_csr_row_offsets", row_nnz, cells, indptr[k], st)
+            pack(k, cells)
+            info[k, 1].copy_(indptr[k][cells])
+            info[k, 2].copy_(self.flags[0])
+            info_host[k].copy_(info[k], non_blocking=True)
+            sized[k] = torch.cuda.Event()
+            sized[k].record(torch.cuda.current_stream(dev))
+
+        def collect(k, lo, hi):
+            sized[k].synchronize()
+            n_sat, nnz, word = info_host[k].tolist()
+            if word:
+                self.flags[0].zero_()
+                raise_flags(word)
+            cells = hi - lo
+            if n_sat > ovf[k].capacity:
+                ovf[k] = _OverflowList(max(n_sat, 2 * ovf[k].capacity), dev)
+                ovf_host[k] = torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory()
+                pack(k, cells)
+                torch.cuda.current_stream(dev).synchronize()   # the copies wait for the first pack only
+            total[0] += nnz
+            at = 8 * (cells + 1)
+            vat = (at + nnz * ibytes + 63) // 64 * 64
+            h = stage_host[k]
+            pairs = [(indptr[k][:cells + 1].view(torch.uint8), h[:at]),
+                     (stage[k][:nnz * ibytes], h[at:at + nnz * ibytes]),
+                     (stage[k][value_at:value_at + 2 * nnz], h[vat:vat + 2 * nnz])]
+            if n_sat:
+                pairs += [(ovf[k].pos[:n_sat].view(torch.uint8), ovf_host[k][:8 * n_sat]),
+                          (ovf[k].value[:n_sat].view(torch.uint8), ovf_host[k][8 * n_sat:12 * n_sat])]
+            return pairs
+
+        def landed(dsts, lo, hi):
+            nnz = dsts[1].numel() // ibytes
+            indices, data = indices_w[:nnz], data_w[:nnz]
+            rc = widen_i(dsts[1].data_ptr(), ibits, indices.ctypes.data, 8 * index_dtype.itemsize, nnz, int(threads))
+            rc |= widen_d(dsts[2].data_ptr(), 16, data.ctypes.data, 8 * data_dtype.itemsize, nnz, int(threads))
+            if rc != 0:
+                raise nat.NativeError("pst_host_widen failed")
+            if len(dsts) > 3:
+                lib.pst_host_apply_overflow(data.ctypes.data, 8 * data_dtype.itemsize, 0, nnz, dsts[3].data_ptr(),
+                                            dsts[4].data_ptr(), dsts[3].numel() // 8)
+            consume(lo, hi, dsts[0].numpy().view(np.int64), indices, data)
+
+        self._copy_chunks(bounds, produce, landed, collect)
+        if int(pack_flags.item()) != 0:
+            raise RuntimeError("the packed counts do not match the row sizes of their chunk")
+        return total[0]
 
     def _dense_chunks(self, rows, scaling32, seed, cell0, tdt, chunk_cells, overflow_cap, host_out=None,
                       consume=None):
@@ -623,49 +738,65 @@ class CountEngine(object):
                 nat.call("pst_narrow_counts", work.data_ptr(), hi - lo, G, G, buf.data_ptr(), G, 8 * width, lo,
                          *ovf.kernel_args, nat.stream_ptr(dev))
             if host_out is not None:
-                return buf, host_out[lo:hi]
-            return buf.view(torch.uint8).view(-1), stage_host[k][:(hi - lo) * G * width]
+                return [(buf, host_out[lo:hi])]
+            return [(buf.view(torch.uint8).view(-1), stage_host[k][:(hi - lo) * G * width])]
 
-        self._copy_chunks(bounds, produce, consume)
+        self._copy_chunks(bounds, produce, consume and (lambda dsts, lo, hi: consume(dsts[0], lo, hi)))
         return ovf
 
-    def _copy_chunks(self, bounds, produce, consume=None):
+    def _copy_chunks(self, bounds, produce, consume=None, collect=None):
         """The double-buffered device->host loop behind every chunked result.  For chunk i, with buffer
         k = i & 1, produce(k, lo, hi) queues the device work that fills device buffer k on the current stream
-        and returns (src, dst): the device bytes and their host destination.  One side stream copies src into
-        dst while the next chunk is produced.  Before buffer k is produced again, the current stream waits on
-        the device for its copy, so without `consume` the host never waits per chunk.  With `consume`, one
-        worker thread calls consume(dst, lo, hi) once the copy has landed, and the host waits for it before
-        buffer k is produced again (dst is pinned staging that the next use of k overwrites).  Owns the
-        overlap and its teardown: whatever ends the loop, the side stream and the worker are drained before
-        the buffers can go back to the allocator."""
+        and returns the chunk's copies: a list of (src, dst) pairs, device bytes and their host destination.
+        One side stream copies every src into its dst while the next chunk is produced.  Before buffer k is
+        produced again, the current stream waits on the device for its copies, so without `consume` the host
+        never waits per chunk.  With `consume`, one worker thread calls consume(dsts, lo, hi) once the copies
+        have landed, and the host waits for it before it copies into buffer k again (the dsts are pinned
+        staging that the next use of k overwrites).
+        With `collect`, the copies run one chunk late: produce only queues chunk i's device work, and
+        collect(k, lo, hi) returns chunk i's copies once chunk i+1's work is queued, so the host can read what
+        chunk i left on the device (its size) while the device works on. The copies wait for chunk i's work
+        only, not for chunk i+1's: device work that collect queues itself must have finished when it returns.
+        Owns the overlap and its teardown: whatever ends the loop, the side stream and the worker are drained
+        before the buffers can go back to the allocator."""
         main = torch.cuda.current_stream(self.dev)
         copy_stream = torch.cuda.Stream(device=self.dev)
         pool = concurrent.futures.ThreadPoolExecutor(max_workers=1)
-        copied = [None, None]                           # the copy out of buffer k has finished
+        filled = [None, None]                           # the device work on buffer k has finished
+        copied = [None, None]                           # the copies out of buffer k have finished
         pending = [None, None]                          # consume still reading the host side of buffer k
 
-        def landed(event, dst, lo, hi):
-            event.synchronize()                         # the chunk is in dst
-            consume(dst, lo, hi)
+        def landed(event, dsts, lo, hi):
+            event.synchronize()                         # the chunk is in dsts
+            consume(dsts, lo, hi)
 
-        try:
-            for i, (lo, hi) in enumerate(bounds):
-                k = i & 1
-                if pending[k] is not None:
-                    pending[k].result()
-                if copied[k] is not None:
-                    main.wait_event(copied[k])
-                src, dst = produce(k, lo, hi)
-                done = torch.cuda.Event()
-                done.record(main)
-                with torch.cuda.stream(copy_stream):
-                    copy_stream.wait_event(done)
+        def copy(k, lo, hi, pairs):
+            if pending[k] is not None:
+                pending[k].result()
+            with torch.cuda.stream(copy_stream):
+                copy_stream.wait_event(filled[k])
+                for src, dst in pairs:
                     dst.copy_(src, non_blocking=True)
-                    copied[k] = torch.cuda.Event()
-                    copied[k].record(copy_stream)
-                if consume is not None:
-                    pending[k] = pool.submit(landed, copied[k], dst, lo, hi)
+                copied[k] = torch.cuda.Event()
+                copied[k].record(copy_stream)
+            if consume is not None:
+                pending[k] = pool.submit(landed, copied[k], [dst for _, dst in pairs], lo, hi)
+
+        lag = 0 if collect is None else 1
+        try:
+            for i in range(len(bounds) + lag):
+                if i < len(bounds):
+                    k = i & 1
+                    if copied[k] is not None:
+                        main.wait_event(copied[k])
+                    pairs = produce(k, *bounds[i])
+                    filled[k] = torch.cuda.Event()
+                    filled[k].record(main)
+                    if not lag:
+                        copy(k, *bounds[i], pairs)
+                if lag and i:
+                    k = (i - 1) & 1
+                    copy(k, *bounds[i - 1], collect(k, *bounds[i - 1]))
             for f in pending:
                 if f is not None:
                     f.result()

@@ -17,6 +17,10 @@ Extra keyword-only arguments (never required):
            scipy.sparse.csr_matrix (canonical: columns ascending, no explicit zeros; int32 indptr/indices,
            int64 when it has 2^31 nonzeros or more) with the same counts as "numpy".  The GPU compacts
            each chunk and only the nonzeros cross PCIe (CountEngine.draw_to_csr); not with host_out
+  path     with out="csr": stream the counts chunk by chunk to a CSR shard directory at `path`
+           (formats.CsrShardWriter, with the cells' pseudotime, branches and scalings) instead of holding
+           them in host memory; X is then the shard's memory-mapped matrix (formats.load_csr_shard).  The
+           counts are those of the in-memory call; every chunk is drawn once (CountEngine.stream_csr)
   sampler  "hybrid" (default): direct inversion of the NB cdf for mean <= 32, sd <= 20, gamma scale <= 32 and
            shape <= 48 - in fp32 below the 1 - 2^-14 quantile of its uniform, with a 64-bit uniform against an
            fp64-accumulated cdf above it, so body and far tail match the exact pmf (checked at 1e9 draws per
@@ -40,6 +44,7 @@ from prosstt_b200 import count_model as cm
 from prosstt_b200 import hostpool
 from prosstt_b200 import sim_utils as sut
 from prosstt_b200.device import CountEngine, TreeTables, choice_cdf, raise_flags, tree_tables
+from prosstt_b200.formats import CsrShardWriter, _csr_matrix, load_csr_shard
 from prosstt_b200.sharding import shard_range
 
 DEFAULT_SAMPLER = "hybrid"
@@ -414,8 +419,10 @@ def _shard_range(n, shard):
     return shard_range(n, rank, world)
 
 
-def _check_csr_request(out, dtype, host_out=None):
-    """out="csr" takes int64 (default) or int32 data and no preallocated host_out."""
+def _check_csr_request(out, dtype, host_out=None, path=None):
+    """out="csr" takes int64 (default) or int32 data and no preallocated host_out; path needs out="csr"."""
+    if path is not None and out != "csr":
+        raise ValueError("path= writes a CSR shard: it needs out='csr'")
     if out != "csr":
         return
     if host_out is not None:
@@ -424,24 +431,15 @@ def _check_csr_request(out, dtype, host_out=None):
         raise ValueError("out='csr' stores int64 or int32 counts, not %s" % np.dtype(dtype))
 
 
-def _csr_matrix(indptr, indices, data, shape):
-    """scipy.sparse.csr_matrix over the given arrays without a copy or a scan: the constructor would check
-    every column index and copy int64 index arrays whose contents fit int32.  The arrays are already in
-    canonical form (columns ascending in every row, no explicit zeros, no duplicates)."""
-    import scipy.sparse as sp
-    m = sp.csr_matrix(shape, dtype=data.dtype)
-    m.indptr, m.indices, m.data = indptr, indices, data
-    m.has_sorted_indices = True
-    m.has_canonical_format = True
-    return m
-
-
-def _sample_counts(engine, rows, s32, seed, first, dtype, out):
+def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=None):
     """The count matrix of the cells described by rows/s32: a device int32 tensor (out="torch"), a
     scipy.sparse.csr_matrix with `dtype` data (out="csr", CountEngine.draw_to_csr: only the nonzeros cross
     PCIe) or a fresh host array of `dtype` (reference: int64, simulation.py:651).  The host forms never hold
     the whole matrix on the GPU: chunks are sampled, copied into pinned staging and expanded into the result
-    by host threads while the next chunk is sampled (CountEngine.draw_to_host)."""
+    by host threads while the next chunk is sampled (CountEngine.draw_to_host).
+    out="csr" with `path`: the chunks go to a CSR shard at path (CountEngine.stream_csr into a
+    formats.CsrShardWriter, which also stores `cells` = (pseudotime, branches, scalings) host arrays) and the
+    shard's memory-mapped matrix is returned."""
     if out == "torch":
         X = engine.draw(rows, s32, seed, first)
         engine.check()
@@ -449,6 +447,11 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out):
     if out == "csr":
         _check_csr_request(out, dtype)
         n = int(rows.numel())
+        if path is not None:
+            with CsrShardWriter(path, (n, engine.G), *cells, dtype=dtype) as shard:
+                engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *chunk: shard.append(*chunk),
+                                  shard.index_dtype, dtype)
+            return load_csr_shard(path)[0]
         indptr, indices, data = engine.draw_to_csr(rows, s32, seed, first, data_dtype=dtype)
         torch.cuda.current_stream(engine.dev).synchronize()
         engine.check()
@@ -467,7 +470,8 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out):
 
 
 def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
-                    seed, first, dev, dtype, out, sampler, host_out=None, host_transport=None, host_threads=0):
+                    seed, first, dev, dtype, out, sampler, host_out=None, host_transport=None, host_threads=0,
+                    path=None):
     """Common tail of every sampler (simulation.py:590-599): scalings, then counts.
     host_out = (X, pseudotime, branch_codes, scalings) preallocated CPU tensors (int32 (n,G),
     int64, int32, float64; ideally pinned): the counts are streamed into them in cell chunks
@@ -476,7 +480,7 @@ def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mea
     and a fifth entry of host_out, a dict, receives the exact values of the saturated elements as
     "index" (flat, into X) and "value" arrays (formats.widen rebuilds the int32 matrix); without
     the dict a saturated element raises OverflowError instead of passing silently."""
-    _check_csr_request(out, dtype, host_out)
+    _check_csr_request(out, dtype, host_out, path)
     n = int(rows.numel())
     s64, s32 = sut.calc_scalings(n, scale, scale_mean, scale_v, seed=nat.derive_seed(seed, 1),
                                  first=first, device=dev, return_device=True)
@@ -502,15 +506,17 @@ def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mea
                                     "or use an int32 buffer"
                                     % (len(engine.overflow[0]), str(hX.dtype).replace("torch.", "")))
         return hX.numpy(), hpt.numpy(), tables.branch_names(hcodes.numpy()), hs.numpy()
-    X = _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out)
     if out == "torch":
-        return X, pt, codes, s64
-    return X, pt.cpu().numpy(), tables.branch_names(codes.cpu().numpy()), s64.cpu().numpy()
+        return _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out), pt, codes, s64
+    cells = pt.cpu().numpy(), tables.branch_names(codes.cpu().numpy()), s64.cpu().numpy()
+    X = _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out, path=path, cells=cells)
+    return (X,) + cells
 
 
 def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, scale_mean=0.,
                    seed=None, device=None, shard=None, dtype=np.int64, out="numpy",
-                   sampler=DEFAULT_SAMPLER, uniforms=None, host_out=None, host_transport=None, host_threads=0):
+                   sampler=DEFAULT_SAMPLER, uniforms=None, host_out=None, host_transport=None, host_threads=0, *,
+                   path=None):
     """Sample `no_cells` (pseudotime, branch) pairs according to tree.density and draw
     their counts (simulation.py:416-471).  Returns (X, pseudotime, branches, scalings).
     `uniforms` (one per cell) replays externally supplied draws through the index map.
@@ -536,7 +542,7 @@ def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, s
              nat.ptr(tables.d("pos_branch")), nat.ptr(rows), nat.ptr(pt), nat.ptr(codes), st)
     return _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
                            seed, lo, dev, dtype, out, sampler, host_out=host_out, host_transport=host_transport,
-                           host_threads=host_threads)
+                           host_threads=host_threads, path=path)
 
 
 def cover_whole_tree(tree):
@@ -554,7 +560,7 @@ def cover_whole_tree(tree):
 
 def sample_whole_tree(tree, n_factor, alpha=0.3, beta=2, scale=True, scale_mean=0., scale_v=0.7,
                       seed=None, device=None, shard=None, dtype=np.int64, out="numpy",
-                      sampler=DEFAULT_SAMPLER):
+                      sampler=DEFAULT_SAMPLER, *, path=None):
     """Every tree position sampled n_factor times (simulation.py:474-517)."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
@@ -569,7 +575,7 @@ def sample_whole_tree(tree, n_factor, alpha=0.3, beta=2, scale=True, scale_mean=
              nat.ptr(tables.d("cover_row")), len(tables.cover_pt), int(n_factor), lo, n,
              nat.ptr(pt), nat.ptr(codes), nat.ptr(rows), nat.stream_ptr(dev))
     return _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
-                           seed, lo, dev, dtype, out, sampler)
+                           seed, lo, dev, dtype, out, sampler, path=path)
 
 
 def draw_times(timepoint, no_cells, max_time, var=4, seed=None, first=0, device=None,
@@ -591,7 +597,7 @@ def draw_times(timepoint, no_cells, max_time, var=4, seed=None, first=0, device=
 
 def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, beta=2, scale=True,
                              scale_mean=0, scale_v=0.7, seed=None, device=None, shard=None,
-                             dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER):
+                             dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, *, path=None):
     """Time-series experiment: normally distributed pseudotimes around each sample point,
     branches picked by density (simulation.py:319-379)."""
     dev = nat.device(device)
@@ -617,23 +623,23 @@ def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, b
         nat.call("pst_times_from_normals", nat.ptr(z), n, int(max_time), nat.ptr(pt), st)
     return _sample_data_at_times(tree, pt, alpha=alpha, beta=beta, scale=scale, scale_mean=scale_mean,
                                  scale_v=scale_v, seed=nat.derive_seed(seed, 3), device=dev,
-                                 dtype=dtype, out=out, sampler=sampler, _first=lo)
+                                 dtype=dtype, out=out, sampler=sampler, _first=lo, path=path)
 
 
 def sample_whole_tree_restricted(tree, alpha=0.2, beta=3, seed=None, device=None, dtype=np.int64,
-                                 out="numpy", sampler=DEFAULT_SAMPLER):
+                                 out="numpy", sampler=DEFAULT_SAMPLER, *, path=None):
     """Bare-bones run with default lineage parameters (simulation.py:289-316): one cell
     per pseudotime value, random branch, per-gene alpha/beta around the given means."""
     sample_time = np.arange(0, tree.get_max_time())
     tree.default_gene_expression()
     alphas, betas = cm.generate_negbin_params(tree, mean_alpha=alpha, mean_beta=beta)
     return _sample_data_at_times(tree, sample_time, alpha=alphas, beta=betas, seed=seed,
-                                 device=device, dtype=dtype, out=out, sampler=sampler)
+                                 device=device, dtype=dtype, out=out, sampler=sampler, path=path)
 
 
 def _sample_data_at_times(tree, sample_pt, branches=None, alpha=0.3, beta=2, scale=True,
                           scale_mean=0., scale_v=0.7, seed=None, device=None, dtype=np.int64,
-                          out="numpy", sampler=DEFAULT_SAMPLER, _first=0):
+                          out="numpy", sampler=DEFAULT_SAMPLER, _first=0, path=None):
     """Cells at given pseudotimes (simulation.py:551-599): pick branches if they are not
     supplied, draw library sizes, draw counts.  `_first` is the global index of the first
     cell (sharded callers)."""
@@ -652,7 +658,7 @@ def _sample_data_at_times(tree, sample_pt, branches=None, alpha=0.3, beta=2, sca
     # the index map's own status word is read after the draw has been queued (no stall in front of it)
     try:
         result = _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
-                                 seed, _first, dev, dtype, out, sampler)
+                                 seed, _first, dev, dtype, out, sampler, path=path)
     except IndexError:
         sut.check_flags(flags)
         raise
@@ -675,12 +681,13 @@ def _rows_for(tables, pt, branches, dev):
 
 
 def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, device=None,
-                dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, first=0):
+                dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, first=0, *, path=None):
     """UMI counts of cells at (pseudotime, branch) with library sizes `scalings`
     (simulation.py:602-651): X[n,g] ~ NB(mean = means[branch_n][t_n - start, g]*scaling_n,
-    variance = alpha_g mean^2 + beta_g mean)."""
+    variance = alpha_g mean^2 + beta_g mean).  out="csr", path=p writes the CSR shard with the
+    pseudotime, branches and scalings given here and returns its memory-mapped matrix."""
     dev = nat.device(device)
-    _check_csr_request(out, dtype)
+    _check_csr_request(out, dtype, path=path)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
     pt = pseudotime if isinstance(pseudotime, torch.Tensor) else \
@@ -693,7 +700,11 @@ def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, de
     if np.ndim(beta) == 0:
         beta = [beta] * tree.G
     engine = CountEngine(tree, tables, alpha, beta, dev, sampler=sampler)
-    return _sample_counts(engine, rows, s32, seed, first, dtype, out)
+    cells = None
+    if path is not None:
+        given = scalings.detach().cpu().numpy() if isinstance(scalings, torch.Tensor) else scalings
+        cells = pt.cpu().numpy(), tables.branch_names(codes.cpu().numpy()), np.asarray(given, dtype=np.float64)
+    return _sample_counts(engine, rows, s32, seed, first, dtype, out, path=path, cells=cells)
 
 
 def add_non_diff_genes(inform_expr_matrix, genes, gene_params, cell_scalings, seed=None,
