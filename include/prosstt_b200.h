@@ -263,8 +263,9 @@ int pst_csr_row_offsets(const int32_t *row_nnz, int64_t n, int64_t *indptr, void
 /* Pass 2 of out="csr": pst_csr_fill for a chunk of rows, writing narrow streams into a window.
  * indptr holds the chunk's n+1 GLOBAL row offsets (from pst_csr_row_offsets); nonzero number p
  * (indptr[0] <= p < indptr[n]) goes to indices[p - base] and data[p - base], columns ascending in
- * each row.  index_bits 16 (uint16, needs G <= 65536) or 32 (int32).  data_bits 32: exact int32
- * values; data_bits 16: uint16 min(v, 65535), and every v >= 65535 is also listed as
+ * each row.  index_bits 16 (uint16, needs G <= 65536), 32 (int32) or 64 (int64).  data_bits 32 / 64:
+ * exact int32 / int64 values (64-bit widths pair with 32- or 64-bit ones: the final bytes of a file's
+ * indices and data, no re-pack); data_bits 16: uint16 min(v, 65535), and every v >= 65535 is also listed as
  * (ovf_pos = p, ovf_value = v), appended at atomicAdd(ovf_count, 1) when that slot is < ovf_cap
  * (ovf_count keeps counting past the cap; pst_csr_row_counts' sat_count is the exact size needed).
  * Sets PST_FLAG_ROW in flags[0] if a row's nonzeros do not match indptr (nothing is written past
@@ -273,6 +274,34 @@ int pst_csr_pack(const int32_t *X, int64_t n, int64_t G, int64_t ldx, const int6
                  int64_t base, void *indices, int32_t index_bits, void *data, int32_t data_bits,
                  int64_t *ovf_pos, int32_t *ovf_value, int64_t ovf_cap, uint64_t *ovf_count,
                  uint32_t *flags, void *stream);
+
+/* The indptr member of a streamed CSR file, one chunk at a time: out[i] = *running + indptr[i+1] for
+ * i < n, as int32 (out_bits 32) or int64 (64), then *running += indptr[n].  indptr: the chunk's local
+ * row pointer (n+1 entries from 0, pst_csr_row_offsets); running: one device int64 the caller zeroes
+ * before the first chunk.  The file's leading 0 is not written here. */
+int pst_csr_indptr_bytes(const int64_t *indptr, int64_t n, int64_t *running, void *out, int32_t out_bits,
+                         void *stream);
+
+/* ---- raw DEFLATE (RFC 1951) on the device: the compressed CSR file (pst_deflate.cu) ---------------
+ * The input is cut into blocks of `block` bytes (a multiple of 1024, at most 32768).  Each block becomes
+ * one dynamic-Huffman block over the literals 0-255 and end-of-block (no length or distance codes; the
+ * one distance code has length 1), followed by an empty stored block (zlib's Z_SYNC_FLUSH marker
+ * 00 00 FF FF), so it ends on a byte boundary; a block whose Huffman form is not smaller is one stored
+ * block.  No block is final: append 03 00 (an empty final fixed block) to end the stream, and any
+ * concatenation of such outputs is one stream.  Codes are at most 15 bits, deterministic for given
+ * bytes.
+ * Input length: (*count) * scale bytes when count (a device int64) is not NULL, else max_bytes; it is
+ * clamped to max_bytes, which sizes the launch, so a length made on the device needs no host read.
+ * out (device, pst_deflate_bound(max_bytes, block) bytes) receives the blocks back to back, *out_bytes
+ * (device int64) their size and *crc (device) the CRC-32 of the input (zlib.crc32).  work: device
+ * workspace of pst_deflate_workspace_bytes(max_bytes, block) bytes. */
+int64_t pst_deflate_bound(int64_t n, int32_t block);
+int64_t pst_deflate_workspace_bytes(int64_t n, int32_t block);
+int pst_deflate_blocks(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes, int32_t block,
+                       void *out, int64_t *out_bytes, uint32_t *crc, void *work, int64_t work_bytes,
+                       void *stream);
+/* *crc = CRC-32 (zlib.crc32) of the n device bytes at in; crc is a device word. */
+int pst_crc32(const void *in, int64_t n, uint32_t *crc, void *stream);
 
 /* Narrow transfer formats for the device->host path (PCIe is the bound at 4 B per count):
  * out[i][g] = min(X[i][g], SAT) as uint8 (out_bits 8, SAT 255) or uint16 (out_bits 16, SAT 65535),
@@ -319,6 +348,8 @@ int pst_host_apply_overflow(void *h_dst, int32_t dst_bits, int64_t base, int64_t
 /* sum of the buffer read as uint32 words: the cheapest consumer that touches every byte (the sink
  * of the streamed many-cells benchmark; a transfer checksum). */
 uint64_t pst_host_checksum(const void *h_src, int64_t bytes, int32_t threads);
+/* zlib's crc32_combine: the CRC-32 of A || B from crc1 = crc32(A), crc2 = crc32(B) and len2 = |B|. */
+uint32_t pst_host_crc32_combine(uint32_t crc1, uint32_t crc2, int64_t len2);
 
 #if defined(__GNUC__)
 #pragma GCC visibility pop

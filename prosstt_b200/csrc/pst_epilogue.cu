@@ -258,6 +258,21 @@ narrow_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx, 
   }
 }
 
+// ---------------------------------------------------------------------------------------------
+// The indptr member of a streamed CSR file: out[i] = *running + indptr[i + 1] (i < n) in the index dtype,
+// then *running += indptr[n].  indptr is a chunk's local row pointer (indptr[0] = 0), so the chunks'
+// outputs concatenate, after the file's leading 0, to the whole matrix's row pointer.  One CTA: the
+// running total is read before and written after every thread's stores.
+// ---------------------------------------------------------------------------------------------
+template <typename OUT>
+__global__ void __launch_bounds__(1024)
+csr_indptr_kernel(const int64_t *__restrict__ indptr, int64_t n, int64_t *__restrict__ running, OUT *__restrict__ out) {
+  const int64_t base = *running;
+  for (int64_t i = threadIdx.x; i < n; i += blockDim.x) out[i] = (OUT)(base + indptr[i + 1]);
+  __syncthreads();
+  if (threadIdx.x == 0) *running = base + indptr[n];
+}
+
 // Pure-store kernel: the write-only HBM ceiling the count write is measured against (SURVEY.md 8d).  Same
 // shape of traffic as the sampler's output: 128-bit stores, 512 contiguous bytes per warp instruction.
 __global__ void __launch_bounds__(256) store_fill_kernel(int4 *__restrict__ out, int64_t n16, int32_t value) {
@@ -360,13 +375,15 @@ extern "C" int pst_csr_pack(const int32_t *X, int64_t n, int64_t G, int64_t ldx,
   const char *fn = "pst_csr_pack";
   PST_REQUIRE(n >= 0 && G >= 0 && ldx >= G && base >= 0 && ovf_cap >= 0, fn,
               "need n, G, base, ovf_cap >= 0 and ldx >= G");
-  PST_REQUIRE(index_bits == 16 || index_bits == 32, fn, "index_bits must be 16 or 32");
-  PST_REQUIRE(data_bits == 16 || data_bits == 32, fn, "data_bits must be 16 or 32");
-  PST_REQUIRE(index_bits == 32 || G <= 65536, fn, "16-bit column indices need G <= 65536");
+  PST_REQUIRE(index_bits == 16 || index_bits == 32 || index_bits == 64, fn, "index_bits must be 16, 32 or 64");
+  PST_REQUIRE(data_bits == 16 || data_bits == 32 || data_bits == 64, fn, "data_bits must be 16, 32 or 64");
+  PST_REQUIRE((index_bits < 64 && data_bits < 64) || (index_bits >= 32 && data_bits >= 32), fn,
+              "64-bit widths go with 32- or 64-bit widths");
+  PST_REQUIRE(index_bits != 16 || G <= 65536, fn, "16-bit column indices need G <= 65536");
   PST_REQUIRE(G < ((int64_t)1 << 31), fn, "column index does not fit int32");
   if (n == 0 || G == 0) return 0;
   PST_REQUIRE(X && indptr && indices && data && flags, fn, "null pointer");
-  PST_REQUIRE(data_bits == 32 || (ovf_count && (ovf_cap == 0 || (ovf_pos && ovf_value))), fn,
+  PST_REQUIRE(data_bits != 16 || (ovf_count && (ovf_cap == 0 || (ovf_pos && ovf_value))), fn,
               "16-bit values need the overflow list");
   const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
   const unsigned grid = stream_grid(n * 32);
@@ -384,7 +401,10 @@ extern "C" int pst_csr_pack(const int32_t *X, int64_t n, int64_t G, int64_t ldx,
   if (index_bits == 16 && data_bits == 16) PST_LAUNCH_PACK(uint16_t, uint16_t, true);
   else if (index_bits == 32 && data_bits == 16) PST_LAUNCH_PACK(int32_t, uint16_t, true);
   else if (index_bits == 16) PST_LAUNCH_PACK(uint16_t, int32_t, false);
-  else PST_LAUNCH_PACK(int32_t, int32_t, false);
+  else if (index_bits == 32 && data_bits == 32) PST_LAUNCH_PACK(int32_t, int32_t, false);
+  else if (index_bits == 32) PST_LAUNCH_PACK(int32_t, int64_t, false);
+  else if (data_bits == 32) PST_LAUNCH_PACK(int64_t, int32_t, false);
+  else PST_LAUNCH_PACK(int64_t, int64_t, false);
 #undef PST_LAUNCH_PACK
   return check_launch(fn);
 }
@@ -411,5 +431,17 @@ extern "C" int pst_narrow_counts(const int32_t *X, int64_t n, int64_t G, int64_t
   if (out_bits == 8) { if (vec) PST_LAUNCH_NARROW(uint8_t, true); else PST_LAUNCH_NARROW(uint8_t, false); }
   else { if (vec) PST_LAUNCH_NARROW(uint16_t, true); else PST_LAUNCH_NARROW(uint16_t, false); }
 #undef PST_LAUNCH_NARROW
+  return check_launch(fn);
+}
+
+extern "C" int pst_csr_indptr_bytes(const int64_t *indptr, int64_t n, int64_t *running, void *out, int32_t out_bits,
+                                    void *stream) {
+  const char *fn = "pst_csr_indptr_bytes";
+  PST_REQUIRE(n >= 0, fn, "need n >= 0");
+  PST_REQUIRE(out_bits == 32 || out_bits == 64, fn, "out_bits must be 32 or 64");
+  PST_REQUIRE(indptr && running && (n == 0 || out), fn, "null pointer");
+  cudaStream_t st = (cudaStream_t)stream;
+  if (out_bits == 32) csr_indptr_kernel<int32_t><<<1, 1024, 0, st>>>(indptr, n, running, (int32_t *)out);
+  else csr_indptr_kernel<int64_t><<<1, 1024, 0, st>>>(indptr, n, running, (int64_t *)out);
   return check_launch(fn);
 }

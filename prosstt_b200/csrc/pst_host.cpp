@@ -250,3 +250,28 @@ extern "C" uint64_t pst_host_checksum(const void *src, int64_t bytes, int32_t th
   for (uint64_t v : part) total += v;
   return total;
 }
+
+// zlib's crc32_combine: the CRC-32 of A || B from crc32(A), crc32(B) and |B| (products in GF(2) modulo the
+// CRC polynomial, x^(8 |B|) by squaring); the compressed CSR file's members are CRC-ed chunk by chunk on the
+// device.
+namespace {
+uint32_t crc_multmodp(uint32_t a, uint32_t b) {
+  uint32_t p = 0;
+  for (uint32_t m = 1u << 31; m != 0; m >>= 1) {
+    if (a & m) p ^= b;
+    b = (b & 1) ? (b >> 1) ^ 0xEDB88320u : b >> 1;
+  }
+  return p;
+}
+}  // namespace
+
+extern "C" uint32_t pst_host_crc32_combine(uint32_t crc1, uint32_t crc2, int64_t len2) {
+  if (len2 <= 0) return crc1 ^ crc2;
+  uint32_t x2n = 1u << 30, p = 1u << 31;             // x^(2^k) for k = 0, and x^0
+  for (int k = 0; k < 3; ++k) x2n = crc_multmodp(x2n, x2n);   // x^8: one byte
+  for (uint64_t n = (uint64_t)len2; n; n >>= 1) {
+    if (n & 1) p = crc_multmodp(x2n, p);
+    x2n = crc_multmodp(x2n, x2n);
+  }
+  return crc_multmodp(p, crc1) ^ crc2;
+}

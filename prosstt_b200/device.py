@@ -217,6 +217,7 @@ _NP_TO_TORCH = {np.dtype(np.int32): torch.int32, np.dtype(np.int64): torch.int64
                 np.dtype(np.uint16): torch.uint16, np.dtype(np.uint8): torch.uint8}
 _STAGE_BYTES = int(os.environ.get("PST_STAGE_MB", "256")) << 20   # one pinned staging buffer (two per device)
 _STAGING = {}
+_DEFLATE_BLOCK = 32768                        # bytes per DEFLATE block of the compressed CSR file (at most 32 KiB)
 
 
 _AUTO_STATE = {"narrow_overflowed": False}     # an automatically chosen uint8 transport overflowed its list once
@@ -592,7 +593,7 @@ class CountEngine(object):
         return indptr, indices, data
 
     def stream_csr(self, rows, scaling32, seed, cell0, consume, index_dtype=np.int64, data_dtype=np.int64,
-                   chunk_cells=None, threads=0, overflow_cap=None):
+                   chunk_cells=None, threads=0, overflow_cap=None, compress=False):
         """Sample the cells in chunks and hand each one as CSR to consume(lo, hi, indptr, indices, data), on a
         worker thread, once per chunk, in cell order.  indptr is chunk-local int64 (hi - lo + 1 entries from 0);
         indices and data are the chunk's nonzeros in `index_dtype` / `data_dtype` (int32 or int64), columns
@@ -608,7 +609,18 @@ class CountEngine(object):
         (_copy_chunks' collect).  Only then are chunk i's copies queued, sized to its nnz: 4 B per nonzero
         over PCIe while G <= 65536.  A chunk with more saturated values than its list holds (overflow_cap
         entries at first) grows the list and is packed again from its work buffer, which survives until chunk
-        i+2 is drawn.  An error in the status word raises as draw() would (raise_flags) and ends the stream."""
+        i+2 is drawn.  An error in the status word raises as draw() would (raise_flags) and ends the stream.
+
+        compress=True: consume(lo, hi, parts) receives the chunk compressed instead, parts = [(member,
+        compressed, crc, raw_len)] for "indptr", "indices" and "data" in the order formats.CsrNpzWriter.append
+        takes them: `compressed` (a reused uint8 host buffer) is raw DEFLATE that decompresses to the raw_len
+        bytes of the member's part, whose CRC-32 is crc.  indptr is the chunk's row ends in index_dtype, offset
+        by the nonzeros of the chunks before it (the file's leading 0 is not included).  The device does all of
+        it, on the sampling stream and with no host wait: pst_csr_pack writes the final index_dtype /
+        data_dtype bytes (no saturation, no re-pack), pst_csr_indptr_bytes the indptr bytes with a running nnz
+        kept on the device, and pst_deflate_blocks compresses each member, reading its length from the device.
+        The host reads (nnz, status word, compressed sizes, CRCs) one chunk late as above and copies exactly
+        the compressed bytes."""
         index_dtype, data_dtype = np.dtype(index_dtype), np.dtype(data_dtype)
         for what, dt in (("indices", index_dtype), ("data", data_dtype)):
             if dt not in (np.dtype(np.int32), np.dtype(np.int64)):
@@ -619,87 +631,152 @@ class CountEngine(object):
         if n == 0:
             return 0
         if G == 0:
-            consume(0, n, np.zeros(n + 1, np.int64), np.zeros(0, index_dtype), np.zeros(0, data_dtype))
+            if compress:
+                from prosstt_b200.formats import sync_deflate
+                consume(0, n, [("indptr",) + sync_deflate(np.zeros(n, index_dtype).tobytes()),
+                               ("indices",) + sync_deflate(b""), ("data",) + sync_deflate(b"")])
+            else:
+                consume(0, n, np.zeros(n + 1, np.int64), np.zeros(0, index_dtype), np.zeros(0, data_dtype))
             return 0
         ibits = 16 if G <= 65536 else 32                 # width of the column stream
         ibytes = ibits // 8
-        chunk, bounds = _plan_chunks(n, chunk_cells, (ibytes + 2) * G, _STAGE_BYTES)
-        value_at = (chunk * G * ibytes + 63) // 64 * 64  # the value stream, after the worst-case column stream
+        if compress:
+            isz, dsz = index_dtype.itemsize, data_dtype.itemsize
+            # the wide streams of a chunk and their compressed form, bounded by about as many bytes again
+            chunk, bounds = _plan_chunks(n, chunk_cells, 2 * (isz + dsz) * G, _STAGE_BYTES)
+        else:
+            chunk, bounds = _plan_chunks(n, chunk_cells, (ibytes + 2) * G, _STAGE_BYTES)
         st = nat.stream_ptr(dev)
         work = [torch.empty((chunk, G), dtype=torch.int32, device=dev) for _ in range(2)]
-        stage = [torch.empty(value_at + 2 * chunk * G, dtype=torch.uint8, device=dev) for _ in range(2)]
         row_nnz = torch.empty(chunk, dtype=torch.int32, device=dev)      # read by the scan right after the count
         indptr = [torch.empty(chunk + 1, dtype=torch.int64, device=dev) for _ in range(2)]
-        info = torch.zeros((2, 3), dtype=torch.int64, device=dev)        # saturated, nnz, status word
-        info_host = torch.zeros((2, 3), dtype=torch.int64).pin_memory()
+        # saturated, nnz, status word; compress: the three compressed sizes and CRCs
+        info = torch.zeros((2, 9), dtype=torch.int64, device=dev)
+        info_host = torch.zeros((2, 9), dtype=torch.int64).pin_memory()
         sized = [None, None]
-        ovf = [_OverflowList(overflow_cap or (1 << 16), dev) for _ in range(2)]
-        ovf_host = [torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory() for k in range(2)]
         pack_flags = torch.zeros(1, dtype=torch.int32, device=dev)
-        # host side: the row pointer, then the streams of the nonzeros, values on a 64-byte boundary
-        stage_host = _pinned_staging(dev, 8 * (chunk + 1) + value_at + 64 + 2 * chunk * G)
-        # the widened chunk, reused from chunk to chunk: its pages are touched as the chunks' nnz needs them and
-        # hostpool keeps them mapped for the next call.  Past the first chunk they are mapped and out of cache,
-        # which is what the streaming stores are for.
-        indices_w = hostpool.result_array((chunk * G,), index_dtype)[0]
-        data_w = hostpool.result_array((chunk * G,), data_dtype)[0]
-        lib = nat.load()
-        widen_i = widen_d = lib.pst_host_widen_stream
         total = [0]
 
-        def pack(k, cells):
-            ovf[k].count.zero_()
-            nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, stage[k].data_ptr(), ibits,
-                     stage[k].data_ptr() + value_at, 16, *ovf[k].kernel_args, pack_flags, st)
-
-        def produce(k, lo, hi):
+        def draw_rows(k, lo, hi):
+            """Chunk [lo, hi) into work buffer k and its chunk-local row pointer into indptr[k]."""
             cells = hi - lo
             self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[k][:cells])
             info[k].zero_()
             nat.call("pst_csr_row_counts", work[k].data_ptr(), cells, G, G, row_nnz, info[k, 0], st)
             nat.call("pst_csr_row_offsets", row_nnz, cells, indptr[k], st)
-            pack(k, cells)
+
+        def record(k, cells):
             info[k, 1].copy_(indptr[k][cells])
             info[k, 2].copy_(self.flags[0])
             info_host[k].copy_(info[k], non_blocking=True)
             sized[k] = torch.cuda.Event()
             sized[k].record(torch.cuda.current_stream(dev))
 
-        def collect(k, lo, hi):
+        def read_info(k):
             sized[k].synchronize()
-            n_sat, nnz, word = info_host[k].tolist()
-            if word:
+            vals = info_host[k].tolist()
+            if vals[2]:
                 self.flags[0].zero_()
-                raise_flags(word)
-            cells = hi - lo
-            if n_sat > ovf[k].capacity:
-                ovf[k] = _OverflowList(max(n_sat, 2 * ovf[k].capacity), dev)
-                ovf_host[k] = torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory()
-                pack(k, cells)
-                torch.cuda.current_stream(dev).synchronize()   # the copies wait for the first pack only
-            total[0] += nnz
-            at = 8 * (cells + 1)
-            vat = (at + nnz * ibytes + 63) // 64 * 64
-            h = stage_host[k]
-            pairs = [(indptr[k][:cells + 1].view(torch.uint8), h[:at]),
-                     (stage[k][:nnz * ibytes], h[at:at + nnz * ibytes]),
-                     (stage[k][value_at:value_at + 2 * nnz], h[vat:vat + 2 * nnz])]
-            if n_sat:
-                pairs += [(ovf[k].pos[:n_sat].view(torch.uint8), ovf_host[k][:8 * n_sat]),
-                          (ovf[k].value[:n_sat].view(torch.uint8), ovf_host[k][8 * n_sat:12 * n_sat])]
-            return pairs
+                raise_flags(vals[2])
+            total[0] += vals[1]
+            return vals
 
-        def landed(dsts, lo, hi):
-            nnz = dsts[1].numel() // ibytes
-            indices, data = indices_w[:nnz], data_w[:nnz]
-            rc = widen_i(dsts[1].data_ptr(), ibits, indices.ctypes.data, 8 * index_dtype.itemsize, nnz, int(threads))
-            rc |= widen_d(dsts[2].data_ptr(), 16, data.ctypes.data, 8 * data_dtype.itemsize, nnz, int(threads))
-            if rc != 0:
-                raise nat.NativeError("pst_host_widen failed")
-            if len(dsts) > 3:
-                lib.pst_host_apply_overflow(data.ctypes.data, 8 * data_dtype.itemsize, 0, nnz, dsts[3].data_ptr(),
-                                            dsts[4].data_ptr(), dsts[3].numel() // 8)
-            consume(lo, hi, dsts[0].numpy().view(np.int64), indices, data)
+        if compress:
+            lib = nat.load()
+            block = _DEFLATE_BLOCK
+            wide = [torch.empty(max(1, chunk * isz), dtype=torch.uint8, device=dev),       # indptr, indices, data
+                    torch.empty(max(1, chunk * G * isz), dtype=torch.uint8, device=dev),
+                    torch.empty(max(1, chunk * G * dsz), dtype=torch.uint8, device=dev)]
+            bound = [int(lib.pst_deflate_bound(w.numel(), block)) for w in wide]
+            packed = [[torch.empty(b, dtype=torch.uint8, device=dev) for b in bound] for _ in range(2)]
+            dwork_bytes = max(int(lib.pst_deflate_workspace_bytes(w.numel(), block)) for w in wide)
+            dwork = torch.empty(dwork_bytes, dtype=torch.uint8, device=dev)
+            running = torch.zeros(1, dtype=torch.int64, device=dev)     # nonzeros of the chunks before
+            stage_host = _pinned_staging(dev, sum(bound) + 3 * 64)
+            meta_host = [torch.empty(9 * 8, dtype=torch.uint8).pin_memory() for _ in range(2)]
+            members = ("indptr", "indices", "data")
+
+            def produce(k, lo, hi):
+                cells = hi - lo
+                draw_rows(k, lo, hi)
+                nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, wide[1], 8 * isz, wide[2],
+                         8 * dsz, None, None, 0, None, pack_flags, st)
+                nat.call("pst_csr_indptr_bytes", indptr[k], cells, running, wide[0], 8 * isz, st)
+                nnz = indptr[k][cells:cells + 1]
+                for j, (count, scale, most) in enumerate(((None, 0, cells * isz), (nnz, isz, cells * G * isz),
+                                                          (nnz, dsz, cells * G * dsz))):
+                    nat.call("pst_deflate_blocks", wide[j], count, scale, most, block, packed[k][j], info[k, 3 + j],
+                             info[k, 6 + j].data_ptr(), dwork, dwork_bytes, st)   # the CRC: low word of a zeroed int64
+                record(k, cells)
+
+            def collect(k, lo, hi):
+                sizes = read_info(k)[3:6]
+                pairs, at = [], 0
+                for j in range(3):
+                    pairs.append((packed[k][j][:sizes[j]], stage_host[k][at:at + sizes[j]]))
+                    at = (at + sizes[j] + 63) // 64 * 64
+                return pairs + [(info[k].view(torch.uint8), meta_host[k])]
+
+            def landed(dsts, lo, hi):
+                vals = dsts[3].view(torch.int64).tolist()
+                raw = ((hi - lo) * isz, vals[1] * isz, vals[1] * dsz)
+                consume(lo, hi, [(members[j], dsts[j].numpy(), vals[6 + j] & 0xFFFFFFFF, raw[j]) for j in range(3)])
+        else:
+            value_at = (chunk * G * ibytes + 63) // 64 * 64  # the value stream, after the worst-case column stream
+            stage = [torch.empty(value_at + 2 * chunk * G, dtype=torch.uint8, device=dev) for _ in range(2)]
+            ovf = [_OverflowList(overflow_cap or (1 << 16), dev) for _ in range(2)]
+            ovf_host = [torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory() for k in range(2)]
+            # host side: the row pointer, then the streams of the nonzeros, values on a 64-byte boundary
+            stage_host = _pinned_staging(dev, 8 * (chunk + 1) + value_at + 64 + 2 * chunk * G)
+            # the widened chunk, reused from chunk to chunk: its pages are touched as the chunks' nnz needs them
+            # and hostpool keeps them mapped for the next call.  Past the first chunk they are mapped and out of
+            # cache, which is what the streaming stores are for.
+            indices_w = hostpool.result_array((chunk * G,), index_dtype)[0]
+            data_w = hostpool.result_array((chunk * G,), data_dtype)[0]
+            lib = nat.load()
+            widen_i = widen_d = lib.pst_host_widen_stream
+
+            def pack(k, cells):
+                ovf[k].count.zero_()
+                nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, stage[k].data_ptr(), ibits,
+                         stage[k].data_ptr() + value_at, 16, *ovf[k].kernel_args, pack_flags, st)
+
+            def produce(k, lo, hi):
+                draw_rows(k, lo, hi)
+                pack(k, hi - lo)
+                record(k, hi - lo)
+
+            def collect(k, lo, hi):
+                n_sat, nnz = read_info(k)[:2]
+                cells = hi - lo
+                if n_sat > ovf[k].capacity:
+                    ovf[k] = _OverflowList(max(n_sat, 2 * ovf[k].capacity), dev)
+                    ovf_host[k] = torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory()
+                    pack(k, cells)
+                    torch.cuda.current_stream(dev).synchronize()   # the copies wait for the first pack only
+                at = 8 * (cells + 1)
+                vat = (at + nnz * ibytes + 63) // 64 * 64
+                h = stage_host[k]
+                pairs = [(indptr[k][:cells + 1].view(torch.uint8), h[:at]),
+                         (stage[k][:nnz * ibytes], h[at:at + nnz * ibytes]),
+                         (stage[k][value_at:value_at + 2 * nnz], h[vat:vat + 2 * nnz])]
+                if n_sat:
+                    pairs += [(ovf[k].pos[:n_sat].view(torch.uint8), ovf_host[k][:8 * n_sat]),
+                              (ovf[k].value[:n_sat].view(torch.uint8), ovf_host[k][8 * n_sat:12 * n_sat])]
+                return pairs
+
+            def landed(dsts, lo, hi):
+                nnz = dsts[1].numel() // ibytes
+                indices, data = indices_w[:nnz], data_w[:nnz]
+                rc = widen_i(dsts[1].data_ptr(), ibits, indices.ctypes.data, 8 * index_dtype.itemsize, nnz,
+                             int(threads))
+                rc |= widen_d(dsts[2].data_ptr(), 16, data.ctypes.data, 8 * data_dtype.itemsize, nnz, int(threads))
+                if rc != 0:
+                    raise nat.NativeError("pst_host_widen failed")
+                if len(dsts) > 3:
+                    lib.pst_host_apply_overflow(data.ctypes.data, 8 * data_dtype.itemsize, 0, nnz, dsts[3].data_ptr(),
+                                                dsts[4].data_ptr(), dsts[3].numel() // 8)
+                consume(lo, hi, dsts[0].numpy().view(np.int64), indices, data)
 
         self._copy_chunks(bounds, produce, landed, collect)
         if int(pack_flags.item()) != 0:

@@ -17,10 +17,21 @@ added, both readable without this package:
   int64, `branches`, `scalings` float64).  `np.load(..., mmap_mode="r")` reads every member, and
   the CSR members zipped uncompressed (ZIP_STORED) form a file `scipy.sparse.load_npz` reads.
   `load_csr_shard` maps it back without a copy.
+* compressed CSR files (`CsrNpzWriter`, written by `out="csr", path=..., compress=True`): one zip64
+  `.npz` whose members are the same `.npy` files, each DEFLATE-compressed (the format
+  `np.savez_compressed` writes), so `scipy.sparse.load_npz(path)` and `np.load(path)` read it.  The
+  GPU compresses each chunk's indptr, indices and data (pst_deflate_blocks: Huffman-only blocks ended by
+  a sync-flush marker, concatenated), so only compressed bytes cross PCIe and reach the disk.  The file
+  cannot be memory-mapped: the call returns a `CompressedCsr` record, and `load_csr_shard` decompresses
+  it into memory.
 """
+import collections
 import errno
+import io
 import os
 import shutil
+import struct
+import zlib
 
 import numpy as np
 import torch
@@ -154,7 +165,8 @@ class NpyShardWriter(object):
 
 
 def shard_path(stem, rank, world, suffix=".npy"):
-    """`<stem><suffix>` for one rank, `<stem>.rank<k>of<w><suffix>` otherwise (suffix ".csr" for CSR shards)."""
+    """`<stem><suffix>` for one rank, `<stem>.rank<k>of<w><suffix>` otherwise (suffix ".csr" for CSR shards,
+    ".npz" for compressed CSR files)."""
     return "%s%s" % (stem, suffix) if world == 1 else "%s.rank%dof%d%s" % (stem, rank, world, suffix)
 
 
@@ -168,6 +180,28 @@ def _csr_matrix(indptr, indices, data, shape):
     m.has_sorted_indices = True
     m.has_canonical_format = True
     return m
+
+
+def _csr_cells(n, pseudotime, branches, scalings):
+    """The cell annotations of a CSR shard or file, checked to hold one value per cell."""
+    branches = np.asarray(branches)
+    if branches.dtype.kind == "O":                       # readable without pickle
+        branches = branches.astype(str)
+    cells = dict(pseudotime=np.asarray(pseudotime, dtype=np.int64), branches=branches,
+                 scalings=np.asarray(scalings, dtype=np.float64))
+    for name, a in cells.items():
+        if a.shape != (n,):
+            raise ValueError("%s must hold one value per cell (%d), not shape %s" % (name, n, a.shape))
+    return cells
+
+
+def _csr_dtypes(shape, dtype):
+    """(index dtype, data dtype) of a CSR shard or file: int32 indices when n_cells x G < 2^31."""
+    dtype = np.dtype(dtype)
+    if dtype not in (np.dtype(np.int32), np.dtype(np.int64)):
+        raise ValueError("CSR data must be int32 or int64, not %s" % dtype)
+    n, G = shape
+    return (np.dtype(np.int32) if n * G < (1 << 31) else np.dtype(np.int64)), dtype
 
 
 class CsrShardWriter(object):
@@ -188,18 +222,8 @@ class CsrShardWriter(object):
             raise FileExistsError(errno.EEXIST, "the CSR shard exists already", self.path)
         n, G = (int(v) for v in shape)
         self.shape = (n, G)
-        self.dtype = np.dtype(dtype)
-        if self.dtype not in (np.dtype(np.int32), np.dtype(np.int64)):
-            raise ValueError("CSR data must be int32 or int64, not %s" % self.dtype)
-        self.index_dtype = np.dtype(np.int32) if n * G < (1 << 31) else np.dtype(np.int64)
-        branches = np.asarray(branches)
-        if branches.dtype.kind == "O":                   # readable without pickle
-            branches = branches.astype(str)
-        cells = dict(pseudotime=np.asarray(pseudotime, dtype=np.int64), branches=branches,
-                     scalings=np.asarray(scalings, dtype=np.float64))
-        for name, a in cells.items():
-            if a.shape != (n,):
-                raise ValueError("%s must hold one value per cell (%d), not shape %s" % (name, n, a.shape))
+        self.index_dtype, self.dtype = _csr_dtypes(self.shape, dtype)
+        cells = _csr_cells(n, pseudotime, branches, scalings)
         self.rows, self.nnz = 0, 0
         self._dir = self.path + ".partial"
         if os.path.lexists(self._dir):                  # left behind by an interrupted writer
@@ -286,9 +310,246 @@ class CsrShardWriter(object):
         return False
 
 
+def sync_deflate(raw):
+    """(bytes, crc32, len) of `raw` compressed as zlib's non-final, sync-flushed raw DEFLATE blocks: the unit
+    CsrNpzWriter.append takes (what pst_deflate_blocks makes on the device)."""
+    c = zlib.compressobj(6, zlib.DEFLATED, -15)
+    raw = bytes(raw)
+    return c.compress(raw) + c.flush(zlib.Z_SYNC_FLUSH), zlib.crc32(raw), len(raw)
+
+
+class CompressedCsr(collections.namedtuple("CompressedCsr", "path shape nnz dtype index_dtype nbytes")):
+    """The X of a `compress=True` call: a compressed CSR file on disk, not loaded (it cannot be memory-mapped).
+    nbytes is the file's size; load() decompresses it (scipy.sparse.load_npz)."""
+    __slots__ = ()
+
+    def load(self):
+        import scipy.sparse as sp
+        return sp.load_npz(self.path)
+
+
+_ZIP_DATE, _ZIP_TIME = (0 << 9) | (1 << 5) | 1, 0       # fixed timestamp 1980-01-01 00:00: identical files
+_ZIP64 = 45                                            # version needed to extract zip64 entries
+_NPY_STORED = 5                                        # stored-block header in front of a member's .npy header
+_FINAL_BLOCK = b"\x03\x00"                            # empty final block (fixed Huffman, end-of-block)
+
+
+def _npy_header(dtype, length):
+    buf = io.BytesIO()
+    np.lib.format.write_array_header_1_0(buf, {"descr": np.lib.format.dtype_to_descr(np.dtype(dtype)),
+                                               "fortran_order": False, "shape": (int(length),)})
+    return buf.getvalue()
+
+
+def _npy_bytes(a):
+    buf = io.BytesIO()
+    np.save(buf, a, allow_pickle=False)
+    return buf.getvalue()
+
+
+class CsrNpzWriter(object):
+    """Writer of one compressed CSR file (the `.npz` of the module docstring), appended chunk by chunk.
+
+    The constructor is CsrShardWriter's, with the same dtypes: indptr and indices int32 when n_cells x G < 2^31
+    and int64 otherwise, data `dtype`.  append(member, compressed, crc, raw_len) takes the next bytes of
+    "indptr", "indices" or "data" as raw DEFLATE blocks that are not final and end on a byte boundary
+    (pst_deflate_blocks' output, or sync_deflate's), with the CRC-32 and length of the bytes they decompress
+    to.  indptr's leading 0 is the writer's: the appended indptr holds the row ends, offset by the nonzeros
+    before them.  The small members are compressed here with zlib.
+
+    Every member is a zip64 entry (local and central zip64 fields, also when small): the .npy header as a
+    stored block, the body, the final block 03 00; its CRC combines the header's with the body's.  Zip
+    members are contiguous and the three streams grow together, so indices, the largest, goes straight into
+    the file and indptr and data into temporaries beside it, which close() appends (copied_at_close: their
+    bytes).  As CsrShardWriter: everything goes to `<path>.partial`, renamed to `<path>` only by a complete
+    close(); an exception inside `with` or abort() leaves nothing behind; an existing `<path>` raises
+    FileExistsError.  The same appends give the same file, byte for byte."""
+
+    def __init__(self, path, shape, pseudotime, branches, scalings, dtype=np.int64):
+        self.path = os.fspath(path)
+        if os.path.lexists(self.path):
+            raise FileExistsError(errno.EEXIST, "the compressed CSR file exists already", self.path)
+        n, G = (int(v) for v in shape)
+        self.shape = (n, G)
+        self.index_dtype, self.dtype = _csr_dtypes(self.shape, dtype)
+        cells = _csr_cells(n, pseudotime, branches, scalings)
+        self.nnz, self.copied_at_close = 0, 0
+        self._partial = self.path + ".partial"
+        self._temps = {m: "%s.%s" % (self._partial, m) for m in ("indptr", "data")}
+        self._central = []
+        self._fh, self._sinks = None, {}
+        self._dtypes = {"indptr": self.index_dtype, "indices": self.index_dtype, "data": self.dtype}
+        self._crc = dict.fromkeys(self._dtypes, 0)
+        self._raw = dict.fromkeys(self._dtypes, 0)
+        self._packed = dict.fromkeys(self._dtypes, 0)
+        try:
+            for p in [self._partial] + list(self._temps.values()):
+                if os.path.lexists(p):                  # left behind by an interrupted writer
+                    os.remove(p)
+            self._fh = open(self._partial, "wb")
+            small = dict(format=np.array(b"csr"), shape=np.array(self.shape, dtype=np.int64), **cells)
+            for name, a in small.items():
+                raw = _npy_bytes(a)
+                c = zlib.compressobj(6, zlib.DEFLATED, -15)
+                self._entry(name, c.compress(raw) + c.flush(), zlib.crc32(raw), len(raw))
+            self._indices_at = self._fh.tell()
+            self._local_header("indices", 0, 0, 0)
+            self._indices_body = self._fh.tell()
+            self._reserved = _NPY_STORED + len(_npy_header(self.index_dtype, 0))
+            self._fh.write(bytes(self._reserved))      # its header block, filled in by close()
+            self._sinks = {"indices": self._fh}
+            for m, p in self._temps.items():
+                self._sinks[m] = open(p, "wb")
+            self.append("indptr", *sync_deflate(np.zeros(1, self.index_dtype).tobytes()))
+        except BaseException:
+            self.abort()
+            raise
+
+    def _local_header(self, name, crc, packed, raw):
+        fname = (name + ".npy").encode("ascii")
+        self._fh.write(struct.pack("<IHHHHHIIIHH", 0x04034B50, _ZIP64, 0, 8, _ZIP_TIME, _ZIP_DATE, crc,
+                                   0xFFFFFFFF, 0xFFFFFFFF, len(fname), 20) + fname
+                       + struct.pack("<HHQQ", 1, 16, raw, packed))
+
+    def _entry(self, name, packed_bytes, crc, raw):
+        """One whole member: its local header and its compressed bytes."""
+        at = self._fh.tell()
+        self._local_header(name, crc, len(packed_bytes), raw)
+        self._fh.write(packed_bytes)
+        self._central.append((name, crc, len(packed_bytes), raw, at))
+
+    def append(self, member, compressed, crc, raw_len):
+        """The next raw_len bytes of member "indptr", "indices" or "data", as non-final DEFLATE blocks."""
+        dt = self._dtypes.get(member)
+        if dt is None:
+            raise ValueError("member must be 'indptr', 'indices' or 'data', not %r" % (member,))
+        if raw_len % dt.itemsize:
+            raise ValueError("%s takes whole %s values, not %d bytes" % (member, dt, raw_len))
+        compressed = memoryview(compressed).cast("B")
+        self._sinks[member].write(compressed)
+        self._crc[member] = int(nat.load().pst_host_crc32_combine(self._crc[member], int(crc) & 0xFFFFFFFF,
+                                                                   int(raw_len)))
+        self._raw[member] += int(raw_len)
+        self._packed[member] += len(compressed)
+
+    def _header_block(self, member):
+        header = _npy_header(self._dtypes[member], self._raw[member] // self._dtypes[member].itemsize)
+        return (struct.pack("<BHH", 0, len(header), len(header) ^ 0xFFFF) + header,
+                zlib.crc32(header), len(header))
+
+    def _finish(self, member, header):
+        """(crc, packed, raw) of a member whose body has been written: header block + body + final block."""
+        block, hcrc, hlen = header
+        crc = int(nat.load().pst_host_crc32_combine(hcrc, self._crc[member], self._raw[member]))
+        return crc, len(block) + self._packed[member] + len(_FINAL_BLOCK), hlen + self._raw[member]
+
+    def close(self):
+        """Finish the file and move it to `path`; raises (and leaves nothing) when rows are missing or the
+        members disagree."""
+        if self._fh is None:
+            return
+        try:
+            n = self.shape[0]
+            rows = self._raw["indptr"] // self.index_dtype.itemsize - 1
+            if rows != n:
+                raise ValueError("%s: %d of %d rows written" % (self.path, rows, n))
+            self.nnz = self._raw["indices"] // self.index_dtype.itemsize
+            if self._raw["data"] // self.dtype.itemsize != self.nnz:
+                raise ValueError("%s: %d column indices but %d values" % (self.path, self.nnz,
+                                                                          self._raw["data"] // self.dtype.itemsize))
+            fh = self._fh
+            for m in self._temps:
+                self._sinks[m].close()
+            # indices: the final block, then its header block and local header in the space kept for them
+            fh.write(_FINAL_BLOCK)
+            end = fh.tell()
+            head = self._header_block("indices")
+            if len(head[0]) != self._reserved:
+                raise RuntimeError("the .npy header of indices outgrew its reserved space")
+            crc, packed, raw = self._finish("indices", head)
+            fh.seek(self._indices_at)
+            self._local_header("indices", crc, packed, raw)
+            fh.write(head[0])
+            fh.seek(end)
+            self._central.append(("indices", crc, packed, raw, self._indices_at))
+            # indptr and data: whole members, their bodies copied from the temporaries
+            for m, p in self._temps.items():
+                head = self._header_block(m)
+                crc, packed, raw = self._finish(m, head)
+                at = fh.tell()
+                self._local_header(m, crc, packed, raw)
+                fh.write(head[0])
+                with open(p, "rb") as src:
+                    shutil.copyfileobj(src, fh, 16 << 20)
+                fh.write(_FINAL_BLOCK)
+                self.copied_at_close += self._packed[m]
+                self._central.append((m, crc, packed, raw, at))
+                os.remove(p)
+            self._central_directory()
+            fh.close()
+            self._fh = None
+            os.rename(self._partial, self.path)
+        except BaseException:
+            self.abort()
+            raise
+
+    def _central_directory(self):
+        fh = self._fh
+        cd_at = fh.tell()
+        for name, crc, packed, raw, at in self._central:
+            fname = (name + ".npy").encode("ascii")
+            fh.write(struct.pack("<IHHHHHHIIIHHHHHII", 0x02014B50, _ZIP64, _ZIP64, 0, 8, _ZIP_TIME, _ZIP_DATE, crc,
+                                 0xFFFFFFFF, 0xFFFFFFFF, len(fname), 28, 0, 0, 0, 0, 0xFFFFFFFF) + fname
+                     + struct.pack("<HHQQQ", 1, 24, raw, packed, at))
+        cd_size, k = fh.tell() - cd_at, len(self._central)
+        eocd64 = fh.tell()
+        fh.write(struct.pack("<IQHHIIQQQQ", 0x06064B50, 44, _ZIP64, _ZIP64, 0, 0, k, k, cd_size, cd_at))
+        fh.write(struct.pack("<IIQI", 0x07064B50, 0, eocd64, 1))
+        fh.write(struct.pack("<IHHHHIIH", 0x06054B50, 0, 0, min(k, 0xFFFF), min(k, 0xFFFF),
+                             min(cd_size, 0xFFFFFFFF), min(cd_at, 0xFFFFFFFF), 0))
+
+    def record(self):
+        """The CompressedCsr of the closed file."""
+        return CompressedCsr(self.path, self.shape, self.nnz, self.dtype, self.index_dtype,
+                             os.path.getsize(self.path))
+
+    def abort(self):
+        """Drop everything written so far."""
+        for f in [self._fh] + list(self._sinks.values()):
+            if f is not None:
+                f.close()
+        self._fh, self._sinks = None, {}
+        for p in [self._partial] + list(self._temps.values()):
+            try:
+                os.remove(p)
+            except OSError:
+                pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, exc, tb):
+        if exc_type is None:
+            self.close()
+        else:
+            self.abort()
+        return False
+
+
 def load_csr_shard(path):
     """(X, pseudotime, branches, scalings) of a shard written by CsrShardWriter: X is a canonical
-    scipy.sparse.csr_matrix over read-only memory maps of indptr, indices and data (no copy)."""
+    scipy.sparse.csr_matrix over read-only memory maps of indptr, indices and data (no copy).  A compressed
+    file written by CsrNpzWriter gives the same tuple, with X decompressed into memory."""
+    if os.path.isfile(path):
+        with np.load(path, allow_pickle=False) as z:
+            fmt = z["format"].item()
+            fmt = fmt.decode("ascii") if isinstance(fmt, bytes) else str(fmt)
+            if fmt != "csr":
+                raise ValueError("expected a csr matrix, found %r" % fmt)
+            shape = tuple(int(v) for v in z["shape"])
+            X = _csr_matrix(z["indptr"], z["indices"], z["data"], shape)
+            return X, z["pseudotime"], z["branches"], z["scalings"]
+
     def member(name, mmap_mode=None):
         return np.load(os.path.join(os.fspath(path), name + ".npy"), mmap_mode=mmap_mode, allow_pickle=False)
 

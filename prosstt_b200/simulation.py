@@ -21,6 +21,10 @@ Extra keyword-only arguments (never required):
            (formats.CsrShardWriter, with the cells' pseudotime, branches and scalings) instead of holding
            them in host memory; X is then the shard's memory-mapped matrix (formats.load_csr_shard).  The
            counts are those of the in-memory call; every chunk is drawn once (CountEngine.stream_csr)
+  compress with out="csr" and path: write one compressed `.npz` at `path` instead (formats.CsrNpzWriter:
+           zip64, DEFLATE members, read by scipy.sparse.load_npz and np.load); the GPU compresses every chunk, so
+           only compressed bytes cross PCIe and reach the disk.  X is then a formats.CompressedCsr record
+           (path, shape, nnz, dtype, index_dtype, nbytes, load()), not the loaded matrix
   sampler  "hybrid" (default): direct inversion of the NB cdf for mean <= 32, sd <= 20, gamma scale <= 32 and
            shape <= 48 - in fp32 below the 1 - 2^-14 quantile of its uniform, with a 64-bit uniform against an
            fp64-accumulated cdf above it, so body and far tail match the exact pmf (checked at 1e9 draws per
@@ -44,7 +48,7 @@ from prosstt_b200 import count_model as cm
 from prosstt_b200 import hostpool
 from prosstt_b200 import sim_utils as sut
 from prosstt_b200.device import CountEngine, TreeTables, choice_cdf, raise_flags, tree_tables
-from prosstt_b200.formats import CsrShardWriter, _csr_matrix, load_csr_shard
+from prosstt_b200.formats import CsrNpzWriter, CsrShardWriter, _csr_matrix, load_csr_shard
 from prosstt_b200.sharding import shard_range
 
 DEFAULT_SAMPLER = "hybrid"
@@ -419,8 +423,11 @@ def _shard_range(n, shard):
     return shard_range(n, rank, world)
 
 
-def _check_csr_request(out, dtype, host_out=None, path=None):
-    """out="csr" takes int64 (default) or int32 data and no preallocated host_out; path needs out="csr"."""
+def _check_csr_request(out, dtype, host_out=None, path=None, compress=False):
+    """out="csr" takes int64 (default) or int32 data and no preallocated host_out; path needs out="csr";
+    compress needs both."""
+    if compress and (path is None or out != "csr"):
+        raise ValueError("compress=True writes a compressed CSR file: it needs out='csr' and path=")
     if path is not None and out != "csr":
         raise ValueError("path= writes a CSR shard: it needs out='csr'")
     if out != "csr":
@@ -431,7 +438,7 @@ def _check_csr_request(out, dtype, host_out=None, path=None):
         raise ValueError("out='csr' stores int64 or int32 counts, not %s" % np.dtype(dtype))
 
 
-def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=None):
+def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=None, compress=False):
     """The count matrix of the cells described by rows/s32: a device int32 tensor (out="torch"), a
     scipy.sparse.csr_matrix with `dtype` data (out="csr", CountEngine.draw_to_csr: only the nonzeros cross
     PCIe) or a fresh host array of `dtype` (reference: int64, simulation.py:651).  The host forms never hold
@@ -439,7 +446,8 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
     by host threads while the next chunk is sampled (CountEngine.draw_to_host).
     out="csr" with `path`: the chunks go to a CSR shard at path (CountEngine.stream_csr into a
     formats.CsrShardWriter, which also stores `cells` = (pseudotime, branches, scalings) host arrays) and the
-    shard's memory-mapped matrix is returned."""
+    shard's memory-mapped matrix is returned; with `compress`, into one compressed file (formats.CsrNpzWriter,
+    stream_csr(compress=True)), and its formats.CompressedCsr record is returned."""
     if out == "torch":
         X = engine.draw(rows, s32, seed, first)
         engine.check()
@@ -447,6 +455,11 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
     if out == "csr":
         _check_csr_request(out, dtype)
         n = int(rows.numel())
+        if path is not None and compress:
+            with CsrNpzWriter(path, (n, engine.G), *cells, dtype=dtype) as w:
+                engine.stream_csr(rows, s32, seed, first, lambda lo, hi, parts: [w.append(*p) for p in parts],
+                                  w.index_dtype, dtype, compress=True)
+            return w.record()
         if path is not None:
             with CsrShardWriter(path, (n, engine.G), *cells, dtype=dtype) as shard:
                 engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *chunk: shard.append(*chunk),
@@ -471,7 +484,7 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
 
 def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
                     seed, first, dev, dtype, out, sampler, host_out=None, host_transport=None, host_threads=0,
-                    path=None):
+                    path=None, compress=False):
     """Common tail of every sampler (simulation.py:590-599): scalings, then counts.
     host_out = (X, pseudotime, branch_codes, scalings) preallocated CPU tensors (int32 (n,G),
     int64, int32, float64; ideally pinned): the counts are streamed into them in cell chunks
@@ -480,7 +493,7 @@ def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mea
     and a fifth entry of host_out, a dict, receives the exact values of the saturated elements as
     "index" (flat, into X) and "value" arrays (formats.widen rebuilds the int32 matrix); without
     the dict a saturated element raises OverflowError instead of passing silently."""
-    _check_csr_request(out, dtype, host_out, path)
+    _check_csr_request(out, dtype, host_out, path, compress)
     n = int(rows.numel())
     s64, s32 = sut.calc_scalings(n, scale, scale_mean, scale_v, seed=nat.derive_seed(seed, 1),
                                  first=first, device=dev, return_device=True)
@@ -509,14 +522,15 @@ def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mea
     if out == "torch":
         return _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out), pt, codes, s64
     cells = pt.cpu().numpy(), tables.branch_names(codes.cpu().numpy()), s64.cpu().numpy()
-    X = _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out, path=path, cells=cells)
+    X = _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out, path=path, cells=cells,
+                       compress=compress)
     return (X,) + cells
 
 
 def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, scale_mean=0.,
                    seed=None, device=None, shard=None, dtype=np.int64, out="numpy",
                    sampler=DEFAULT_SAMPLER, uniforms=None, host_out=None, host_transport=None, host_threads=0, *,
-                   path=None):
+                   path=None, compress=False):
     """Sample `no_cells` (pseudotime, branch) pairs according to tree.density and draw
     their counts (simulation.py:416-471).  Returns (X, pseudotime, branches, scalings).
     `uniforms` (one per cell) replays externally supplied draws through the index map.
@@ -542,7 +556,7 @@ def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, s
              nat.ptr(tables.d("pos_branch")), nat.ptr(rows), nat.ptr(pt), nat.ptr(codes), st)
     return _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
                            seed, lo, dev, dtype, out, sampler, host_out=host_out, host_transport=host_transport,
-                           host_threads=host_threads, path=path)
+                           host_threads=host_threads, path=path, compress=compress)
 
 
 def cover_whole_tree(tree):
@@ -560,7 +574,7 @@ def cover_whole_tree(tree):
 
 def sample_whole_tree(tree, n_factor, alpha=0.3, beta=2, scale=True, scale_mean=0., scale_v=0.7,
                       seed=None, device=None, shard=None, dtype=np.int64, out="numpy",
-                      sampler=DEFAULT_SAMPLER, *, path=None):
+                      sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
     """Every tree position sampled n_factor times (simulation.py:474-517)."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
@@ -575,7 +589,7 @@ def sample_whole_tree(tree, n_factor, alpha=0.3, beta=2, scale=True, scale_mean=
              nat.ptr(tables.d("cover_row")), len(tables.cover_pt), int(n_factor), lo, n,
              nat.ptr(pt), nat.ptr(codes), nat.ptr(rows), nat.stream_ptr(dev))
     return _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
-                           seed, lo, dev, dtype, out, sampler, path=path)
+                           seed, lo, dev, dtype, out, sampler, path=path, compress=compress)
 
 
 def draw_times(timepoint, no_cells, max_time, var=4, seed=None, first=0, device=None,
@@ -597,7 +611,7 @@ def draw_times(timepoint, no_cells, max_time, var=4, seed=None, first=0, device=
 
 def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, beta=2, scale=True,
                              scale_mean=0, scale_v=0.7, seed=None, device=None, shard=None,
-                             dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, *, path=None):
+                             dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
     """Time-series experiment: normally distributed pseudotimes around each sample point,
     branches picked by density (simulation.py:319-379)."""
     dev = nat.device(device)
@@ -623,23 +637,24 @@ def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, b
         nat.call("pst_times_from_normals", nat.ptr(z), n, int(max_time), nat.ptr(pt), st)
     return _sample_data_at_times(tree, pt, alpha=alpha, beta=beta, scale=scale, scale_mean=scale_mean,
                                  scale_v=scale_v, seed=nat.derive_seed(seed, 3), device=dev,
-                                 dtype=dtype, out=out, sampler=sampler, _first=lo, path=path)
+                                 dtype=dtype, out=out, sampler=sampler, _first=lo, path=path, compress=compress)
 
 
 def sample_whole_tree_restricted(tree, alpha=0.2, beta=3, seed=None, device=None, dtype=np.int64,
-                                 out="numpy", sampler=DEFAULT_SAMPLER, *, path=None):
+                                 out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
     """Bare-bones run with default lineage parameters (simulation.py:289-316): one cell
     per pseudotime value, random branch, per-gene alpha/beta around the given means."""
     sample_time = np.arange(0, tree.get_max_time())
     tree.default_gene_expression()
     alphas, betas = cm.generate_negbin_params(tree, mean_alpha=alpha, mean_beta=beta)
     return _sample_data_at_times(tree, sample_time, alpha=alphas, beta=betas, seed=seed,
-                                 device=device, dtype=dtype, out=out, sampler=sampler, path=path)
+                                 device=device, dtype=dtype, out=out, sampler=sampler, path=path,
+                                 compress=compress)
 
 
 def _sample_data_at_times(tree, sample_pt, branches=None, alpha=0.3, beta=2, scale=True,
                           scale_mean=0., scale_v=0.7, seed=None, device=None, dtype=np.int64,
-                          out="numpy", sampler=DEFAULT_SAMPLER, _first=0, path=None):
+                          out="numpy", sampler=DEFAULT_SAMPLER, _first=0, path=None, compress=False):
     """Cells at given pseudotimes (simulation.py:551-599): pick branches if they are not
     supplied, draw library sizes, draw counts.  `_first` is the global index of the first
     cell (sharded callers)."""
@@ -658,7 +673,7 @@ def _sample_data_at_times(tree, sample_pt, branches=None, alpha=0.3, beta=2, sca
     # the index map's own status word is read after the draw has been queued (no stall in front of it)
     try:
         result = _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
-                                 seed, _first, dev, dtype, out, sampler, path=path)
+                                 seed, _first, dev, dtype, out, sampler, path=path, compress=compress)
     except IndexError:
         sut.check_flags(flags)
         raise
@@ -681,13 +696,14 @@ def _rows_for(tables, pt, branches, dev):
 
 
 def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, device=None,
-                dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, first=0, *, path=None):
+                dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, first=0, *, path=None, compress=False):
     """UMI counts of cells at (pseudotime, branch) with library sizes `scalings`
     (simulation.py:602-651): X[n,g] ~ NB(mean = means[branch_n][t_n - start, g]*scaling_n,
     variance = alpha_g mean^2 + beta_g mean).  out="csr", path=p writes the CSR shard with the
-    pseudotime, branches and scalings given here and returns its memory-mapped matrix."""
+    pseudotime, branches and scalings given here and returns its memory-mapped matrix; with compress=True the
+    compressed file, and its formats.CompressedCsr record."""
     dev = nat.device(device)
-    _check_csr_request(out, dtype, path=path)
+    _check_csr_request(out, dtype, path=path, compress=compress)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
     pt = pseudotime if isinstance(pseudotime, torch.Tensor) else \
@@ -704,7 +720,7 @@ def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, de
     if path is not None:
         given = scalings.detach().cpu().numpy() if isinstance(scalings, torch.Tensor) else scalings
         cells = pt.cpu().numpy(), tables.branch_names(codes.cpu().numpy()), np.asarray(given, dtype=np.float64)
-    return _sample_counts(engine, rows, s32, seed, first, dtype, out, path=path, cells=cells)
+    return _sample_counts(engine, rows, s32, seed, first, dtype, out, path=path, cells=cells, compress=compress)
 
 
 def add_non_diff_genes(inform_expr_matrix, genes, gene_params, cell_scalings, seed=None,
