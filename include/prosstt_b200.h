@@ -282,6 +282,19 @@ int pst_csr_pack(const int32_t *X, int64_t n, int64_t G, int64_t ldx, const int6
 int pst_csr_indptr_bytes(const int64_t *indptr, int64_t n, int64_t *running, void *out, int32_t out_bits,
                          void *stream);
 
+/* Matrix Market text of a chunk of cells (the 10x matrix.mtx.gz, genes x cells): row i of the int32
+ * chunk X is cell col0 + i + 1 of the file, and each nonzero X[i][g] = v is the line
+ * "<g+1> <col0+i+1> <v>\n", genes ascending.  pst_mtx_row_bytes writes each row's text length,
+ * row_bytes[i] = nnz_i (digits(col0+i+1) + 3) + sum over the nonzeros of digits(g+1) + digits(v) (int32;
+ * G <= 2^31 / 42); pst_csr_row_offsets scans it into the chunk's text pointer (n+1 int64 entries).
+ * pst_mtx_format writes row i's lines at out + text_ptr[i] (out 16-byte aligned), or nothing at all when
+ * text_ptr[n] > cap, so a text pointer made on the device needs no host read: the caller sees text_ptr[n]
+ * later and formats again into a larger buffer. */
+int pst_mtx_row_bytes(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t col0, int32_t *row_bytes,
+                      void *stream);
+int pst_mtx_format(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t col0, const int64_t *text_ptr,
+                   int64_t cap, char *out, void *stream);
+
 /* ---- raw DEFLATE (RFC 1951) on the device: the compressed CSR file (pst_deflate.cu) ---------------
  * The input is cut into blocks of `block` bytes (a multiple of 1024, at most 32768).  Each block becomes
  * one dynamic-Huffman block over the literals 0-255 and end-of-block (no length or distance codes; the

@@ -273,6 +273,176 @@ csr_indptr_kernel(const int64_t *__restrict__ indptr, int64_t n, int64_t *__rest
   if (threadIdx.x == 0) *running = base + indptr[n];
 }
 
+// ---------------------------------------------------------------------------------------------
+// Matrix Market text of a chunk (the 10x `matrix.mtx.gz`, genes x cells): row i of the chunk is cell
+// col0 + i + 1 of the file, and its nonzero X[i][g] = v is the line "<g+1> <col0+i+1> <v>\n", genes
+// ascending.  pst_mtx_row_bytes gives each row's text length, pst_csr_row_offsets scans them into the
+// chunk's text pointer and pst_mtx_format writes the text.  Both walk a row with one warp, a lane owning
+// a gene quad, like the CSR kernels above.
+// ---------------------------------------------------------------------------------------------
+constexpr int kMtxWarps = 4;                           // warps per block of pst_mtx_format
+constexpr int kMtxLine = 42;                           // longest line: 10 + 19 + 10 digits, 3 separators
+constexpr int kMtxStage = 16 + 128 * kMtxLine;         // one 16-byte carry + the text of 128 genes
+static_assert(kMtxStage % 16 == 0, "the staging of each warp stays 16-byte aligned");
+constexpr int64_t kMtxMaxG = ((int64_t)1 << 31) / kMtxLine;   // a row's text fits int32
+
+__device__ __forceinline__ int dec_digits32(uint32_t v) {
+  return 1 + (v >= 10u) + (v >= 100u) + (v >= 1000u) + (v >= 10000u) + (v >= 100000u) + (v >= 1000000u) +
+         (v >= 10000000u) + (v >= 100000000u) + (v >= 1000000000u);
+}
+
+__device__ __forceinline__ int dec_digits64(uint64_t v) {     // once per row
+  int d = 1;
+  for (; v >= 10u; v /= 10u) ++d;
+  return d;
+}
+
+// the d decimal digits of v at p, two at a time from the table "00" ... "99"
+template <typename U>
+__device__ __forceinline__ void put_dec(char *p, U v, int d, const char *__restrict__ pairs) {
+  char *e = p + d;
+  while (v >= 100u) {
+    const U q = v / 100u;
+    const unsigned r = (unsigned)(v - q * 100u);
+    e -= 2;
+    e[0] = pairs[2 * r];
+    e[1] = pairs[2 * r + 1];
+    v = q;
+  }
+  if (v >= 10u) {
+    e[-2] = pairs[2 * (unsigned)v];
+    e[-1] = pairs[2 * (unsigned)v + 1];
+  } else {
+    e[-1] = (char)('0' + (unsigned)v);
+  }
+}
+
+// row_bytes[i] = nnz_i (digits(col0 + i + 1) + 3) + sum over the row's nonzeros of digits(g + 1) + digits(v):
+// csr_row_count_kernel's walk (four 128-bit streaming loads in flight per lane, one REDUX per row)
+template <bool VEC>
+__global__ void __launch_bounds__(256)
+mtx_row_bytes_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx, int64_t col0,
+                     int32_t *__restrict__ row_bytes) {
+  const int lane = threadIdx.x & 31;
+  const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
+  const int64_t Q = (G + 3) / 4;
+  for (int64_t row = warp0; row < n; row += n_warps) {
+    const int32_t *src = X + row * ldx;
+    unsigned c = 0, b = 0;
+    for (int64_t q0 = 0; q0 < Q; q0 += 128) {
+      int4 v[4];
+#pragma unroll
+      for (int j = 0; j < 4; ++j) v[j] = load_quad<VEC>(src, q0 + 32 * j + lane, Q, G);
+#pragma unroll
+      for (int j = 0; j < 4; ++j) {
+        const uint32_t g = (uint32_t)((q0 + 32 * j + lane) * 4) + 1u;
+        const int32_t vv[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
+#pragma unroll
+        for (int k = 0; k < 4; ++k) {
+          const bool nz = vv[k] != 0;
+          c += nz;
+          b += nz ? (unsigned)(dec_digits32(g + k) + dec_digits32((uint32_t)vv[k])) : 0u;
+        }
+      }
+    }
+    c = __reduce_add_sync(0xffffffffu, c);
+    b = __reduce_add_sync(0xffffffffu, b);
+    if (lane == 0) row_bytes[row] = (int32_t)(b + c * (unsigned)(dec_digits64((uint64_t)(col0 + row + 1)) + 3));
+  }
+}
+
+// The text of row i at out + text_ptr[i].  Per tile of 128 genes a lane writes its lines into the warp's
+// shared staging at a warp-exclusive scan of their lengths, then the warp stores the staging's whole
+// 16-byte pieces with 128-bit stores (512 contiguous bytes per instruction) and carries the last partial
+// piece to the next tile.  A row's first and last pieces are shared with its neighbours' text: their bytes
+// are stored one by one, only the row's own.  Writes nothing when text_ptr[n] > cap.
+template <bool VEC>
+__global__ void __launch_bounds__(kMtxWarps * 32, 8)   // 8 blocks per SM: at most 64 registers, no spill
+mtx_format_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx, int64_t col0,
+                  const int64_t *__restrict__ text_ptr, int64_t cap, char *__restrict__ out) {
+  __shared__ char pairs[200];
+  __shared__ __align__(16) char stage[kMtxWarps][kMtxStage];
+  __shared__ char cell_field[kMtxWarps][20];
+  if (text_ptr[n] > cap) return;                               // the same for every thread of the grid
+  for (int t = threadIdx.x; t < 100; t += blockDim.x) {
+    pairs[2 * t] = (char)('0' + t / 10);
+    pairs[2 * t + 1] = (char)('0' + t % 10);
+  }
+  __syncthreads();
+  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
+  char *s = stage[wid];
+  char *cf = cell_field[wid];
+  const int64_t Q = (G + 3) / 4;
+  for (int64_t row = (int64_t)blockIdx.x * kMtxWarps + wid; row < n; row += (int64_t)gridDim.x * kMtxWarps) {
+    const int64_t pos = text_ptr[row];
+    if (pos == text_ptr[row + 1]) continue;                    // no nonzeros
+    const uint64_t cell = (uint64_t)(col0 + row + 1);
+    const int cl = dec_digits64(cell);
+    if (lane == 0) put_dec(cf, cell, cl, pairs);               // the cell field, once per row
+    __syncwarp();
+    const int32_t *src = X + row * ldx;
+    int64_t base = pos & ~(int64_t)15;                         // staging byte 0 belongs at out + base
+    int head = (int)(pos & 15);                                // bytes before it that are not this row's
+    int fill = head;
+    for (int64_t q0 = 0; q0 < Q; q0 += 32) {
+      const int64_t q = q0 + lane;
+      const int4 v = load_quad<VEC>(src, q, Q, G);
+      const int32_t vv[4] = {v.x, v.y, v.z, v.w};
+      const uint32_t g = (uint32_t)(q * 4) + 1u;
+      int len[4], tot = 0;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        len[k] = vv[k] != 0 ? dec_digits32(g + k) + cl + dec_digits32((uint32_t)vv[k]) + 3 : 0;
+        tot += len[k];
+      }
+      int incl = tot;
+#pragma unroll
+      for (int d = 1; d < 32; d <<= 1) {
+        const int o = __shfl_up_sync(0xffffffffu, incl, d);
+        if (lane >= d) incl += o;
+      }
+      const int T = __shfl_sync(0xffffffffu, incl, 31);
+      if (T == 0) continue;
+      int at = fill + incl - tot;
+#pragma unroll
+      for (int k = 0; k < 4; ++k) {
+        if (vv[k] != 0) {
+          const int dg = dec_digits32(g + k);
+          char *p = s + at;
+          put_dec(p, g + k, dg, pairs);
+          p[dg] = ' ';
+          p += dg + 1;
+          for (int c = 0; c < cl; ++c) p[c] = cf[c];
+          p[cl] = ' ';
+          p += cl + 1;
+          const int dv = dec_digits32((uint32_t)vv[k]);
+          put_dec(p, (uint32_t)vv[k], dv, pairs);
+          p[dv] = '\n';
+          at += len[k];
+        }
+      }
+      __syncwarp();
+      const int have = fill + T, whole = have >> 4;
+      for (int p = (head ? 1 : 0) + lane; p < whole; p += 32)
+        __stcs(reinterpret_cast<int4 *>(out + base) + p, reinterpret_cast<const int4 *>(s)[p]);
+      if (head && whole) {
+        if (lane >= head && lane < 16) out[base + lane] = s[lane];
+        head = 0;
+      }
+      const int rem = have - 16 * whole;
+      const char carried = lane < rem ? s[16 * whole + lane] : 0;
+      __syncwarp();
+      if (lane < rem) s[lane] = carried;
+      __syncwarp();
+      base += 16 * whole;
+      fill = rem;
+    }
+    if (lane >= head && lane < fill) out[base + lane] = s[lane];
+    __syncwarp();                                              // the staging is rewritten by the next row
+  }
+}
+
 // Pure-store kernel: the write-only HBM ceiling the count write is measured against (SURVEY.md 8d).  Same
 // shape of traffic as the sampler's output: 128-bit stores, 512 contiguous bytes per warp instruction.
 __global__ void __launch_bounds__(256) store_fill_kernel(int4 *__restrict__ out, int64_t n16, int32_t value) {
@@ -443,5 +613,39 @@ extern "C" int pst_csr_indptr_bytes(const int64_t *indptr, int64_t n, int64_t *r
   cudaStream_t st = (cudaStream_t)stream;
   if (out_bits == 32) csr_indptr_kernel<int32_t><<<1, 1024, 0, st>>>(indptr, n, running, (int32_t *)out);
   else csr_indptr_kernel<int64_t><<<1, 1024, 0, st>>>(indptr, n, running, (int64_t *)out);
+  return check_launch(fn);
+}
+
+extern "C" int pst_mtx_row_bytes(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t col0, int32_t *row_bytes,
+                                 void *stream) {
+  const char *fn = "pst_mtx_row_bytes";
+  PST_REQUIRE(n >= 0 && G >= 0 && ldx >= G && col0 >= 0, fn, "need n, G, col0 >= 0 and ldx >= G");
+  PST_REQUIRE(G <= kMtxMaxG, fn, "a row's text does not fit int32");
+  PST_REQUIRE(col0 <= INT64_MAX - n, fn, "cell numbers do not fit int64");
+  if (n == 0) return 0;
+  PST_REQUIRE(row_bytes && (G == 0 || X), fn, "null pointer");
+  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
+  const unsigned grid = stream_grid(n * 32);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec) mtx_row_bytes_kernel<true><<<grid, 256, 0, st>>>(X, n, G, ldx, col0, row_bytes);
+  else mtx_row_bytes_kernel<false><<<grid, 256, 0, st>>>(X, n, G, ldx, col0, row_bytes);
+  return check_launch(fn);
+}
+
+extern "C" int pst_mtx_format(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t col0,
+                              const int64_t *text_ptr, int64_t cap, char *out, void *stream) {
+  const char *fn = "pst_mtx_format";
+  PST_REQUIRE(n >= 0 && G >= 0 && ldx >= G && col0 >= 0 && cap >= 0, fn, "need n, G, col0, cap >= 0 and ldx >= G");
+  PST_REQUIRE(G <= kMtxMaxG, fn, "a row's text does not fit int32");
+  PST_REQUIRE(col0 <= INT64_MAX - n, fn, "cell numbers do not fit int64");
+  if (n == 0 || G == 0) return 0;
+  PST_REQUIRE(X && text_ptr && out, fn, "null pointer");
+  PST_REQUIRE((uintptr_t)out % 16 == 0, fn, "out must be 16-byte aligned");
+  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
+  const unsigned grid = (unsigned)std::max<int64_t>(
+      1, std::min<int64_t>((n + kMtxWarps - 1) / kMtxWarps, (int64_t)num_sm() * 16));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec) mtx_format_kernel<true><<<grid, kMtxWarps * 32, 0, st>>>(X, n, G, ldx, col0, text_ptr, cap, out);
+  else mtx_format_kernel<false><<<grid, kMtxWarps * 32, 0, st>>>(X, n, G, ldx, col0, text_ptr, cap, out);
   return check_launch(fn);
 }

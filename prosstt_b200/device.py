@@ -263,6 +263,13 @@ def _pinned_staging(dev, nbytes):
     return have
 
 
+def _mtx_slot_bytes(G, n):
+    """Matrix Market text bytes budgeted per gene slot of a chunk of a file of n cells: one line
+    "<gene> <cell> <count>\n" with a count of up to 3 digits.  A chunk with more text is formatted again into
+    a larger buffer (CountEngine.stream_csr)."""
+    return len(str(G)) + len(str(n)) + 6
+
+
 def _plan_chunks(n, chunk_cells, cell_bytes, budget):
     """The cell chunks of a chunked device->host call: (chunk, [(lo, hi), ...]) covering [0, n) in order, where
     chunk is the largest chunk (the size of the buffers).  Owns the chunk size and the ramp-up.
@@ -593,7 +600,7 @@ class CountEngine(object):
         return indptr, indices, data
 
     def stream_csr(self, rows, scaling32, seed, cell0, consume, index_dtype=np.int64, data_dtype=np.int64,
-                   chunk_cells=None, threads=0, overflow_cap=None, compress=False):
+                   chunk_cells=None, threads=0, overflow_cap=None, compress=False, mtx=False):
         """Sample the cells in chunks and hand each one as CSR to consume(lo, hi, indptr, indices, data), on a
         worker thread, once per chunk, in cell order.  indptr is chunk-local int64 (hi - lo + 1 entries from 0);
         indices and data are the chunk's nonzeros in `index_dtype` / `data_dtype` (int32 or int64), columns
@@ -620,7 +627,18 @@ class CountEngine(object):
         data_dtype bytes (no saturation, no re-pack), pst_csr_indptr_bytes the indptr bytes with a running nnz
         kept on the device, and pst_deflate_blocks compresses each member, reading its length from the device.
         The host reads (nnz, status word, compressed sizes, CRCs) one chunk late as above and copies exactly
-        the compressed bytes."""
+        the compressed bytes.
+
+        mtx=True: consume(lo, hi, compressed, crc, text_len, nnz) receives the chunk as Matrix Market text
+        (formats.MtxWriter.append): `compressed` (a reused uint8 host buffer) is raw DEFLATE that decompresses to
+        the text_len bytes of the chunk's nnz lines "<g+1> <c+1> <v>\n", c = lo + row within the chunk, whose
+        CRC-32 is crc; index_dtype and data_dtype do not apply.  Per chunk, on the sampling stream with no host
+        wait: the draw and the row pointer as above, pst_mtx_row_bytes and pst_csr_row_offsets (the chunk's text
+        pointer), pst_mtx_format into the text buffer and pst_deflate_blocks over text_ptr[n] bytes of it.  The
+        text buffer holds _mtx_slot_bytes per gene slot (every count of up to 3 digits); a chunk
+        with more text is not formatted (pst_mtx_format writes nothing), and when the host reads its text length
+        one chunk late the buffers grow and the chunk is formatted and compressed again from its work buffer,
+        which survives until chunk i+2 is drawn - there is no redraw."""
         index_dtype, data_dtype = np.dtype(index_dtype), np.dtype(data_dtype)
         for what, dt in (("indices", index_dtype), ("data", data_dtype)):
             if dt not in (np.dtype(np.int32), np.dtype(np.int64)):
@@ -631,8 +649,10 @@ class CountEngine(object):
         if n == 0:
             return 0
         if G == 0:
-            if compress:
-                from prosstt_b200.formats import sync_deflate
+            from prosstt_b200.formats import sync_deflate
+            if mtx:
+                consume(0, n, *sync_deflate(b""), 0)
+            elif compress:
                 consume(0, n, [("indptr",) + sync_deflate(np.zeros(n, index_dtype).tobytes()),
                                ("indices",) + sync_deflate(b""), ("data",) + sync_deflate(b"")])
             else:
@@ -640,7 +660,11 @@ class CountEngine(object):
             return 0
         ibits = 16 if G <= 65536 else 32                 # width of the column stream
         ibytes = ibits // 8
-        if compress:
+        if mtx:
+            slot = _mtx_slot_bytes(G, n)
+            # the text of a chunk and its compressed form, bounded by about as many bytes again
+            chunk, bounds = _plan_chunks(n, chunk_cells, 2 * slot * G, _STAGE_BYTES)
+        elif compress:
             isz, dsz = index_dtype.itemsize, data_dtype.itemsize
             # the wide streams of a chunk and their compressed form, bounded by about as many bytes again
             chunk, bounds = _plan_chunks(n, chunk_cells, 2 * (isz + dsz) * G, _STAGE_BYTES)
@@ -650,7 +674,8 @@ class CountEngine(object):
         work = [torch.empty((chunk, G), dtype=torch.int32, device=dev) for _ in range(2)]
         row_nnz = torch.empty(chunk, dtype=torch.int32, device=dev)      # read by the scan right after the count
         indptr = [torch.empty(chunk + 1, dtype=torch.int64, device=dev) for _ in range(2)]
-        # saturated, nnz, status word; compress: the three compressed sizes and CRCs
+        # saturated, nnz, status word; compress: the three compressed sizes and CRCs; mtx: the text length, the
+        # compressed size and the CRC
         info = torch.zeros((2, 9), dtype=torch.int64, device=dev)
         info_host = torch.zeros((2, 9), dtype=torch.int64).pin_memory()
         sized = [None, None]
@@ -681,7 +706,65 @@ class CountEngine(object):
             total[0] += vals[1]
             return vals
 
-        if compress:
+        if mtx:
+            lib = nat.load()
+            block = _DEFLATE_BLOCK
+            row_bytes = torch.empty(chunk, dtype=torch.int32, device=dev)
+            text_ptr = [torch.empty(chunk + 1, dtype=torch.int64, device=dev) for _ in range(2)]
+            buf = {"cap": -1}                             # the text buffer, its deflate workspace and capacity
+            packed = [None, None]
+            formatted_cap = [0, 0]                        # the capacity chunk k was formatted against
+            stage_host = list(_pinned_staging(dev, int(lib.pst_deflate_bound(chunk * G * slot, block))))
+            landed_info = {}                              # chunk start -> its record, from collect to landed
+
+            def reserve(k, cap):
+                """Text buffer of at least cap bytes, and room in packed[k] for its compressed form."""
+                if cap > buf["cap"]:
+                    buf["cap"] = cap
+                    buf["text"] = torch.empty(max(16, cap), dtype=torch.uint8, device=dev)
+                    buf["work_bytes"] = int(lib.pst_deflate_workspace_bytes(cap, block))
+                    buf["work"] = torch.empty(max(1, buf["work_bytes"]), dtype=torch.uint8, device=dev)
+                bound = int(lib.pst_deflate_bound(buf["cap"], block))
+                if packed[k] is None or packed[k].numel() < bound:
+                    packed[k] = torch.empty(max(1, bound), dtype=torch.uint8, device=dev)
+
+            def text(k, lo, cells):
+                """Format chunk k from its work buffer and compress the text."""
+                reserve(k, buf["cap"])
+                formatted_cap[k] = buf["cap"]
+                nat.call("pst_mtx_format", work[k], cells, G, G, lo, text_ptr[k], buf["cap"], buf["text"], st)
+                nat.call("pst_deflate_blocks", buf["text"], text_ptr[k][cells:cells + 1], 1, buf["cap"], block,
+                         packed[k], info[k, 4], info[k, 5].data_ptr(), buf["work"], buf["work_bytes"], st)
+
+            reserve(0, chunk * G * slot)
+
+            def produce(k, lo, hi):
+                cells = hi - lo
+                draw_rows(k, lo, hi)
+                nat.call("pst_mtx_row_bytes", work[k], cells, G, G, lo, row_bytes, st)
+                nat.call("pst_csr_row_offsets", row_bytes, cells, text_ptr[k], st)
+                info[k, 3].copy_(text_ptr[k][cells])
+                text(k, lo, cells)
+                record(k, cells)
+
+            def collect(k, lo, hi):
+                vals = read_info(k)
+                # the text did not fit the buffer as it was when the chunk was queued: nothing was formatted.  The
+                # buffer may have grown since (for the chunk before), so the test is against that capacity.
+                if vals[3] > formatted_cap[k]:
+                    reserve(k, max(vals[3], 2 * formatted_cap[k]))
+                    text(k, lo, hi - lo)
+                    vals = info[k].tolist()               # waits for the second format: the copies wait for the first
+                size = vals[4]
+                if stage_host[k].numel() < size:
+                    stage_host[k] = torch.empty(size, dtype=torch.uint8).pin_memory()
+                landed_info[lo] = vals
+                return [(packed[k][:size], stage_host[k][:size])]
+
+            def landed(dsts, lo, hi):
+                vals = landed_info.pop(lo)
+                consume(lo, hi, dsts[0].numpy(), vals[5] & 0xFFFFFFFF, vals[3], vals[1])
+        elif compress:
             lib = nat.load()
             block = _DEFLATE_BLOCK
             wide = [torch.empty(max(1, chunk * isz), dtype=torch.uint8, device=dev),       # indptr, indices, data

@@ -24,8 +24,14 @@ added, both readable without this package:
   a sync-flush marker, concatenated), so only compressed bytes cross PCIe and reach the disk.  The file
   cannot be memory-mapped: the call returns a `CompressedCsr` record, and `load_csr_shard` decompresses
   it into memory.
+* 10x directories (`MtxWriter`, written by `out="mtx", path=...`): the gzipped Matrix Market matrix, features
+  and barcodes that Seurat::Read10X, DropletUtils::read10xCounts, Matrix::readMM and scanpy.read_10x_mtx read,
+  plus the cells' parameters.  The GPU formats each chunk as text (pst_mtx_format) and compresses it
+  (pst_deflate_blocks), so only compressed text crosses PCIe and reaches the disk.  The call returns an
+  `MtxRecord`.
 """
 import collections
+import concurrent.futures
 import errno
 import io
 import os
@@ -524,6 +530,170 @@ class CsrNpzWriter(object):
                 os.remove(p)
             except OSError:
                 pass
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, exc, tb):
+        if exc_type is None:
+            self.close()
+        else:
+            self.abort()
+        return False
+
+
+_GZIP_HEADER = b"\x1f\x8b\x08\x00\x00\x00\x00\x00\x00\xff"   # DEFLATE, no flags, MTIME 0, XFL 0, OS 255 (unknown)
+MTX_HEADER_BYTES = 128                                        # the three header lines of matrix.mtx.gz together
+_MTX_BANNER = b"%%MatrixMarket matrix coordinate integer general\n"
+
+
+def gzip_member(raw, level=6):
+    """`raw` as one gzip member (RFC 1952) with the fixed header of every .gz of a 10x directory."""
+    c = zlib.compressobj(level, zlib.DEFLATED, -15)
+    return _GZIP_HEADER + c.compress(raw) + c.flush() + struct.pack("<II", zlib.crc32(raw), len(raw) & 0xFFFFFFFF)
+
+
+def mtx_header(G, n, nnz):
+    """The first MTX_HEADER_BYTES bytes of the text of matrix.mtx.gz: the banner, a comment line of spaces that
+    takes up the slack (so the size line can be rewritten in place once nnz is known) and "<G> <n> <nnz>"."""
+    size = b"%d %d %d\n" % (G, n, nnz)
+    pad = MTX_HEADER_BYTES - len(_MTX_BANNER) - len(size) - 2
+    if pad < 0:
+        raise ValueError("the Matrix Market size line %r does not fit the header" % size)
+    return _MTX_BANNER + b"%" + b" " * pad + b"\n" + size
+
+
+def mtx_barcodes(first, n):
+    """barcodes.tsv text: cell_<i> for the global cell indices first ... first + n - 1."""
+    return "".join("cell_%d\n" % i for i in range(first, first + n)).encode("ascii")
+
+
+def mtx_features(G):
+    """features.tsv text: gene_<j>, gene_<j>, Gene Expression for j = 0 ... G - 1 (the column names of the
+    reference's _simulation.txt)."""
+    return "".join("gene_%d\tgene_%d\tGene Expression\n" % (j, j) for j in range(G)).encode("ascii")
+
+
+def mtx_cell_params(first, pseudotime, branches, scalings):
+    """cellparams.tsv text: the reference's _cellparams.txt (tree_utils.save_cell_params) indexed by the
+    barcodes."""
+    from prosstt_b200 import tree_utils
+    names = ["cell_%d" % i for i in range(first, first + len(pseudotime))]
+    return tree_utils.cell_params_frame(pseudotime, branches, scalings, index=names).to_csv(sep="\t").encode("utf-8")
+
+
+class MtxRecord(collections.namedtuple("MtxRecord", "path shape nnz nbytes")):
+    """The X of an out="mtx" call: a 10x directory on disk.  shape is (cells, genes); nbytes is the size of
+    matrix.mtx.gz; load() reads it back (scipy.io.mmread) as the cells x genes int64 csr_matrix."""
+    __slots__ = ()
+
+    def load(self):
+        import scipy.io
+        import scipy.sparse as sp
+        m = scipy.io.mmread(os.path.join(self.path, "matrix.mtx.gz"), spmatrix=False)
+        return sp.csr_matrix(m.T, dtype=np.int64)
+
+
+class MtxWriter(object):
+    """Writer of one 10x directory (Cell Ranger v3 layout), the matrix appended chunk by chunk:
+      matrix.mtx.gz     genes x cells Matrix Market coordinate text, cell-major, genes ascending in a cell;
+      features.tsv.gz   gene_<j> \\t gene_<j> \\t Gene Expression;
+      barcodes.tsv.gz   cell_<i>, i the global cell index (first + local index);
+      cellparams.tsv.gz the reference's _cellparams.txt for these cells, indexed by the barcodes.
+    Every .gz is one gzip member with MTIME 0, XFL 0 and OS 255, so the same appends give the same bytes.
+
+    append(rows, nnz, compressed, crc, raw_len) takes the text of the next `rows` cells (their `nnz` lines)
+    as raw DEFLATE blocks that are not final and end on a byte boundary (pst_deflate_blocks' output over
+    pst_mtx_format's text, or sync_deflate's), with the CRC-32 and length of the text.  The first
+    MTX_HEADER_BYTES of the text, whose nnz is not known before close(), are a stored block written at once
+    and rewritten in place at close() with the same length; the member's CRC combines the header's with the
+    body's.  The three small files are built on a worker thread while the matrix streams.  As CsrShardWriter:
+    everything goes to `<path>.partial`, renamed to `<path>` only by a complete close(); an exception inside
+    `with` or abort() leaves nothing behind; an existing `<path>` raises FileExistsError."""
+
+    def __init__(self, path, shape, pseudotime, branches, scalings, first=0):
+        self.path = os.fspath(path)
+        if os.path.lexists(self.path):
+            raise FileExistsError(errno.EEXIST, "the 10x directory exists already", self.path)
+        n, G = (int(v) for v in shape)
+        self.shape, self.first = (n, G), int(first)
+        cells = _csr_cells(n, pseudotime, branches, scalings)
+        self.rows, self.nnz = 0, 0
+        self._crc, self._raw = 0, 0
+        self._dir = self.path + ".partial"
+        self._fh, self._small = None, None
+        if os.path.lexists(self._dir):                  # left behind by an interrupted writer
+            shutil.rmtree(self._dir)
+        os.makedirs(self._dir)
+        try:
+            self._fh = open(os.path.join(self._dir, "matrix.mtx.gz"), "wb")
+            self._fh.write(_GZIP_HEADER)
+            self._header_at = self._fh.tell()
+            self._fh.write(self._header_block(0))
+            pool = concurrent.futures.ThreadPoolExecutor(max_workers=1)
+            self._small = pool.submit(self._write_small, (cells["pseudotime"], cells["branches"], cells["scalings"]))
+            pool.shutdown(wait=False)
+        except BaseException:
+            self.abort()
+            raise
+
+    def _header_block(self, nnz):
+        header = mtx_header(self.shape[1], self.shape[0], nnz)
+        return struct.pack("<BHH", 0, len(header), len(header) ^ 0xFFFF) + header
+
+    def _write_small(self, cells):
+        n, G = self.shape
+        for name, text in (("features", lambda: mtx_features(G)), ("barcodes", lambda: mtx_barcodes(self.first, n)),
+                           ("cellparams", lambda: mtx_cell_params(self.first, *cells))):
+            with open(os.path.join(self._dir, name + ".tsv.gz"), "wb") as fh:
+                fh.write(gzip_member(text()))
+
+    def append(self, rows, nnz, compressed, crc, raw_len):
+        """The text of the next `rows` cells, `nnz` lines of raw_len bytes, as non-final DEFLATE blocks."""
+        if self.rows + int(rows) > self.shape[0]:
+            raise ValueError("more rows than announced (%d)" % self.shape[0])
+        compressed = memoryview(compressed).cast("B")
+        self._fh.write(compressed)
+        self._crc = int(nat.load().pst_host_crc32_combine(self._crc, int(crc) & 0xFFFFFFFF, int(raw_len)))
+        self._raw += int(raw_len)
+        self.rows += int(rows)
+        self.nnz += int(nnz)
+
+    def close(self):
+        """Finish the directory and move it to `path`; raises (and leaves nothing) when rows are missing."""
+        if self._fh is None:
+            return
+        try:
+            if self.rows != self.shape[0]:
+                raise ValueError("%s: %d of %d rows written" % (self.path, self.rows, self.shape[0]))
+            fh = self._fh
+            block = self._header_block(self.nnz)
+            header = block[5:]
+            crc = int(nat.load().pst_host_crc32_combine(zlib.crc32(header), self._crc, self._raw))
+            fh.write(_FINAL_BLOCK + struct.pack("<II", crc, (len(header) + self._raw) & 0xFFFFFFFF))
+            fh.flush()
+            if os.pwrite(fh.fileno(), block, self._header_at) != len(block):
+                raise OSError("short write of the matrix.mtx.gz header")
+            fh.close()
+            self._fh = None
+            self._small.result()
+            os.rename(self._dir, self.path)
+        except BaseException:
+            self.abort()
+            raise
+
+    def record(self):
+        """The MtxRecord of the closed directory."""
+        return MtxRecord(self.path, self.shape, self.nnz, os.path.getsize(os.path.join(self.path, "matrix.mtx.gz")))
+
+    def abort(self):
+        """Drop everything written so far."""
+        if self._fh is not None:
+            self._fh.close()
+        self._fh = None
+        if self._small is not None:
+            concurrent.futures.wait([self._small])      # it writes into the directory removed below
+        shutil.rmtree(self._dir, ignore_errors=True)
 
     def __enter__(self):
         return self

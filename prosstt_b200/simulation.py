@@ -25,6 +25,12 @@ Extra keyword-only arguments (never required):
            zip64, DEFLATE members, read by scipy.sparse.load_npz and np.load); the GPU compresses every chunk, so
            only compressed bytes cross PCIe and reach the disk.  X is then a formats.CompressedCsr record
            (path, shape, nnz, dtype, index_dtype, nbytes, load()), not the loaded matrix
+           out="mtx" with path: write a 10x directory at `path` (formats.MtxWriter: matrix.mtx.gz genes x cells,
+           features.tsv.gz, barcodes.tsv.gz named by the global cell index, cellparams.tsv.gz), read by
+           Seurat::Read10X, DropletUtils::read10xCounts, Matrix::readMM and scanpy.read_10x_mtx.  The GPU formats
+           and compresses every chunk, so only gzipped text crosses PCIe and reaches the disk.  X is then a
+           formats.MtxRecord (path, shape, nnz, nbytes, load()); the counts are those of out="csr".  The file is
+           always gzipped (compress=True is an error), and dtype must be int64 or int32 as for "csr"
   sampler  "hybrid" (default): direct inversion of the NB cdf for mean <= 32, sd <= 20, gamma scale <= 32 and
            shape <= 48 - in fp32 below the 1 - 2^-14 quantile of its uniform, with a 64-bit uniform against an
            fp64-accumulated cdf above it, so body and far tail match the exact pmf (checked at 1e9 draws per
@@ -48,7 +54,7 @@ from prosstt_b200 import count_model as cm
 from prosstt_b200 import hostpool
 from prosstt_b200 import sim_utils as sut
 from prosstt_b200.device import CountEngine, TreeTables, choice_cdf, raise_flags, tree_tables
-from prosstt_b200.formats import CsrNpzWriter, CsrShardWriter, _csr_matrix, load_csr_shard
+from prosstt_b200.formats import CsrNpzWriter, CsrShardWriter, MtxWriter, _csr_matrix, load_csr_shard
 from prosstt_b200.sharding import shard_range
 
 DEFAULT_SAMPLER = "hybrid"
@@ -425,7 +431,17 @@ def _shard_range(n, shard):
 
 def _check_csr_request(out, dtype, host_out=None, path=None, compress=False):
     """out="csr" takes int64 (default) or int32 data and no preallocated host_out; path needs out="csr";
-    compress needs both."""
+    compress needs both.  out="mtx" needs path, takes int64 or int32 and neither host_out nor compress."""
+    if out == "mtx":
+        if path is None:
+            raise ValueError("out='mtx' writes a 10x directory: it needs path=")
+        if compress:
+            raise ValueError("out='mtx' always gzips its files: compress=True does not apply")
+        if host_out is not None:
+            raise ValueError("host_out cannot be combined with out='mtx'")
+        if np.dtype(dtype) not in (np.dtype(np.int64), np.dtype(np.int32)):
+            raise ValueError("out='mtx' takes dtype int64 or int32, not %s" % np.dtype(dtype))
+        return
     if compress and (path is None or out != "csr"):
         raise ValueError("compress=True writes a compressed CSR file: it needs out='csr' and path=")
     if path is not None and out != "csr":
@@ -447,11 +463,19 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
     out="csr" with `path`: the chunks go to a CSR shard at path (CountEngine.stream_csr into a
     formats.CsrShardWriter, which also stores `cells` = (pseudotime, branches, scalings) host arrays) and the
     shard's memory-mapped matrix is returned; with `compress`, into one compressed file (formats.CsrNpzWriter,
-    stream_csr(compress=True)), and its formats.CompressedCsr record is returned."""
+    stream_csr(compress=True)), and its formats.CompressedCsr record is returned.
+    out="mtx": the chunks go to a 10x directory at path (stream_csr(mtx=True) into a formats.MtxWriter, whose
+    barcodes count from the global cell index `first`), and its formats.MtxRecord is returned."""
     if out == "torch":
         X = engine.draw(rows, s32, seed, first)
         engine.check()
         return X
+    if out == "mtx":
+        _check_csr_request(out, dtype, path=path)
+        with MtxWriter(path, (int(rows.numel()), engine.G), *cells, first=first) as w:
+            engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *text: w.append(hi - lo, text[3], *text[:3]),
+                              mtx=True)
+        return w.record()
     if out == "csr":
         _check_csr_request(out, dtype)
         n = int(rows.numel())
@@ -536,7 +560,9 @@ def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, s
     `uniforms` (one per cell) replays externally supplied draws through the index map.
     host_transport ("direct", "i32", "u16", "u8"; with host_out): the format in which the counts cross
     PCIe; the narrow ones are expanded into the int32 / int64 host matrix by `host_threads` host threads
-    (0 = all) together with their exact overflow list - the caller receives the same counts either way."""
+    (0 = all) together with their exact overflow list - the caller receives the same counts either way.
+    out="csr" / "mtx", path, compress: the sparse and on-disk forms of the module docstring; out="mtx",
+    path="counts_10x" writes a 10x directory and returns its formats.MtxRecord."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
@@ -575,7 +601,8 @@ def cover_whole_tree(tree):
 def sample_whole_tree(tree, n_factor, alpha=0.3, beta=2, scale=True, scale_mean=0., scale_v=0.7,
                       seed=None, device=None, shard=None, dtype=np.int64, out="numpy",
                       sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
-    """Every tree position sampled n_factor times (simulation.py:474-517)."""
+    """Every tree position sampled n_factor times (simulation.py:474-517).  out / path / compress: see
+    sample_density."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
@@ -613,7 +640,7 @@ def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, b
                              scale_mean=0, scale_v=0.7, seed=None, device=None, shard=None,
                              dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
     """Time-series experiment: normally distributed pseudotimes around each sample point,
-    branches picked by density (simulation.py:319-379)."""
+    branches picked by density (simulation.py:319-379).  out / path / compress: see sample_density."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     series_points, cells, point_std = sut.process_timeseries_input(series_points, cells, point_std)
@@ -643,7 +670,8 @@ def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, b
 def sample_whole_tree_restricted(tree, alpha=0.2, beta=3, seed=None, device=None, dtype=np.int64,
                                  out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
     """Bare-bones run with default lineage parameters (simulation.py:289-316): one cell
-    per pseudotime value, random branch, per-gene alpha/beta around the given means."""
+    per pseudotime value, random branch, per-gene alpha/beta around the given means.  out / path / compress:
+    see sample_density."""
     sample_time = np.arange(0, tree.get_max_time())
     tree.default_gene_expression()
     alphas, betas = cm.generate_negbin_params(tree, mean_alpha=alpha, mean_beta=beta)
@@ -657,7 +685,7 @@ def _sample_data_at_times(tree, sample_pt, branches=None, alpha=0.3, beta=2, sca
                           out="numpy", sampler=DEFAULT_SAMPLER, _first=0, path=None, compress=False):
     """Cells at given pseudotimes (simulation.py:551-599): pick branches if they are not
     supplied, draw library sizes, draw counts.  `_first` is the global index of the first
-    cell (sharded callers)."""
+    cell (sharded callers).  out / path / compress: see sample_density."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
@@ -701,7 +729,8 @@ def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, de
     (simulation.py:602-651): X[n,g] ~ NB(mean = means[branch_n][t_n - start, g]*scaling_n,
     variance = alpha_g mean^2 + beta_g mean).  out="csr", path=p writes the CSR shard with the
     pseudotime, branches and scalings given here and returns its memory-mapped matrix; with compress=True the
-    compressed file, and its formats.CompressedCsr record."""
+    compressed file, and its formats.CompressedCsr record.  out="mtx", path=p writes the 10x directory with
+    them (barcodes cell_<first + i>) and returns its formats.MtxRecord."""
     dev = nat.device(device)
     _check_csr_request(out, dtype, path=path, compress=compress)
     seed = nat.split_seed(seed)

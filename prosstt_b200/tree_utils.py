@@ -92,12 +92,17 @@ def _names(prefix, n):
     return [prefix + str(i) for i in range(n)]
 
 
+def cell_params_frame(labs, brns, scalings, index=None):
+    """The frame of the _cellparams.txt file: pseudotime, branches and scalings per cell, indexed by the cell
+    names (cell_0, cell_1, ... unless `index` names them)."""
+    cols = ["pseudotime", "branches", "scalings"]
+    return pd.DataFrame({"pseudotime": labs, "branches": brns, "scalings": scalings},
+                        index=_names("cell_", len(labs)) if index is None else index, columns=cols)
+
+
 def save_cell_params(job_id, save_dir, labs, brns, scalings):
     """<save_dir>/<job_id>_cellparams.txt (tree_utils.py:59-83)."""
-    cols = ["pseudotime", "branches", "scalings"]
-    frame = pd.DataFrame({"pseudotime": labs, "branches": brns, "scalings": scalings},
-                         index=_names("cell_", len(labs)), columns=cols)
-    frame.to_csv(save_dir + "/" + job_id + "_cellparams.txt", sep="\t")
+    cell_params_frame(labs, brns, scalings).to_csv(save_dir + "/" + job_id + "_cellparams.txt", sep="\t")
 
 
 def save_gene_params(job_id, save_dir, gene_scale, alpha, beta):
