@@ -313,6 +313,18 @@ int64_t pst_deflate_workspace_bytes(int64_t n, int32_t block);
 int pst_deflate_blocks(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes, int32_t block,
                        void *out, int64_t *out_bytes, uint32_t *crc, void *work, int64_t work_bytes,
                        void *stream);
+/* LZ77 + Huffman (`compression="lz77"`): the contract of pst_deflate_blocks, with the full DEFLATE
+ * alphabet in each dynamic block - literal/length symbols 0-285 and distance codes 0-29, both at most 15
+ * bits.  Matches (3-258 bytes) reach back at most to the start of their own block, so each block still
+ * decodes on its own and the same framing, bound and CRC hold.  The match search is deterministic: the
+ * nearest-first hash chain of each position, at most 8 candidates, and a greedy parse of 512-byte
+ * segments (a match is cut at its segment's end).  The same bytes and block give the same output.
+ * work: device workspace of pst_deflate_lz_workspace_bytes(max_bytes, block) bytes (that of
+ * pst_deflate_blocks plus 2 bytes per input byte for the tokens). */
+int64_t pst_deflate_lz_workspace_bytes(int64_t n, int32_t block);
+int pst_deflate_lz_blocks(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes, int32_t block,
+                          void *out, int64_t *out_bytes, uint32_t *crc, void *work, int64_t work_bytes,
+                          void *stream);
 /* *crc = CRC-32 (zlib.crc32) of the n device bytes at in; crc is a device word. */
 int pst_crc32(const void *in, int64_t n, uint32_t *crc, void *stream);
 

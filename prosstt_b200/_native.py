@@ -68,6 +68,8 @@ _SIGNATURES = {
     "pst_deflate_bound": (_i64, [_i64, _i32]),
     "pst_deflate_workspace_bytes": (_i64, [_i64, _i32]),
     "pst_deflate_blocks": (C.c_int, [_p, _p, _i64, _i64, _i32, _p, _p, _p, _p, _i64, _p]),
+    "pst_deflate_lz_workspace_bytes": (_i64, [_i64, _i32]),
+    "pst_deflate_lz_blocks": (C.c_int, [_p, _p, _i64, _i64, _i32, _p, _p, _p, _p, _i64, _p]),
     "pst_crc32": (C.c_int, [_p, _i64, _p, _p]),
     "pst_host_crc32_combine": (_u32, [_u32, _u32, _i64]),
     "pst_narrow_counts": (C.c_int, [_p, _i64, _i64, _i64, _p, _i64, _i32, _i64, _p, _p, _i64, _p, _p]),

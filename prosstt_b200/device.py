@@ -218,6 +218,9 @@ _NP_TO_TORCH = {np.dtype(np.int32): torch.int32, np.dtype(np.int64): torch.int64
 _STAGE_BYTES = int(os.environ.get("PST_STAGE_MB", "256")) << 20   # one pinned staging buffer (two per device)
 _STAGING = {}
 _DEFLATE_BLOCK = 32768                        # bytes per DEFLATE block of the compressed CSR file (at most 32 KiB)
+# stream_csr's `compression`: the device compressor and its workspace size
+_DEFLATE = {"huffman": ("pst_deflate_blocks", "pst_deflate_workspace_bytes"),
+            "lz77": ("pst_deflate_lz_blocks", "pst_deflate_lz_workspace_bytes")}
 
 
 _AUTO_STATE = {"narrow_overflowed": False}     # an automatically chosen uint8 transport overflowed its list once
@@ -600,7 +603,7 @@ class CountEngine(object):
         return indptr, indices, data
 
     def stream_csr(self, rows, scaling32, seed, cell0, consume, index_dtype=np.int64, data_dtype=np.int64,
-                   chunk_cells=None, threads=0, overflow_cap=None, compress=False, mtx=False):
+                   chunk_cells=None, threads=0, overflow_cap=None, compress=False, mtx=False, compression="huffman"):
         """Sample the cells in chunks and hand each one as CSR to consume(lo, hi, indptr, indices, data), on a
         worker thread, once per chunk, in cell order.  indptr is chunk-local int64 (hi - lo + 1 entries from 0);
         indices and data are the chunk's nonzeros in `index_dtype` / `data_dtype` (int32 or int64), columns
@@ -638,11 +641,19 @@ class CountEngine(object):
         text buffer holds _mtx_slot_bytes per gene slot (every count of up to 3 digits); a chunk
         with more text is not formatted (pst_mtx_format writes nothing), and when the host reads its text length
         one chunk late the buffers grow and the chunk is formatted and compressed again from its work buffer,
-        which survives until chunk i+2 is drawn - there is no redraw."""
+        which survives until chunk i+2 is drawn - there is no redraw.
+
+        compression ("huffman" or "lz77", with compress=True or mtx=True): the device compressor,
+        pst_deflate_blocks (Huffman-only) or pst_deflate_lz_blocks (LZ77 matches within each 32 KiB block,
+        smaller output, a larger workspace).  Both write the same framing, so the consumer is the same."""
         index_dtype, data_dtype = np.dtype(index_dtype), np.dtype(data_dtype)
         for what, dt in (("indices", index_dtype), ("data", data_dtype)):
             if dt not in (np.dtype(np.int32), np.dtype(np.int64)):
                 raise ValueError("CSR %s must be int32 or int64, not %s" % (what, dt))
+        if compression not in _DEFLATE:
+            raise ValueError("compression must be 'huffman' or 'lz77', not %r" % (compression,))
+        deflate, deflate_work = _DEFLATE[compression]
+        tokens = 2 if compression == "lz77" else 0       # the LZ workspace's token bytes per input byte
         n, G, dev = int(rows.numel()), self.G, self.dev
         if not threads:
             threads = _host_threads()
@@ -662,12 +673,14 @@ class CountEngine(object):
         ibytes = ibits // 8
         if mtx:
             slot = _mtx_slot_bytes(G, n)
-            # the text of a chunk and its compressed form, bounded by about as many bytes again
-            chunk, bounds = _plan_chunks(n, chunk_cells, 2 * slot * G, _STAGE_BYTES)
+            # the text of a chunk and its compressed form, bounded by about as many bytes again, and the tokens
+            chunk, bounds = _plan_chunks(n, chunk_cells, (2 + tokens) * slot * G, _STAGE_BYTES)
         elif compress:
             isz, dsz = index_dtype.itemsize, data_dtype.itemsize
-            # the wide streams of a chunk and their compressed form, bounded by about as many bytes again
-            chunk, bounds = _plan_chunks(n, chunk_cells, 2 * (isz + dsz) * G, _STAGE_BYTES)
+            # the wide streams of a chunk and their compressed form, bounded by about as many bytes again, and
+            # the tokens of the largest stream
+            chunk, bounds = _plan_chunks(n, chunk_cells, (2 * (isz + dsz) + tokens * max(isz, dsz)) * G,
+                                         _STAGE_BYTES)
         else:
             chunk, bounds = _plan_chunks(n, chunk_cells, (ibytes + 2) * G, _STAGE_BYTES)
         st = nat.stream_ptr(dev)
@@ -722,7 +735,7 @@ class CountEngine(object):
                 if cap > buf["cap"]:
                     buf["cap"] = cap
                     buf["text"] = torch.empty(max(16, cap), dtype=torch.uint8, device=dev)
-                    buf["work_bytes"] = int(lib.pst_deflate_workspace_bytes(cap, block))
+                    buf["work_bytes"] = int(getattr(lib, deflate_work)(cap, block))
                     buf["work"] = torch.empty(max(1, buf["work_bytes"]), dtype=torch.uint8, device=dev)
                 bound = int(lib.pst_deflate_bound(buf["cap"], block))
                 if packed[k] is None or packed[k].numel() < bound:
@@ -733,7 +746,7 @@ class CountEngine(object):
                 reserve(k, buf["cap"])
                 formatted_cap[k] = buf["cap"]
                 nat.call("pst_mtx_format", work[k], cells, G, G, lo, text_ptr[k], buf["cap"], buf["text"], st)
-                nat.call("pst_deflate_blocks", buf["text"], text_ptr[k][cells:cells + 1], 1, buf["cap"], block,
+                nat.call(deflate, buf["text"], text_ptr[k][cells:cells + 1], 1, buf["cap"], block,
                          packed[k], info[k, 4], info[k, 5].data_ptr(), buf["work"], buf["work_bytes"], st)
 
             reserve(0, chunk * G * slot)
@@ -772,7 +785,7 @@ class CountEngine(object):
                     torch.empty(max(1, chunk * G * dsz), dtype=torch.uint8, device=dev)]
             bound = [int(lib.pst_deflate_bound(w.numel(), block)) for w in wide]
             packed = [[torch.empty(b, dtype=torch.uint8, device=dev) for b in bound] for _ in range(2)]
-            dwork_bytes = max(int(lib.pst_deflate_workspace_bytes(w.numel(), block)) for w in wide)
+            dwork_bytes = max(int(getattr(lib, deflate_work)(w.numel(), block)) for w in wide)
             dwork = torch.empty(dwork_bytes, dtype=torch.uint8, device=dev)
             running = torch.zeros(1, dtype=torch.int64, device=dev)     # nonzeros of the chunks before
             stage_host = _pinned_staging(dev, sum(bound) + 3 * 64)
@@ -788,7 +801,7 @@ class CountEngine(object):
                 nnz = indptr[k][cells:cells + 1]
                 for j, (count, scale, most) in enumerate(((None, 0, cells * isz), (nnz, isz, cells * G * isz),
                                                           (nnz, dsz, cells * G * dsz))):
-                    nat.call("pst_deflate_blocks", wide[j], count, scale, most, block, packed[k][j], info[k, 3 + j],
+                    nat.call(deflate, wide[j], count, scale, most, block, packed[k][j], info[k, 3 + j],
                              info[k, 6 + j].data_ptr(), dwork, dwork_bytes, st)   # the CRC: low word of a zeroed int64
                 record(k, cells)
 

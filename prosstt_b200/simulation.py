@@ -31,6 +31,9 @@ Extra keyword-only arguments (never required):
            and compresses every chunk, so only gzipped text crosses PCIe and reaches the disk.  X is then a
            formats.MtxRecord (path, shape, nnz, nbytes, load()); the counts are those of out="csr".  The file is
            always gzipped (compress=True is an error), and dtype must be int64 or int32 as for "csr"
+  compression  "huffman" (default) or "lz77", where the GPU compresses (compress=True, out="mtx"): "lz77" adds
+           LZ77 matches within each 32 KiB DEFLATE block (pst_deflate_lz_blocks), so the same content is written
+           in a smaller file; "huffman" writes Huffman-only blocks.  Both files decompress to the same bytes
   sampler  "hybrid" (default): direct inversion of the NB cdf for mean <= 32, sd <= 20, gamma scale <= 32 and
            shape <= 48 - in fp32 below the 1 - 2^-14 quantile of its uniform, with a 64-bit uniform against an
            fp64-accumulated cdf above it, so body and far tail match the exact pmf (checked at 1e9 draws per
@@ -429,9 +432,15 @@ def _shard_range(n, shard):
     return shard_range(n, rank, world)
 
 
-def _check_csr_request(out, dtype, host_out=None, path=None, compress=False):
+def _check_csr_request(out, dtype, host_out=None, path=None, compress=False, compression="huffman"):
     """out="csr" takes int64 (default) or int32 data and no preallocated host_out; path needs out="csr";
-    compress needs both.  out="mtx" needs path, takes int64 or int32 and neither host_out nor compress."""
+    compress needs both.  out="mtx" needs path, takes int64 or int32 and neither host_out nor compress.
+    compression is "huffman" or "lz77"; "lz77" only where the GPU compresses (compress=True or out="mtx")."""
+    if compression not in ("huffman", "lz77"):
+        raise ValueError("compression must be 'huffman' or 'lz77', not %r" % (compression,))
+    if compression == "lz77" and out != "mtx" and not compress:
+        raise ValueError("compression='lz77' applies where the GPU compresses: out='csr', path=, compress=True "
+                         "or out='mtx', path=")
     if out == "mtx":
         if path is None:
             raise ValueError("out='mtx' writes a 10x directory: it needs path=")
@@ -454,7 +463,8 @@ def _check_csr_request(out, dtype, host_out=None, path=None, compress=False):
         raise ValueError("out='csr' stores int64 or int32 counts, not %s" % np.dtype(dtype))
 
 
-def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=None, compress=False):
+def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=None, compress=False,
+                   compression="huffman"):
     """The count matrix of the cells described by rows/s32: a device int32 tensor (out="torch"), a
     scipy.sparse.csr_matrix with `dtype` data (out="csr", CountEngine.draw_to_csr: only the nonzeros cross
     PCIe) or a fresh host array of `dtype` (reference: int64, simulation.py:651).  The host forms never hold
@@ -465,7 +475,8 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
     shard's memory-mapped matrix is returned; with `compress`, into one compressed file (formats.CsrNpzWriter,
     stream_csr(compress=True)), and its formats.CompressedCsr record is returned.
     out="mtx": the chunks go to a 10x directory at path (stream_csr(mtx=True) into a formats.MtxWriter, whose
-    barcodes count from the global cell index `first`), and its formats.MtxRecord is returned."""
+    barcodes count from the global cell index `first`), and its formats.MtxRecord is returned.  `compression`
+    picks the device compressor of both compressed forms (stream_csr)."""
     if out == "torch":
         X = engine.draw(rows, s32, seed, first)
         engine.check()
@@ -474,7 +485,7 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
         _check_csr_request(out, dtype, path=path)
         with MtxWriter(path, (int(rows.numel()), engine.G), *cells, first=first) as w:
             engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *text: w.append(hi - lo, text[3], *text[:3]),
-                              mtx=True)
+                              mtx=True, compression=compression)
         return w.record()
     if out == "csr":
         _check_csr_request(out, dtype)
@@ -482,7 +493,7 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
         if path is not None and compress:
             with CsrNpzWriter(path, (n, engine.G), *cells, dtype=dtype) as w:
                 engine.stream_csr(rows, s32, seed, first, lambda lo, hi, parts: [w.append(*p) for p in parts],
-                                  w.index_dtype, dtype, compress=True)
+                                  w.index_dtype, dtype, compress=True, compression=compression)
             return w.record()
         if path is not None:
             with CsrShardWriter(path, (n, engine.G), *cells, dtype=dtype) as shard:
@@ -508,7 +519,7 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
 
 def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
                     seed, first, dev, dtype, out, sampler, host_out=None, host_transport=None, host_threads=0,
-                    path=None, compress=False):
+                    path=None, compress=False, compression="huffman"):
     """Common tail of every sampler (simulation.py:590-599): scalings, then counts.
     host_out = (X, pseudotime, branch_codes, scalings) preallocated CPU tensors (int32 (n,G),
     int64, int32, float64; ideally pinned): the counts are streamed into them in cell chunks
@@ -517,7 +528,7 @@ def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mea
     and a fifth entry of host_out, a dict, receives the exact values of the saturated elements as
     "index" (flat, into X) and "value" arrays (formats.widen rebuilds the int32 matrix); without
     the dict a saturated element raises OverflowError instead of passing silently."""
-    _check_csr_request(out, dtype, host_out, path, compress)
+    _check_csr_request(out, dtype, host_out, path, compress, compression)
     n = int(rows.numel())
     s64, s32 = sut.calc_scalings(n, scale, scale_mean, scale_v, seed=nat.derive_seed(seed, 1),
                                  first=first, device=dev, return_device=True)
@@ -547,21 +558,21 @@ def _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mea
         return _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out), pt, codes, s64
     cells = pt.cpu().numpy(), tables.branch_names(codes.cpu().numpy()), s64.cpu().numpy()
     X = _sample_counts(engine, rows, s32, nat.derive_seed(seed, 2), first, dtype, out, path=path, cells=cells,
-                       compress=compress)
+                       compress=compress, compression=compression)
     return (X,) + cells
 
 
 def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, scale_mean=0.,
                    seed=None, device=None, shard=None, dtype=np.int64, out="numpy",
                    sampler=DEFAULT_SAMPLER, uniforms=None, host_out=None, host_transport=None, host_threads=0, *,
-                   path=None, compress=False):
+                   path=None, compress=False, compression="huffman"):
     """Sample `no_cells` (pseudotime, branch) pairs according to tree.density and draw
     their counts (simulation.py:416-471).  Returns (X, pseudotime, branches, scalings).
     `uniforms` (one per cell) replays externally supplied draws through the index map.
     host_transport ("direct", "i32", "u16", "u8"; with host_out): the format in which the counts cross
     PCIe; the narrow ones are expanded into the int32 / int64 host matrix by `host_threads` host threads
     (0 = all) together with their exact overflow list - the caller receives the same counts either way.
-    out="csr" / "mtx", path, compress: the sparse and on-disk forms of the module docstring; out="mtx",
+    out="csr" / "mtx", path, compress, compression: the sparse and on-disk forms of the module docstring; out="mtx",
     path="counts_10x" writes a 10x directory and returns its formats.MtxRecord."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
@@ -582,7 +593,7 @@ def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, s
              nat.ptr(tables.d("pos_branch")), nat.ptr(rows), nat.ptr(pt), nat.ptr(codes), st)
     return _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
                            seed, lo, dev, dtype, out, sampler, host_out=host_out, host_transport=host_transport,
-                           host_threads=host_threads, path=path, compress=compress)
+                           host_threads=host_threads, path=path, compress=compress, compression=compression)
 
 
 def cover_whole_tree(tree):
@@ -600,9 +611,9 @@ def cover_whole_tree(tree):
 
 def sample_whole_tree(tree, n_factor, alpha=0.3, beta=2, scale=True, scale_mean=0., scale_v=0.7,
                       seed=None, device=None, shard=None, dtype=np.int64, out="numpy",
-                      sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
-    """Every tree position sampled n_factor times (simulation.py:474-517).  out / path / compress: see
-    sample_density."""
+                      sampler=DEFAULT_SAMPLER, *, path=None, compress=False, compression="huffman"):
+    """Every tree position sampled n_factor times (simulation.py:474-517).  out / path / compress /
+    compression: see sample_density."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
@@ -616,7 +627,7 @@ def sample_whole_tree(tree, n_factor, alpha=0.3, beta=2, scale=True, scale_mean=
              nat.ptr(tables.d("cover_row")), len(tables.cover_pt), int(n_factor), lo, n,
              nat.ptr(pt), nat.ptr(codes), nat.ptr(rows), nat.stream_ptr(dev))
     return _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
-                           seed, lo, dev, dtype, out, sampler, path=path, compress=compress)
+                           seed, lo, dev, dtype, out, sampler, path=path, compress=compress, compression=compression)
 
 
 def draw_times(timepoint, no_cells, max_time, var=4, seed=None, first=0, device=None,
@@ -638,9 +649,11 @@ def draw_times(timepoint, no_cells, max_time, var=4, seed=None, first=0, device=
 
 def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, beta=2, scale=True,
                              scale_mean=0, scale_v=0.7, seed=None, device=None, shard=None,
-                             dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
+                             dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False,
+                             compression="huffman"):
     """Time-series experiment: normally distributed pseudotimes around each sample point,
-    branches picked by density (simulation.py:319-379).  out / path / compress: see sample_density."""
+    branches picked by density (simulation.py:319-379).  out / path / compress / compression: see
+    sample_density."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     series_points, cells, point_std = sut.process_timeseries_input(series_points, cells, point_std)
@@ -664,28 +677,31 @@ def sample_pseudotime_series(tree, cells, series_points, point_std, alpha=0.3, b
         nat.call("pst_times_from_normals", nat.ptr(z), n, int(max_time), nat.ptr(pt), st)
     return _sample_data_at_times(tree, pt, alpha=alpha, beta=beta, scale=scale, scale_mean=scale_mean,
                                  scale_v=scale_v, seed=nat.derive_seed(seed, 3), device=dev,
-                                 dtype=dtype, out=out, sampler=sampler, _first=lo, path=path, compress=compress)
+                                 dtype=dtype, out=out, sampler=sampler, _first=lo, path=path, compress=compress,
+                                 compression=compression)
 
 
 def sample_whole_tree_restricted(tree, alpha=0.2, beta=3, seed=None, device=None, dtype=np.int64,
-                                 out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False):
+                                 out="numpy", sampler=DEFAULT_SAMPLER, *, path=None, compress=False,
+                                 compression="huffman"):
     """Bare-bones run with default lineage parameters (simulation.py:289-316): one cell
-    per pseudotime value, random branch, per-gene alpha/beta around the given means.  out / path / compress:
-    see sample_density."""
+    per pseudotime value, random branch, per-gene alpha/beta around the given means.  out / path / compress /
+    compression: see sample_density."""
     sample_time = np.arange(0, tree.get_max_time())
     tree.default_gene_expression()
     alphas, betas = cm.generate_negbin_params(tree, mean_alpha=alpha, mean_beta=beta)
     return _sample_data_at_times(tree, sample_time, alpha=alphas, beta=betas, seed=seed,
                                  device=device, dtype=dtype, out=out, sampler=sampler, path=path,
-                                 compress=compress)
+                                 compress=compress, compression=compression)
 
 
 def _sample_data_at_times(tree, sample_pt, branches=None, alpha=0.3, beta=2, scale=True,
                           scale_mean=0., scale_v=0.7, seed=None, device=None, dtype=np.int64,
-                          out="numpy", sampler=DEFAULT_SAMPLER, _first=0, path=None, compress=False):
+                          out="numpy", sampler=DEFAULT_SAMPLER, _first=0, path=None, compress=False,
+                          compression="huffman"):
     """Cells at given pseudotimes (simulation.py:551-599): pick branches if they are not
     supplied, draw library sizes, draw counts.  `_first` is the global index of the first
-    cell (sharded callers).  out / path / compress: see sample_density."""
+    cell (sharded callers).  out / path / compress / compression: see sample_density."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
@@ -701,7 +717,8 @@ def _sample_data_at_times(tree, sample_pt, branches=None, alpha=0.3, beta=2, sca
     # the index map's own status word is read after the draw has been queued (no stall in front of it)
     try:
         result = _draw_for_cells(tree, tables, pt, codes, rows, alpha, beta, scale, scale_mean, scale_v,
-                                 seed, _first, dev, dtype, out, sampler, path=path, compress=compress)
+                                 seed, _first, dev, dtype, out, sampler, path=path, compress=compress,
+                                 compression=compression)
     except IndexError:
         sut.check_flags(flags)
         raise
@@ -724,15 +741,16 @@ def _rows_for(tables, pt, branches, dev):
 
 
 def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, device=None,
-                dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, first=0, *, path=None, compress=False):
+                dtype=np.int64, out="numpy", sampler=DEFAULT_SAMPLER, first=0, *, path=None, compress=False,
+                compression="huffman"):
     """UMI counts of cells at (pseudotime, branch) with library sizes `scalings`
     (simulation.py:602-651): X[n,g] ~ NB(mean = means[branch_n][t_n - start, g]*scaling_n,
     variance = alpha_g mean^2 + beta_g mean).  out="csr", path=p writes the CSR shard with the
     pseudotime, branches and scalings given here and returns its memory-mapped matrix; with compress=True the
     compressed file, and its formats.CompressedCsr record.  out="mtx", path=p writes the 10x directory with
-    them (barcodes cell_<first + i>) and returns its formats.MtxRecord."""
+    them (barcodes cell_<first + i>) and returns its formats.MtxRecord.  compression="lz77": see sample_density."""
     dev = nat.device(device)
-    _check_csr_request(out, dtype, path=path, compress=compress)
+    _check_csr_request(out, dtype, path=path, compress=compress, compression=compression)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
     pt = pseudotime if isinstance(pseudotime, torch.Tensor) else \
@@ -749,7 +767,8 @@ def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, de
     if path is not None:
         given = scalings.detach().cpu().numpy() if isinstance(scalings, torch.Tensor) else scalings
         cells = pt.cpu().numpy(), tables.branch_names(codes.cpu().numpy()), np.asarray(given, dtype=np.float64)
-    return _sample_counts(engine, rows, s32, seed, first, dtype, out, path=path, cells=cells, compress=compress)
+    return _sample_counts(engine, rows, s32, seed, first, dtype, out, path=path, cells=cells, compress=compress,
+                          compression=compression)
 
 
 def add_non_diff_genes(inform_expr_matrix, genes, gene_params, cell_scalings, seed=None,
