@@ -12,6 +12,7 @@ import torch
 
 from prosstt_b200 import _native as nat
 from prosstt_b200 import hostpool
+from prosstt_b200.formats import sync_deflate
 
 
 def tree_tables(tree, dev):
@@ -218,9 +219,12 @@ _NP_TO_TORCH = {np.dtype(np.int32): torch.int32, np.dtype(np.int64): torch.int64
 _STAGE_BYTES = int(os.environ.get("PST_STAGE_MB", "256")) << 20   # one pinned staging buffer (two per device)
 _STAGING = {}
 _DEFLATE_BLOCK = 32768                        # bytes per DEFLATE block of the compressed CSR file (at most 32 KiB)
-# stream_csr's `compression`: the device compressor and its workspace size
-_DEFLATE = {"huffman": ("pst_deflate_blocks", "pst_deflate_workspace_bytes"),
-            "lz77": ("pst_deflate_lz_blocks", "pst_deflate_lz_workspace_bytes")}
+# stream_csr's `compression`: the device compressor, its workspace size and the workspace's token bytes per input byte
+_DEFLATE = {"huffman": ("pst_deflate_blocks", "pst_deflate_workspace_bytes", 0),
+            "lz77": ("pst_deflate_lz_blocks", "pst_deflate_lz_workspace_bytes", 2)}
+# stream_csr's per-chunk record of int64 slots, read by the host one chunk late: those of every format, then its own
+_REC_SAT, _REC_NNZ, _REC_STATUS, _REC_OWN = range(4)
+_REC_SLOTS = _REC_OWN + 6                     # the .npz has the most slots of its own
 
 
 _AUTO_STATE = {"narrow_overflowed": False}     # an automatically chosen uint8 transport overflowed its list once
@@ -610,38 +614,21 @@ class CountEngine(object):
         ascending in every row.  They are reused host buffers, valid during the call only.  Returns the total
         nnz.  Concatenated over the chunks, the arrays are draw_to_csr's, so the counts are those of draw().
 
-        Nothing is sized by the whole matrix, and every chunk is drawn once.  Chunk i is drawn into int32 work
-        buffer k = i & 1.  pst_csr_row_counts and pst_csr_row_offsets give its chunk-local row pointer and its
-        count of values >= 65535, and pst_csr_pack writes it at once into device staging k: a uint16 column
-        stream (int32 when G > 65536) and, at the fixed offset of chunk x G column entries, a uint16 value
-        stream, plus the saturated values in overflow list k.  The chunk's (saturated, nnz, status word) reach
-        pinned memory by a small async copy, which the host reads one chunk late, once chunk i+1 is queued
-        (_copy_chunks' collect).  Only then are chunk i's copies queued, sized to its nnz: 4 B per nonzero
-        over PCIe while G <= 65536.  A chunk with more saturated values than its list holds (overflow_cap
-        entries at first) grows the list and is packed again from its work buffer, which survives until chunk
-        i+2 is drawn.  An error in the status word raises as draw() would (raise_flags) and ends the stream.
+        Nothing is sized by the whole matrix, and every chunk is drawn once, into int32 work buffer k = i & 1,
+        which survives until chunk i+2 is drawn: a chunk that did not fit a device buffer of k is encoded again
+        from it.  The host reads the chunk's record (_REC_*) one chunk late (_copy_chunks' collect); an error in
+        its status word raises as draw() would (raise_flags) and ends the stream.
 
         compress=True: consume(lo, hi, parts) receives the chunk compressed instead, parts = [(member,
         compressed, crc, raw_len)] for "indptr", "indices" and "data" in the order formats.CsrNpzWriter.append
         takes them: `compressed` (a reused uint8 host buffer) is raw DEFLATE that decompresses to the raw_len
         bytes of the member's part, whose CRC-32 is crc.  indptr is the chunk's row ends in index_dtype, offset
-        by the nonzeros of the chunks before it (the file's leading 0 is not included).  The device does all of
-        it, on the sampling stream and with no host wait: pst_csr_pack writes the final index_dtype /
-        data_dtype bytes (no saturation, no re-pack), pst_csr_indptr_bytes the indptr bytes with a running nnz
-        kept on the device, and pst_deflate_blocks compresses each member, reading its length from the device.
-        The host reads (nnz, status word, compressed sizes, CRCs) one chunk late as above and copies exactly
-        the compressed bytes.
+        by the nonzeros of the chunks before it (the file's leading 0 is not included).
 
         mtx=True: consume(lo, hi, compressed, crc, text_len, nnz) receives the chunk as Matrix Market text
         (formats.MtxWriter.append): `compressed` (a reused uint8 host buffer) is raw DEFLATE that decompresses to
         the text_len bytes of the chunk's nnz lines "<g+1> <c+1> <v>\n", c = lo + row within the chunk, whose
-        CRC-32 is crc; index_dtype and data_dtype do not apply.  Per chunk, on the sampling stream with no host
-        wait: the draw and the row pointer as above, pst_mtx_row_bytes and pst_csr_row_offsets (the chunk's text
-        pointer), pst_mtx_format into the text buffer and pst_deflate_blocks over text_ptr[n] bytes of it.  The
-        text buffer holds _mtx_slot_bytes per gene slot (every count of up to 3 digits); a chunk
-        with more text is not formatted (pst_mtx_format writes nothing), and when the host reads its text length
-        one chunk late the buffers grow and the chunk is formatted and compressed again from its work buffer,
-        which survives until chunk i+2 is drawn - there is no redraw.
+        CRC-32 is crc; index_dtype and data_dtype do not apply.
 
         compression ("huffman" or "lz77", with compress=True or mtx=True): the device compressor,
         pst_deflate_blocks (Huffman-only) or pst_deflate_lz_blocks (LZ77 matches within each 32 KiB block,
@@ -652,83 +639,193 @@ class CountEngine(object):
                 raise ValueError("CSR %s must be int32 or int64, not %s" % (what, dt))
         if compression not in _DEFLATE:
             raise ValueError("compression must be 'huffman' or 'lz77', not %r" % (compression,))
-        deflate, deflate_work = _DEFLATE[compression]
-        tokens = 2 if compression == "lz77" else 0       # the LZ workspace's token bytes per input byte
         n, G, dev = int(rows.numel()), self.G, self.dev
-        if not threads:
-            threads = _host_threads()
         if n == 0:
             return 0
+        # an encoder gives its budget per cell, its output when G == 0 and start(), which allocates its buffers and
+        # returns step, grow (True if a buffer of k grew for the chunk), encode (what then runs again), copies, deliver
+        cell_bytes, empty, start = (
+            self._mtx_encoder(n, consume, compression) if mtx else
+            self._npz_encoder(n, consume, index_dtype, data_dtype, compression) if compress else
+            self._shard_encoder(n, consume, index_dtype, data_dtype, threads, overflow_cap))
         if G == 0:
-            from prosstt_b200.formats import sync_deflate
-            if mtx:
-                consume(0, n, *sync_deflate(b""), 0)
-            elif compress:
-                consume(0, n, [("indptr",) + sync_deflate(np.zeros(n, index_dtype).tobytes()),
-                               ("indices",) + sync_deflate(b""), ("data",) + sync_deflate(b"")])
-            else:
-                consume(0, n, np.zeros(n + 1, np.int64), np.zeros(0, index_dtype), np.zeros(0, data_dtype))
+            empty()
             return 0
-        ibits = 16 if G <= 65536 else 32                 # width of the column stream
-        ibytes = ibits // 8
-        if mtx:
-            slot = _mtx_slot_bytes(G, n)
-            # the text of a chunk and its compressed form, bounded by about as many bytes again, and the tokens
-            chunk, bounds = _plan_chunks(n, chunk_cells, (2 + tokens) * slot * G, _STAGE_BYTES)
-        elif compress:
-            isz, dsz = index_dtype.itemsize, data_dtype.itemsize
-            # the wide streams of a chunk and their compressed form, bounded by about as many bytes again, and
-            # the tokens of the largest stream
-            chunk, bounds = _plan_chunks(n, chunk_cells, (2 * (isz + dsz) + tokens * max(isz, dsz)) * G,
-                                         _STAGE_BYTES)
-        else:
-            chunk, bounds = _plan_chunks(n, chunk_cells, (ibytes + 2) * G, _STAGE_BYTES)
+        chunk, bounds = _plan_chunks(n, chunk_cells, cell_bytes, _STAGE_BYTES)
         st = nat.stream_ptr(dev)
         work = [torch.empty((chunk, G), dtype=torch.int32, device=dev) for _ in range(2)]
         row_nnz = torch.empty(chunk, dtype=torch.int32, device=dev)      # read by the scan right after the count
         indptr = [torch.empty(chunk + 1, dtype=torch.int64, device=dev) for _ in range(2)]
-        # saturated, nnz, status word; compress: the three compressed sizes and CRCs; mtx: the text length, the
-        # compressed size and the CRC
-        info = torch.zeros((2, 9), dtype=torch.int64, device=dev)
-        info_host = torch.zeros((2, 9), dtype=torch.int64).pin_memory()
-        sized = [None, None]
+        info = torch.zeros((2, _REC_SLOTS), dtype=torch.int64, device=dev)
+        info_host = torch.zeros((2, _REC_SLOTS), dtype=torch.int64).pin_memory()
         pack_flags = torch.zeros(1, dtype=torch.int32, device=dev)
         total = [0]
+        step, grow, encode, copies, deliver = start(chunk, work, indptr, info, pack_flags)
 
-        def draw_rows(k, lo, hi):
-            """Chunk [lo, hi) into work buffer k and its chunk-local row pointer into indptr[k]."""
+        def produce(k, lo, hi):
             cells = hi - lo
             self.draw(rows[lo:hi], scaling32[lo:hi], seed, cell0 + lo, out=work[k][:cells])
-            info[k].zero_()
-            nat.call("pst_csr_row_counts", work[k].data_ptr(), cells, G, G, row_nnz, info[k, 0], st)
+            info[k].zero_()                     # the compressors write each CRC into the low word of a zeroed slot
+            nat.call("pst_csr_row_counts", work[k].data_ptr(), cells, G, G, row_nnz, info[k, _REC_SAT], st)
             nat.call("pst_csr_row_offsets", row_nnz, cells, indptr[k], st)
-
-        def record(k, cells):
-            info[k, 1].copy_(indptr[k][cells])
-            info[k, 2].copy_(self.flags[0])
+            step(k, lo, cells)
+            info[k, _REC_NNZ].copy_(indptr[k][cells])
+            info[k, _REC_STATUS].copy_(self.flags[0])
             info_host[k].copy_(info[k], non_blocking=True)
-            sized[k] = torch.cuda.Event()
-            sized[k].record(torch.cuda.current_stream(dev))
 
-        def read_info(k):
-            sized[k].synchronize()
-            vals = info_host[k].tolist()
-            if vals[2]:
+        def collect(k, lo, hi):
+            record = info_host[k].tolist()
+            if record[_REC_STATUS]:
                 self.flags[0].zero_()
-                raise_flags(vals[2])
-            total[0] += vals[1]
-            return vals
+                raise_flags(record[_REC_STATUS])
+            total[0] += record[_REC_NNZ]
+            if grow(k, record):
+                encode(k, lo, hi - lo)
+                record = info[k].tolist()                # waits for it: the copies wait for the first encode only
+            return copies(k, hi - lo, record), record
 
-        if mtx:
-            lib = nat.load()
-            block = _DEFLATE_BLOCK
+        self._copy_chunks(bounds, produce, deliver, collect)
+        if int(pack_flags.item()) != 0:
+            raise RuntimeError("the packed counts do not match the row sizes of their chunk")
+        return total[0]
+
+    def _shard_encoder(self, n, consume, index_dtype, data_dtype, threads, overflow_cap):
+        """stream_csr's CSR shard.  pst_csr_pack writes chunk k into device staging k: a uint16 column stream (int32
+        when G > 65536) and, at the fixed offset of chunk x G column entries, a uint16 value stream (4 B per
+        nonzero over PCIe), plus the saturated values in overflow list k, which grows when they do not fit."""
+        G, dev, st, lib = self.G, self.dev, nat.stream_ptr(self.dev), nat.load()
+        ibytes = 2 if G <= 65536 else 4                  # bytes per entry of the column stream
+        threads = int(threads or _host_threads())
+
+        def empty():
+            consume(0, n, np.zeros(n + 1, np.int64), np.zeros(0, index_dtype), np.zeros(0, data_dtype))
+
+        def start(chunk, work, indptr, info, pack_flags):
+            value_at = (chunk * G * ibytes + 63) // 64 * 64  # the value stream, after the worst-case column stream
+            stage = [torch.empty(value_at + 2 * chunk * G, dtype=torch.uint8, device=dev) for _ in range(2)]
+            ovf = [_OverflowList(overflow_cap or (1 << 16), dev) for _ in range(2)]
+            ovf_host = [torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory() for k in range(2)]
+            # host side: the row pointer, then the streams of the nonzeros, values on a 64-byte boundary
+            stage_host = _pinned_staging(dev, 8 * (chunk + 1) + value_at + 64 + 2 * chunk * G)
+            # the widened chunk, reused from chunk to chunk (by the one worker): its pages are touched as the chunks'
+            # nnz needs them and hostpool keeps them mapped for the next call.  Past the first chunk they are mapped
+            # and out of cache, which is what the streaming stores are for.
+            indices_w = hostpool.result_array((chunk * G,), index_dtype)[0]
+            data_w = hostpool.result_array((chunk * G,), data_dtype)[0]
+            widen = lib.pst_host_widen_stream
+
+            def pack(k, lo, cells):
+                ovf[k].count.zero_()
+                nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, stage[k].data_ptr(),
+                         8 * ibytes, stage[k].data_ptr() + value_at, 16, *ovf[k].kernel_args, pack_flags, st)
+
+            def grow(k, record):
+                if record[_REC_SAT] <= ovf[k].capacity:
+                    return False
+                ovf[k] = _OverflowList(max(record[_REC_SAT], 2 * ovf[k].capacity), dev)
+                ovf_host[k] = torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory()
+                return True
+
+            def copies(k, cells, record):
+                n_sat, nnz = record[_REC_SAT], record[_REC_NNZ]
+                at = 8 * (cells + 1)
+                vat = (at + nnz * ibytes + 63) // 64 * 64
+                h = stage_host[k]
+                pairs = [(indptr[k][:cells + 1].view(torch.uint8), h[:at]),
+                         (stage[k][:nnz * ibytes], h[at:at + nnz * ibytes]),
+                         (stage[k][value_at:value_at + 2 * nnz], h[vat:vat + 2 * nnz])]
+                if n_sat:
+                    pairs += [(ovf[k].pos[:n_sat].view(torch.uint8), ovf_host[k][:8 * n_sat]),
+                              (ovf[k].value[:n_sat].view(torch.uint8), ovf_host[k][8 * n_sat:12 * n_sat])]
+                return pairs
+
+            def deliver(dsts, lo, hi, record):
+                n_sat, nnz = record[_REC_SAT], record[_REC_NNZ]
+                indices, data = indices_w[:nnz], data_w[:nnz]
+                rc = widen(dsts[1].data_ptr(), 8 * ibytes, indices.ctypes.data, 8 * index_dtype.itemsize, nnz, threads)
+                rc |= widen(dsts[2].data_ptr(), 16, data.ctypes.data, 8 * data_dtype.itemsize, nnz, threads)
+                if rc != 0:
+                    raise nat.NativeError("pst_host_widen failed")
+                if n_sat:
+                    lib.pst_host_apply_overflow(data.ctypes.data, 8 * data_dtype.itemsize, 0, nnz, dsts[3].data_ptr(),
+                                                dsts[4].data_ptr(), n_sat)
+                consume(lo, hi, dsts[0].numpy().view(np.int64), indices, data)
+
+            return pack, grow, pack, copies, deliver
+
+        return (ibytes + 2) * G, empty, start
+
+    def _npz_encoder(self, n, consume, index_dtype, data_dtype, compression):
+        """stream_csr(compress=True): pst_csr_pack writes the final index_dtype / data_dtype bytes, pst_csr_indptr_bytes
+        the indptr bytes after a running nnz kept on the device, and the compressor each member, reading its length
+        from the device.  That running nnz adds up the chunks in order, so a chunk is never encoded again."""
+        G, dev, st, lib, block = self.G, self.dev, nat.stream_ptr(self.dev), nat.load(), _DEFLATE_BLOCK
+        isz, dsz = index_dtype.itemsize, data_dtype.itemsize
+        deflate, deflate_work, tokens = _DEFLATE[compression]
+        SIZE, CRC = _REC_OWN, _REC_OWN + 3               # record: the members' compressed sizes, then their CRCs
+        members = ("indptr", "indices", "data")
+
+        def empty():
+            consume(0, n, [(m,) + sync_deflate(raw) for m, raw in zip(members, (bytes(n * isz), b"", b""))])
+
+        def start(chunk, work, indptr, info, pack_flags):
+            wide = [torch.empty(max(1, size), dtype=torch.uint8, device=dev)                # indptr, indices, data
+                    for size in (chunk * isz, chunk * G * isz, chunk * G * dsz)]
+            bound = [int(lib.pst_deflate_bound(w.numel(), block)) for w in wide]
+            packed = [[torch.empty(b, dtype=torch.uint8, device=dev) for b in bound] for _ in range(2)]
+            dwork_bytes = max(int(getattr(lib, deflate_work)(w.numel(), block)) for w in wide)
+            dwork = torch.empty(dwork_bytes, dtype=torch.uint8, device=dev)
+            running = torch.zeros(1, dtype=torch.int64, device=dev)     # nonzeros of the chunks before
+            stage_host = _pinned_staging(dev, sum(bound) + 3 * 64)
+
+            def step(k, lo, cells):
+                nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, wide[1], 8 * isz, wide[2],
+                         8 * dsz, None, None, 0, None, pack_flags, st)
+                nat.call("pst_csr_indptr_bytes", indptr[k], cells, running, wide[0], 8 * isz, st)
+                nnz = indptr[k][cells:cells + 1]
+                for j, (count, scale, most) in enumerate(((None, 0, cells * isz), (nnz, isz, cells * G * isz),
+                                                          (nnz, dsz, cells * G * dsz))):
+                    nat.call(deflate, wide[j], count, scale, most, block, packed[k][j], info[k, SIZE + j],
+                             info[k, CRC + j].data_ptr(), dwork, dwork_bytes, st)
+
+            def copies(k, cells, record):
+                pairs, at = [], 0
+                for j in range(3):
+                    size = record[SIZE + j]
+                    pairs.append((packed[k][j][:size], stage_host[k][at:at + size]))
+                    at = (at + size + 63) // 64 * 64
+                return pairs
+
+            def deliver(dsts, lo, hi, record):
+                raw = ((hi - lo) * isz, record[_REC_NNZ] * isz, record[_REC_NNZ] * dsz)
+                consume(lo, hi, [(members[j], dsts[j].numpy(), record[CRC + j] & 0xFFFFFFFF, raw[j]) for j in range(3)])
+
+            return step, (lambda k, record: False), None, copies, deliver
+
+        # the wide streams of a chunk and their compressed form, bounded by about as many bytes again, and the
+        # tokens of the largest stream
+        return (2 * (isz + dsz) + tokens * max(isz, dsz)) * G, empty, start
+
+    def _mtx_encoder(self, n, consume, compression):
+        """stream_csr(mtx=True): pst_mtx_row_bytes and pst_csr_row_offsets (the text pointer), pst_mtx_format into the
+        text buffer, shared by both k, of _mtx_slot_bytes per gene slot, and the compressor over the text.  A chunk
+        with more text is not formatted (pst_mtx_format writes nothing), and is formatted again in a larger buffer."""
+        G, dev, st, lib, block = self.G, self.dev, nat.stream_ptr(self.dev), nat.load(), _DEFLATE_BLOCK
+        deflate, deflate_work, tokens = _DEFLATE[compression]
+        slot = _mtx_slot_bytes(G, n)
+        TEXT_LEN, SIZE, CRC = range(_REC_OWN, _REC_OWN + 3)     # record: text length, compressed size, CRC
+
+        def empty():
+            consume(0, n, *sync_deflate(b""), 0)
+
+        def start(chunk, work, indptr, info, pack_flags):
             row_bytes = torch.empty(chunk, dtype=torch.int32, device=dev)
             text_ptr = [torch.empty(chunk + 1, dtype=torch.int64, device=dev) for _ in range(2)]
             buf = {"cap": -1}                             # the text buffer, its deflate workspace and capacity
             packed = [None, None]
             formatted_cap = [0, 0]                        # the capacity chunk k was formatted against
+            # a copy of the cached pair, so that growing one k leaves the cache as it is
             stage_host = list(_pinned_staging(dev, int(lib.pst_deflate_bound(chunk * G * slot, block))))
-            landed_info = {}                              # chunk start -> its record, from collect to landed
 
             def reserve(k, cap):
                 """Text buffer of at least cap bytes, and room in packed[k] for its compressed form."""
@@ -741,143 +838,43 @@ class CountEngine(object):
                 if packed[k] is None or packed[k].numel() < bound:
                     packed[k] = torch.empty(max(1, bound), dtype=torch.uint8, device=dev)
 
-            def text(k, lo, cells):
+            def encode(k, lo, cells):
                 """Format chunk k from its work buffer and compress the text."""
                 reserve(k, buf["cap"])
                 formatted_cap[k] = buf["cap"]
                 nat.call("pst_mtx_format", work[k], cells, G, G, lo, text_ptr[k], buf["cap"], buf["text"], st)
                 nat.call(deflate, buf["text"], text_ptr[k][cells:cells + 1], 1, buf["cap"], block,
-                         packed[k], info[k, 4], info[k, 5].data_ptr(), buf["work"], buf["work_bytes"], st)
+                         packed[k], info[k, SIZE], info[k, CRC].data_ptr(), buf["work"], buf["work_bytes"], st)
 
             reserve(0, chunk * G * slot)
 
-            def produce(k, lo, hi):
-                cells = hi - lo
-                draw_rows(k, lo, hi)
+            def step(k, lo, cells):
                 nat.call("pst_mtx_row_bytes", work[k], cells, G, G, lo, row_bytes, st)
                 nat.call("pst_csr_row_offsets", row_bytes, cells, text_ptr[k], st)
-                info[k, 3].copy_(text_ptr[k][cells])
-                text(k, lo, cells)
-                record(k, cells)
+                info[k, TEXT_LEN].copy_(text_ptr[k][cells])
+                encode(k, lo, cells)
 
-            def collect(k, lo, hi):
-                vals = read_info(k)
+            def grow(k, record):
                 # the text did not fit the buffer as it was when the chunk was queued: nothing was formatted.  The
                 # buffer may have grown since (for the chunk before), so the test is against that capacity.
-                if vals[3] > formatted_cap[k]:
-                    reserve(k, max(vals[3], 2 * formatted_cap[k]))
-                    text(k, lo, hi - lo)
-                    vals = info[k].tolist()               # waits for the second format: the copies wait for the first
-                size = vals[4]
+                if record[TEXT_LEN] <= formatted_cap[k]:
+                    return False
+                reserve(k, max(record[TEXT_LEN], 2 * formatted_cap[k]))
+                return True
+
+            def copies(k, cells, record):
+                size = record[SIZE]
                 if stage_host[k].numel() < size:
                     stage_host[k] = torch.empty(size, dtype=torch.uint8).pin_memory()
-                landed_info[lo] = vals
                 return [(packed[k][:size], stage_host[k][:size])]
 
-            def landed(dsts, lo, hi):
-                vals = landed_info.pop(lo)
-                consume(lo, hi, dsts[0].numpy(), vals[5] & 0xFFFFFFFF, vals[3], vals[1])
-        elif compress:
-            lib = nat.load()
-            block = _DEFLATE_BLOCK
-            wide = [torch.empty(max(1, chunk * isz), dtype=torch.uint8, device=dev),       # indptr, indices, data
-                    torch.empty(max(1, chunk * G * isz), dtype=torch.uint8, device=dev),
-                    torch.empty(max(1, chunk * G * dsz), dtype=torch.uint8, device=dev)]
-            bound = [int(lib.pst_deflate_bound(w.numel(), block)) for w in wide]
-            packed = [[torch.empty(b, dtype=torch.uint8, device=dev) for b in bound] for _ in range(2)]
-            dwork_bytes = max(int(getattr(lib, deflate_work)(w.numel(), block)) for w in wide)
-            dwork = torch.empty(dwork_bytes, dtype=torch.uint8, device=dev)
-            running = torch.zeros(1, dtype=torch.int64, device=dev)     # nonzeros of the chunks before
-            stage_host = _pinned_staging(dev, sum(bound) + 3 * 64)
-            meta_host = [torch.empty(9 * 8, dtype=torch.uint8).pin_memory() for _ in range(2)]
-            members = ("indptr", "indices", "data")
+            def deliver(dsts, lo, hi, record):
+                consume(lo, hi, dsts[0].numpy(), record[CRC] & 0xFFFFFFFF, record[TEXT_LEN], record[_REC_NNZ])
 
-            def produce(k, lo, hi):
-                cells = hi - lo
-                draw_rows(k, lo, hi)
-                nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, wide[1], 8 * isz, wide[2],
-                         8 * dsz, None, None, 0, None, pack_flags, st)
-                nat.call("pst_csr_indptr_bytes", indptr[k], cells, running, wide[0], 8 * isz, st)
-                nnz = indptr[k][cells:cells + 1]
-                for j, (count, scale, most) in enumerate(((None, 0, cells * isz), (nnz, isz, cells * G * isz),
-                                                          (nnz, dsz, cells * G * dsz))):
-                    nat.call(deflate, wide[j], count, scale, most, block, packed[k][j], info[k, 3 + j],
-                             info[k, 6 + j].data_ptr(), dwork, dwork_bytes, st)   # the CRC: low word of a zeroed int64
-                record(k, cells)
+            return step, grow, encode, copies, deliver
 
-            def collect(k, lo, hi):
-                sizes = read_info(k)[3:6]
-                pairs, at = [], 0
-                for j in range(3):
-                    pairs.append((packed[k][j][:sizes[j]], stage_host[k][at:at + sizes[j]]))
-                    at = (at + sizes[j] + 63) // 64 * 64
-                return pairs + [(info[k].view(torch.uint8), meta_host[k])]
-
-            def landed(dsts, lo, hi):
-                vals = dsts[3].view(torch.int64).tolist()
-                raw = ((hi - lo) * isz, vals[1] * isz, vals[1] * dsz)
-                consume(lo, hi, [(members[j], dsts[j].numpy(), vals[6 + j] & 0xFFFFFFFF, raw[j]) for j in range(3)])
-        else:
-            value_at = (chunk * G * ibytes + 63) // 64 * 64  # the value stream, after the worst-case column stream
-            stage = [torch.empty(value_at + 2 * chunk * G, dtype=torch.uint8, device=dev) for _ in range(2)]
-            ovf = [_OverflowList(overflow_cap or (1 << 16), dev) for _ in range(2)]
-            ovf_host = [torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory() for k in range(2)]
-            # host side: the row pointer, then the streams of the nonzeros, values on a 64-byte boundary
-            stage_host = _pinned_staging(dev, 8 * (chunk + 1) + value_at + 64 + 2 * chunk * G)
-            # the widened chunk, reused from chunk to chunk: its pages are touched as the chunks' nnz needs them
-            # and hostpool keeps them mapped for the next call.  Past the first chunk they are mapped and out of
-            # cache, which is what the streaming stores are for.
-            indices_w = hostpool.result_array((chunk * G,), index_dtype)[0]
-            data_w = hostpool.result_array((chunk * G,), data_dtype)[0]
-            lib = nat.load()
-            widen_i = widen_d = lib.pst_host_widen_stream
-
-            def pack(k, cells):
-                ovf[k].count.zero_()
-                nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, stage[k].data_ptr(), ibits,
-                         stage[k].data_ptr() + value_at, 16, *ovf[k].kernel_args, pack_flags, st)
-
-            def produce(k, lo, hi):
-                draw_rows(k, lo, hi)
-                pack(k, hi - lo)
-                record(k, hi - lo)
-
-            def collect(k, lo, hi):
-                n_sat, nnz = read_info(k)[:2]
-                cells = hi - lo
-                if n_sat > ovf[k].capacity:
-                    ovf[k] = _OverflowList(max(n_sat, 2 * ovf[k].capacity), dev)
-                    ovf_host[k] = torch.empty(12 * ovf[k].capacity, dtype=torch.uint8).pin_memory()
-                    pack(k, cells)
-                    torch.cuda.current_stream(dev).synchronize()   # the copies wait for the first pack only
-                at = 8 * (cells + 1)
-                vat = (at + nnz * ibytes + 63) // 64 * 64
-                h = stage_host[k]
-                pairs = [(indptr[k][:cells + 1].view(torch.uint8), h[:at]),
-                         (stage[k][:nnz * ibytes], h[at:at + nnz * ibytes]),
-                         (stage[k][value_at:value_at + 2 * nnz], h[vat:vat + 2 * nnz])]
-                if n_sat:
-                    pairs += [(ovf[k].pos[:n_sat].view(torch.uint8), ovf_host[k][:8 * n_sat]),
-                              (ovf[k].value[:n_sat].view(torch.uint8), ovf_host[k][8 * n_sat:12 * n_sat])]
-                return pairs
-
-            def landed(dsts, lo, hi):
-                nnz = dsts[1].numel() // ibytes
-                indices, data = indices_w[:nnz], data_w[:nnz]
-                rc = widen_i(dsts[1].data_ptr(), ibits, indices.ctypes.data, 8 * index_dtype.itemsize, nnz,
-                             int(threads))
-                rc |= widen_d(dsts[2].data_ptr(), 16, data.ctypes.data, 8 * data_dtype.itemsize, nnz, int(threads))
-                if rc != 0:
-                    raise nat.NativeError("pst_host_widen failed")
-                if len(dsts) > 3:
-                    lib.pst_host_apply_overflow(data.ctypes.data, 8 * data_dtype.itemsize, 0, nnz, dsts[3].data_ptr(),
-                                                dsts[4].data_ptr(), dsts[3].numel() // 8)
-                consume(lo, hi, dsts[0].numpy().view(np.int64), indices, data)
-
-        self._copy_chunks(bounds, produce, landed, collect)
-        if int(pack_flags.item()) != 0:
-            raise RuntimeError("the packed counts do not match the row sizes of their chunk")
-        return total[0]
+        # the text of a chunk and its compressed form, bounded by about as many bytes again, and the tokens
+        return (2 + tokens) * slot * G, empty, start
 
     def _dense_chunks(self, rows, scaling32, seed, cell0, tdt, chunk_cells, overflow_cap, host_out=None,
                       consume=None):
@@ -926,10 +923,10 @@ class CountEngine(object):
         never waits per chunk.  With `consume`, one worker thread calls consume(dsts, lo, hi) once the copies
         have landed, and the host waits for it before it copies into buffer k again (the dsts are pinned
         staging that the next use of k overwrites).
-        With `collect`, the copies run one chunk late: produce only queues chunk i's device work, and
-        collect(k, lo, hi) returns chunk i's copies once chunk i+1's work is queued, so the host can read what
-        chunk i left on the device (its size) while the device works on. The copies wait for chunk i's work
-        only, not for chunk i+1's: device work that collect queues itself must have finished when it returns.
+        With `collect`, the copies run one chunk late: once chunk i+1's work is queued and chunk i's has finished,
+        collect(k, lo, hi) reads what chunk i left on the device while the device works on and returns (chunk i's
+        copies, a record for consume(dsts, lo, hi, record)).  The copies wait for chunk i's work only: device work
+        that collect queues itself must have finished when it returns.
         Owns the overlap and its teardown: whatever ends the loop, the side stream and the worker are drained
         before the buffers can go back to the allocator."""
         main = torch.cuda.current_stream(self.dev)
@@ -939,11 +936,11 @@ class CountEngine(object):
         copied = [None, None]                           # the copies out of buffer k have finished
         pending = [None, None]                          # consume still reading the host side of buffer k
 
-        def landed(event, dsts, lo, hi):
+        def landed(event, dsts, *args):
             event.synchronize()                         # the chunk is in dsts
-            consume(dsts, lo, hi)
+            consume(dsts, *args)
 
-        def copy(k, lo, hi, pairs):
+        def copy(k, pairs, *args):                      # args: lo, hi and, with collect, the chunk's record
             if pending[k] is not None:
                 pending[k].result()
             with torch.cuda.stream(copy_stream):
@@ -953,7 +950,7 @@ class CountEngine(object):
                 copied[k] = torch.cuda.Event()
                 copied[k].record(copy_stream)
             if consume is not None:
-                pending[k] = pool.submit(landed, copied[k], [dst for _, dst in pairs], lo, hi)
+                pending[k] = pool.submit(landed, copied[k], [dst for _, dst in pairs], *args)
 
         lag = 0 if collect is None else 1
         try:
@@ -966,10 +963,12 @@ class CountEngine(object):
                     filled[k] = torch.cuda.Event()
                     filled[k].record(main)
                     if not lag:
-                        copy(k, *bounds[i], pairs)
+                        copy(k, pairs, *bounds[i])
                 if lag and i:
                     k = (i - 1) & 1
-                    copy(k, *bounds[i - 1], collect(k, *bounds[i - 1]))
+                    filled[k].synchronize()
+                    pairs, record = collect(k, *bounds[i - 1])
+                    copy(k, pairs, *bounds[i - 1], record)
             for f in pending:
                 if f is not None:
                     f.result()
