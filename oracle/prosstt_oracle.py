@@ -20,7 +20,9 @@ the legacy RandomState stream).  `nb_draw_legacy` below calls that very function
 its published algorithm (gamma-Poisson mixture: Marsaglia-Tsang gamma, PTRS
 Poisson for lam >= 10, multiplication method below) is what the CUDA sampler
 re-implements on a counter-based generator, so counts are compared in
-distribution, not bit for bit (north star, correctness part 3).
+distribution, not bit for bit (north star, correctness part 3).  Our own counter-based
+sampler is, in addition, replayed count by count from its Philox words
+(oracle/count_replay.py, tests/test_count_replay.py).
 
 All file:line citations are relative to /root/reference/prosstt/.
 """
