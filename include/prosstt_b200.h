@@ -295,6 +295,17 @@ int pst_mtx_row_bytes(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64
 int pst_mtx_format(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t col0, const int64_t *text_ptr,
                    int64_t cap, char *out, void *stream);
 
+/* Dense tab-separated text of a chunk of cells (the reference's <job>_simulation.txt, written by
+ * tree_utils.save_matrices): row i of the int32 chunk X is the line "cell_<row0+i>", then "\t<v>" for every
+ * gene including zeros, then "\n".  pst_tsv_row_bytes writes each row's text length,
+ * row_bytes[i] = 5 + digits(row0+i) + sum over the genes of (1 + digits(v)) + 1 (int32; G * 11 + 32 must fit);
+ * pst_csr_row_offsets scans it into the chunk's text pointer.  pst_tsv_format writes row i at
+ * out + text_ptr[i] (out 16-byte aligned), or nothing at all when text_ptr[n] > cap, as pst_mtx_format. */
+int pst_tsv_row_bytes(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t row0, int32_t *row_bytes,
+                      void *stream);
+int pst_tsv_format(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t row0, const int64_t *text_ptr,
+                   int64_t cap, char *out, void *stream);
+
 /* ---- raw DEFLATE (RFC 1951) on the device: the compressed CSR file (pst_deflate.cu) ---------------
  * The input is cut into blocks of `block` bytes (a multiple of 1024, at most 32768).  Each block becomes
  * one dynamic-Huffman block over the literals 0-255 and end-of-block (no length or distance codes; the

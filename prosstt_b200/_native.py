@@ -65,6 +65,8 @@ _SIGNATURES = {
     "pst_csr_indptr_bytes": (C.c_int, [_p, _i64, _p, _p, _i32, _p]),
     "pst_mtx_row_bytes": (C.c_int, [_p, _i64, _i64, _i64, _i64, _p, _p]),
     "pst_mtx_format": (C.c_int, [_p, _i64, _i64, _i64, _i64, _p, _i64, _p, _p]),
+    "pst_tsv_row_bytes": (C.c_int, [_p, _i64, _i64, _i64, _i64, _p, _p]),
+    "pst_tsv_format": (C.c_int, [_p, _i64, _i64, _i64, _i64, _p, _i64, _p, _p]),
     "pst_deflate_bound": (_i64, [_i64, _i32]),
     "pst_deflate_workspace_bytes": (_i64, [_i64, _i32]),
     "pst_deflate_blocks": (C.c_int, [_p, _p, _i64, _i64, _i32, _p, _p, _p, _p, _i64, _p]),

@@ -274,17 +274,12 @@ csr_indptr_kernel(const int64_t *__restrict__ indptr, int64_t n, int64_t *__rest
 }
 
 // ---------------------------------------------------------------------------------------------
-// Matrix Market text of a chunk (the 10x `matrix.mtx.gz`, genes x cells): row i of the chunk is cell
-// col0 + i + 1 of the file, and its nonzero X[i][g] = v is the line "<g+1> <col0+i+1> <v>\n", genes
-// ascending.  pst_mtx_row_bytes gives each row's text length, pst_csr_row_offsets scans them into the
-// chunk's text pointer and pst_mtx_format writes the text.  Both walk a row with one warp, a lane owning
-// a gene quad, like the CSR kernels above.
+// Text of a chunk of rows, one formatter per on-disk text format (the Text policies below).  Row i of the
+// chunk is cell number Text::cell(first, i) of the file.  Text::row_bytes gives each row's text length,
+// pst_csr_row_offsets scans them into the chunk's text pointer and text_format_kernel writes the text.  Both
+// walk a row with one warp, a lane owning a gene quad, like the CSR kernels above.
 // ---------------------------------------------------------------------------------------------
-constexpr int kMtxWarps = 4;                           // warps per block of pst_mtx_format
-constexpr int kMtxLine = 42;                           // longest line: 10 + 19 + 10 digits, 3 separators
-constexpr int kMtxStage = 16 + 128 * kMtxLine;         // one 16-byte carry + the text of 128 genes
-static_assert(kMtxStage % 16 == 0, "the staging of each warp stays 16-byte aligned");
-constexpr int64_t kMtxMaxG = ((int64_t)1 << 31) / kMtxLine;   // a row's text fits int32
+constexpr int kTextWarps = 4;                          // warps per block of text_format_kernel
 
 __device__ __forceinline__ int dec_digits32(uint32_t v) {
   return 1 + (v >= 10u) + (v >= 100u) + (v >= 1000u) + (v >= 10000u) + (v >= 100000u) + (v >= 1000000u) +
@@ -317,53 +312,105 @@ __device__ __forceinline__ void put_dec(char *p, U v, int d, const char *__restr
   }
 }
 
-// row_bytes[i] = nnz_i (digits(col0 + i + 1) + 3) + sum over the row's nonzeros of digits(g + 1) + digits(v):
-// csr_row_count_kernel's walk (four 128-bit streaming loads in flight per lane, one REDUX per row)
-template <bool VEC>
+// Matrix Market text (the 10x `matrix.mtx.gz`, genes x cells): cell first + i + 1, and each nonzero
+// X[i][g] = v is the line "<g+1> <cell> <v>\n", genes ascending; a row without nonzeros has no text.  The
+// cell field is put once per row into the warp's `field` and copied into each line.
+struct MtxText {
+  static constexpr int kGene = 42;                     // longest line: 10 + 19 + 10 digits, 3 separators
+  static constexpr int kLabel = 0;                     // staging bytes of a row before its first gene
+  __device__ static uint64_t cell(int64_t first, int64_t row) { return (uint64_t)(first + row + 1); }
+  // the text of gene g1 - 1 (in: g1 <= G) with value v, cell field of cl digits
+  __device__ static int gene(int32_t v, uint32_t g1, bool, int cl) {
+    return v != 0 ? dec_digits32(g1) + cl + dec_digits32((uint32_t)v) + 3 : 0;
+  }
+  __device__ static int other(int) { return 0; }       // bytes of a row outside its genes' text
+  __device__ static int label(char *, char *field, uint64_t cell, int cl, const char *pairs) {
+    put_dec(field, cell, cl, pairs);
+    return 0;
+  }
+  __device__ static void put(char *p, int32_t v, uint32_t g1, int cl, const char *field, const char *pairs) {
+    const int dg = dec_digits32(g1);
+    put_dec(p, g1, dg, pairs);
+    p[dg] = ' ';
+    p += dg + 1;
+    for (int c = 0; c < cl; ++c) p[c] = field[c];
+    p[cl] = ' ';
+    p += cl + 1;
+    const int dv = dec_digits32((uint32_t)v);
+    put_dec(p, (uint32_t)v, dv, pairs);
+    p[dv] = '\n';
+  }
+  __device__ static int end(char *) { return 0; }
+};
+
+// Dense tab-separated text (the reference's `_simulation.txt`, tree_utils.save_matrices): the row of cell
+// first + i is "cell_<first+i>", then "\t<v>" for every gene including zeros, then "\n".
+struct TsvText {
+  static constexpr int kGene = 11;                     // a tab and up to 10 digits
+  static constexpr int kLabel = 5 + 20;                // "cell_" and up to 20 digits
+  __device__ static uint64_t cell(int64_t first, int64_t row) { return (uint64_t)(first + row); }
+  __device__ static int gene(int32_t v, uint32_t, bool in, int) { return in ? 1 + dec_digits32((uint32_t)v) : 0; }
+  __device__ static int other(int cl) { return 5 + cl + 1; }
+  __device__ static int label(char *s, char *, uint64_t cell, int cl, const char *pairs) {
+    s[0] = 'c'; s[1] = 'e'; s[2] = 'l'; s[3] = 'l'; s[4] = '_';
+    put_dec(s + 5, cell, cl, pairs);
+    return 5 + cl;
+  }
+  __device__ static void put(char *p, int32_t v, uint32_t, int, const char *, const char *pairs) {
+    p[0] = '\t';
+    put_dec(p + 1, (uint32_t)v, dec_digits32((uint32_t)v), pairs);
+  }
+  __device__ static int end(char *s) { *s = '\n'; return 1; }
+};
+
+// the staging of each warp: a partial 16-byte piece carried over, a row's label and the text of 128 genes
+template <class Text>
+__host__ __device__ constexpr int text_stage() { return (16 + Text::kLabel + 128 * Text::kGene + 15) / 16 * 16; }
+
+// row_bytes[i] = Text::other(digits(cell)) + sum over the row's genes of Text::gene: csr_row_count_kernel's walk
+// (four 128-bit streaming loads in flight per lane, one REDUX per row)
+template <class Text, bool VEC>
 __global__ void __launch_bounds__(256)
-mtx_row_bytes_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx, int64_t col0,
-                     int32_t *__restrict__ row_bytes) {
+text_row_bytes_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx, int64_t first,
+                      int32_t *__restrict__ row_bytes) {
   const int lane = threadIdx.x & 31;
   const int64_t warp0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   const int64_t n_warps = ((int64_t)gridDim.x * blockDim.x) >> 5;
   const int64_t Q = (G + 3) / 4;
   for (int64_t row = warp0; row < n; row += n_warps) {
     const int32_t *src = X + row * ldx;
-    unsigned c = 0, b = 0;
+    const int cl = dec_digits64(Text::cell(first, row));
+    unsigned b = 0;
     for (int64_t q0 = 0; q0 < Q; q0 += 128) {
       int4 v[4];
 #pragma unroll
       for (int j = 0; j < 4; ++j) v[j] = load_quad<VEC>(src, q0 + 32 * j + lane, Q, G);
 #pragma unroll
       for (int j = 0; j < 4; ++j) {
-        const uint32_t g = (uint32_t)((q0 + 32 * j + lane) * 4) + 1u;
+        const int64_t g0 = (q0 + 32 * j + lane) * 4;
         const int32_t vv[4] = {v[j].x, v[j].y, v[j].z, v[j].w};
 #pragma unroll
-        for (int k = 0; k < 4; ++k) {
-          const bool nz = vv[k] != 0;
-          c += nz;
-          b += nz ? (unsigned)(dec_digits32(g + k) + dec_digits32((uint32_t)vv[k])) : 0u;
-        }
+        for (int k = 0; k < 4; ++k) b += (unsigned)Text::gene(vv[k], (uint32_t)g0 + k + 1u, g0 + k < G, cl);
       }
     }
-    c = __reduce_add_sync(0xffffffffu, c);
     b = __reduce_add_sync(0xffffffffu, b);
-    if (lane == 0) row_bytes[row] = (int32_t)(b + c * (unsigned)(dec_digits64((uint64_t)(col0 + row + 1)) + 3));
+    if (lane == 0) row_bytes[row] = (int32_t)(b + (unsigned)Text::other(cl));
   }
 }
 
-// The text of row i at out + text_ptr[i].  Per tile of 128 genes a lane writes its lines into the warp's
-// shared staging at a warp-exclusive scan of their lengths, then the warp stores the staging's whole
-// 16-byte pieces with 128-bit stores (512 contiguous bytes per instruction) and carries the last partial
-// piece to the next tile.  A row's first and last pieces are shared with its neighbours' text: their bytes
-// are stored one by one, only the row's own.  Writes nothing when text_ptr[n] > cap.
-template <bool VEC>
-__global__ void __launch_bounds__(kMtxWarps * 32, 8)   // 8 blocks per SM: at most 64 registers, no spill
-mtx_format_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx, int64_t col0,
-                  const int64_t *__restrict__ text_ptr, int64_t cap, char *__restrict__ out) {
+// The text of row i at out + text_ptr[i].  Lane 0 puts the row's label into the warp's shared staging; then per
+// tile of 128 genes a lane writes its genes' text into the staging at a warp-exclusive scan of their lengths,
+// and the warp stores the staging's whole 16-byte pieces with 128-bit stores (512 contiguous bytes per
+// instruction) and carries the last partial piece to the next tile.  A row's first and last pieces are shared
+// with its neighbours' text: their bytes are stored one by one, only the row's own.  Writes nothing when
+// text_ptr[n] > cap.
+template <class Text, bool VEC>
+__global__ void __launch_bounds__(kTextWarps * 32, 8)   // 8 blocks per SM: at most 64 registers, no spill
+text_format_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t ldx, int64_t first,
+                   const int64_t *__restrict__ text_ptr, int64_t cap, char *__restrict__ out) {
   __shared__ char pairs[200];
-  __shared__ __align__(16) char stage[kMtxWarps][kMtxStage];
-  __shared__ char cell_field[kMtxWarps][20];
+  __shared__ __align__(16) char stage[kTextWarps][text_stage<Text>()];
+  __shared__ char cell_field[kTextWarps][20];
   if (text_ptr[n] > cap) return;                               // the same for every thread of the grid
   for (int t = threadIdx.x; t < 100; t += blockDim.x) {
     pairs[2 * t] = (char)('0' + t / 10);
@@ -374,17 +421,17 @@ mtx_format_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t l
   char *s = stage[wid];
   char *cf = cell_field[wid];
   const int64_t Q = (G + 3) / 4;
-  for (int64_t row = (int64_t)blockIdx.x * kMtxWarps + wid; row < n; row += (int64_t)gridDim.x * kMtxWarps) {
+  for (int64_t row = (int64_t)blockIdx.x * kTextWarps + wid; row < n; row += (int64_t)gridDim.x * kTextWarps) {
     const int64_t pos = text_ptr[row];
-    if (pos == text_ptr[row + 1]) continue;                    // no nonzeros
-    const uint64_t cell = (uint64_t)(col0 + row + 1);
+    if (pos == text_ptr[row + 1]) continue;                    // no text
+    const uint64_t cell = Text::cell(first, row);
     const int cl = dec_digits64(cell);
-    if (lane == 0) put_dec(cf, cell, cl, pairs);               // the cell field, once per row
-    __syncwarp();
-    const int32_t *src = X + row * ldx;
     int64_t base = pos & ~(int64_t)15;                         // staging byte 0 belongs at out + base
     int head = (int)(pos & 15);                                // bytes before it that are not this row's
-    int fill = head;
+    int fill = head + (lane == 0 ? Text::label(s + head, cf, cell, cl, pairs) : 0);   // once per row
+    fill = __shfl_sync(0xffffffffu, fill, 0);
+    __syncwarp();
+    const int32_t *src = X + row * ldx;
     for (int64_t q0 = 0; q0 < Q; q0 += 32) {
       const int64_t q = q0 + lane;
       const int4 v = load_quad<VEC>(src, q, Q, G);
@@ -393,7 +440,7 @@ mtx_format_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t l
       int len[4], tot = 0;
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
-        len[k] = vv[k] != 0 ? dec_digits32(g + k) + cl + dec_digits32((uint32_t)vv[k]) + 3 : 0;
+        len[k] = Text::gene(vv[k], g + k, q * 4 + k < G, cl);
         tot += len[k];
       }
       int incl = tot;
@@ -407,18 +454,8 @@ mtx_format_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t l
       int at = fill + incl - tot;
 #pragma unroll
       for (int k = 0; k < 4; ++k) {
-        if (vv[k] != 0) {
-          const int dg = dec_digits32(g + k);
-          char *p = s + at;
-          put_dec(p, g + k, dg, pairs);
-          p[dg] = ' ';
-          p += dg + 1;
-          for (int c = 0; c < cl; ++c) p[c] = cf[c];
-          p[cl] = ' ';
-          p += cl + 1;
-          const int dv = dec_digits32((uint32_t)vv[k]);
-          put_dec(p, (uint32_t)vv[k], dv, pairs);
-          p[dv] = '\n';
+        if (len[k] != 0) {
+          Text::put(s + at, vv[k], g + k, cl, cf, pairs);
           at += len[k];
         }
       }
@@ -438,7 +475,11 @@ mtx_format_kernel(const int32_t *__restrict__ X, int64_t n, int64_t G, int64_t l
       base += 16 * whole;
       fill = rem;
     }
-    if (lane >= head && lane < fill) out[base + lane] = s[lane];
+    if (lane == 0) fill += Text::end(s + fill);
+    fill = __shfl_sync(0xffffffffu, fill, 0);
+    __syncwarp();
+    for (int p = lane; p < fill; p += 32)                      // the row's last piece (and, for a short row
+      if (p >= head) out[base + p] = s[p];                     // that never filled one, its first)
     __syncwarp();                                              // the staging is rewritten by the next row
   }
 }
@@ -454,6 +495,32 @@ __global__ void __launch_bounds__(256) store_fill_kernel(int4 *__restrict__ out,
 inline unsigned stream_grid(int64_t threads) {
   return (unsigned)std::max<int64_t>(1, std::min<int64_t>((threads + 255) / 256, (int64_t)num_sm() * 16));
 }
+
+// pst_mtx_row_bytes / pst_tsv_row_bytes: one warp per row
+template <class Text>
+void launch_text_row_bytes(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t first, int32_t *row_bytes,
+                           void *stream) {
+  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
+  const unsigned grid = stream_grid(n * 32);
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec) text_row_bytes_kernel<Text, true><<<grid, 256, 0, st>>>(X, n, G, ldx, first, row_bytes);
+  else text_row_bytes_kernel<Text, false><<<grid, 256, 0, st>>>(X, n, G, ldx, first, row_bytes);
+}
+
+// pst_mtx_format / pst_tsv_format: kTextWarps rows per block
+template <class Text>
+void launch_text_format(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t first, const int64_t *text_ptr,
+                        int64_t cap, char *out, void *stream) {
+  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
+  const unsigned grid = (unsigned)std::max<int64_t>(
+      1, std::min<int64_t>((n + kTextWarps - 1) / kTextWarps, (int64_t)num_sm() * 16));
+  cudaStream_t st = (cudaStream_t)stream;
+  if (vec) text_format_kernel<Text, true><<<grid, kTextWarps * 32, 0, st>>>(X, n, G, ldx, first, text_ptr, cap, out);
+  else text_format_kernel<Text, false><<<grid, kTextWarps * 32, 0, st>>>(X, n, G, ldx, first, text_ptr, cap, out);
+}
+
+constexpr int64_t kMtxMaxG = ((int64_t)1 << 31) / MtxText::kGene;       // a row's text fits int32
+constexpr int64_t kTsvMaxG = (INT32_MAX - 32) / TsvText::kGene;          // G * 11 + 32 fits int32
 
 }  // namespace
 }  // namespace pst
@@ -624,11 +691,7 @@ extern "C" int pst_mtx_row_bytes(const int32_t *X, int64_t n, int64_t G, int64_t
   PST_REQUIRE(col0 <= INT64_MAX - n, fn, "cell numbers do not fit int64");
   if (n == 0) return 0;
   PST_REQUIRE(row_bytes && (G == 0 || X), fn, "null pointer");
-  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
-  const unsigned grid = stream_grid(n * 32);
-  cudaStream_t st = (cudaStream_t)stream;
-  if (vec) mtx_row_bytes_kernel<true><<<grid, 256, 0, st>>>(X, n, G, ldx, col0, row_bytes);
-  else mtx_row_bytes_kernel<false><<<grid, 256, 0, st>>>(X, n, G, ldx, col0, row_bytes);
+  launch_text_row_bytes<MtxText>(X, n, G, ldx, col0, row_bytes, stream);
   return check_launch(fn);
 }
 
@@ -641,11 +704,31 @@ extern "C" int pst_mtx_format(const int32_t *X, int64_t n, int64_t G, int64_t ld
   if (n == 0 || G == 0) return 0;
   PST_REQUIRE(X && text_ptr && out, fn, "null pointer");
   PST_REQUIRE((uintptr_t)out % 16 == 0, fn, "out must be 16-byte aligned");
-  const bool vec = (G % 4 == 0) && (ldx % 4 == 0) && ((uintptr_t)X % 16 == 0);
-  const unsigned grid = (unsigned)std::max<int64_t>(
-      1, std::min<int64_t>((n + kMtxWarps - 1) / kMtxWarps, (int64_t)num_sm() * 16));
-  cudaStream_t st = (cudaStream_t)stream;
-  if (vec) mtx_format_kernel<true><<<grid, kMtxWarps * 32, 0, st>>>(X, n, G, ldx, col0, text_ptr, cap, out);
-  else mtx_format_kernel<false><<<grid, kMtxWarps * 32, 0, st>>>(X, n, G, ldx, col0, text_ptr, cap, out);
+  launch_text_format<MtxText>(X, n, G, ldx, col0, text_ptr, cap, out, stream);
+  return check_launch(fn);
+}
+
+extern "C" int pst_tsv_row_bytes(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t row0, int32_t *row_bytes,
+                                 void *stream) {
+  const char *fn = "pst_tsv_row_bytes";
+  PST_REQUIRE(n >= 0 && G >= 0 && ldx >= G && row0 >= 0, fn, "need n, G, row0 >= 0 and ldx >= G");
+  PST_REQUIRE(G <= kTsvMaxG, fn, "a row's text does not fit int32");
+  PST_REQUIRE(row0 <= INT64_MAX - n, fn, "cell numbers do not fit int64");
+  if (n == 0) return 0;
+  PST_REQUIRE(row_bytes && (G == 0 || X), fn, "null pointer");
+  launch_text_row_bytes<TsvText>(X, n, G, ldx, row0, row_bytes, stream);
+  return check_launch(fn);
+}
+
+extern "C" int pst_tsv_format(const int32_t *X, int64_t n, int64_t G, int64_t ldx, int64_t row0,
+                              const int64_t *text_ptr, int64_t cap, char *out, void *stream) {
+  const char *fn = "pst_tsv_format";
+  PST_REQUIRE(n >= 0 && G >= 0 && ldx >= G && row0 >= 0 && cap >= 0, fn, "need n, G, row0, cap >= 0 and ldx >= G");
+  PST_REQUIRE(G <= kTsvMaxG, fn, "a row's text does not fit int32");
+  PST_REQUIRE(row0 <= INT64_MAX - n, fn, "cell numbers do not fit int64");
+  if (n == 0) return 0;
+  PST_REQUIRE(text_ptr && out && (G == 0 || X), fn, "null pointer");
+  PST_REQUIRE((uintptr_t)out % 16 == 0, fn, "out must be 16-byte aligned");
+  launch_text_format<TsvText>(X, n, G, ldx, row0, text_ptr, cap, out, stream);
   return check_launch(fn);
 }

@@ -277,6 +277,12 @@ def _mtx_slot_bytes(G, n):
     return len(str(G)) + len(str(n)) + 6
 
 
+def _tsv_slot_bytes(G, n):
+    """Tab-separated text bytes budgeted per gene slot of a chunk of a file of n cells: a tab and a count of up to 3
+    digits.  A chunk with more text is formatted again into a larger buffer (CountEngine.stream_csr)."""
+    return 4
+
+
 def _plan_chunks(n, chunk_cells, cell_bytes, budget):
     """The cell chunks of a chunked device->host call: (chunk, [(lo, hi), ...]) covering [0, n) in order, where
     chunk is the largest chunk (the size of the buffers).  Owns the chunk size and the ramp-up.
@@ -607,7 +613,8 @@ class CountEngine(object):
         return indptr, indices, data
 
     def stream_csr(self, rows, scaling32, seed, cell0, consume, index_dtype=np.int64, data_dtype=np.int64,
-                   chunk_cells=None, threads=0, overflow_cap=None, compress=False, mtx=False, compression="huffman"):
+                   chunk_cells=None, threads=0, overflow_cap=None, compress=False, mtx=False, compression="huffman",
+                   tsv=False):
         """Sample the cells in chunks and hand each one as CSR to consume(lo, hi, indptr, indices, data), on a
         worker thread, once per chunk, in cell order.  indptr is chunk-local int64 (hi - lo + 1 entries from 0);
         indices and data are the chunk's nonzeros in `index_dtype` / `data_dtype` (int32 or int64), columns
@@ -630,6 +637,12 @@ class CountEngine(object):
         the text_len bytes of the chunk's nnz lines "<g+1> <c+1> <v>\n", c = lo + row within the chunk, whose
         CRC-32 is crc; index_dtype and data_dtype do not apply.
 
+        tsv=True: consume(lo, hi, text, crc, text_len) receives the chunk as dense tab-separated text
+        (formats.TsvWriter.append): the text_len bytes of its rows "cell_<cell0+c>" "\t<v>" for every gene "\n",
+        c = lo + row within the chunk.  `text` (a reused uint8 host buffer) is that text itself, crc 0; with
+        compress=True it is raw DEFLATE that decompresses to it, whose CRC-32 is crc.  index_dtype and data_dtype
+        do not apply.
+
         compression ("huffman" or "lz77", with compress=True or mtx=True): the device compressor,
         pst_deflate_blocks (Huffman-only) or pst_deflate_lz_blocks (LZ77 matches within each 32 KiB block,
         smaller output, a larger workspace).  Both write the same framing, so the consumer is the same."""
@@ -646,6 +659,7 @@ class CountEngine(object):
         # returns step, grow (True if a buffer of k grew for the chunk), encode (what then runs again), copies, deliver
         cell_bytes, empty, start = (
             self._mtx_encoder(n, consume, compression) if mtx else
+            self._tsv_encoder(n, consume, compress, compression, cell0) if tsv else
             self._npz_encoder(n, consume, index_dtype, data_dtype, compression) if compress else
             self._shard_encoder(n, consume, index_dtype, data_dtype, threads, overflow_cap))
         if G == 0:
@@ -875,6 +889,82 @@ class CountEngine(object):
 
         # the text of a chunk and its compressed form, bounded by about as many bytes again, and the tokens
         return (2 + tokens) * slot * G, empty, start
+
+    def _tsv_encoder(self, n, consume, compress, compression, row0):
+        """stream_csr(tsv=True): pst_tsv_row_bytes and pst_csr_row_offsets (the text pointer), pst_tsv_format into text
+        buffer k, of _tsv_slot_bytes per gene slot and the label per cell, and, with compress, the compressor over the
+        text.  A chunk with more text is not formatted (pst_tsv_format writes nothing), and is formatted again in a
+        larger buffer.  Without compress the text itself is copied, so it needs one buffer per k."""
+        G, dev, st, lib, block = self.G, self.dev, nat.stream_ptr(self.dev), nat.load(), _DEFLATE_BLOCK
+        deflate, deflate_work, tokens = _DEFLATE[compression]
+        cell_text = _tsv_slot_bytes(G, n) * G + len("cell_%d\n" % (row0 + n))
+        TEXT_LEN, SIZE, CRC = range(_REC_OWN, _REC_OWN + 3)     # record: text length, compressed size, CRC
+
+        def empty():
+            text = "".join("cell_%d\n" % i for i in range(row0, row0 + n)).encode("ascii")
+            consume(0, n, *(sync_deflate(text) if compress else (np.frombuffer(text, np.uint8), 0, len(text))))
+
+        def start(chunk, work, indptr, info, pack_flags):
+            row_bytes = torch.empty(chunk, dtype=torch.int32, device=dev)
+            text_ptr = [torch.empty(chunk + 1, dtype=torch.int64, device=dev) for _ in range(2)]
+            text, packed = [None, None], [None, None]
+            dwork = {"bytes": -1}                         # the deflate workspace, shared by both k
+            formatted_cap = [0, 0]                        # the capacity chunk k was formatted against
+            out_bytes = chunk * cell_text
+            if compress:
+                out_bytes = int(lib.pst_deflate_bound(out_bytes, block))
+            # a copy of the cached pair, so that growing one k leaves the cache as it is
+            stage_host = list(_pinned_staging(dev, out_bytes))
+
+            def reserve(k, cap):
+                """Text buffer k of cap bytes and, with compress, room for its compressed form."""
+                text[k] = torch.empty(max(16, cap), dtype=torch.uint8, device=dev)
+                if compress:
+                    packed[k] = torch.empty(max(1, int(lib.pst_deflate_bound(cap, block))), dtype=torch.uint8,
+                                            device=dev)
+                    need = int(getattr(lib, deflate_work)(cap, block))
+                    if need > dwork["bytes"]:
+                        dwork["bytes"] = need
+                        dwork["buf"] = torch.empty(max(1, need), dtype=torch.uint8, device=dev)
+
+            def encode(k, lo, cells):
+                """Format chunk k from its work buffer and, with compress, compress the text."""
+                cap = formatted_cap[k] = text[k].numel()
+                nat.call("pst_tsv_format", work[k], cells, G, G, row0 + lo, text_ptr[k], cap, text[k], st)
+                if compress:
+                    nat.call(deflate, text[k], text_ptr[k][cells:cells + 1], 1, cap, block, packed[k], info[k, SIZE],
+                             info[k, CRC].data_ptr(), dwork["buf"], dwork["bytes"], st)
+
+            for k in range(2):
+                reserve(k, chunk * cell_text)
+
+            def step(k, lo, cells):
+                nat.call("pst_tsv_row_bytes", work[k], cells, G, G, row0 + lo, row_bytes, st)
+                nat.call("pst_csr_row_offsets", row_bytes, cells, text_ptr[k], st)
+                info[k, TEXT_LEN].copy_(text_ptr[k][cells])
+                encode(k, lo, cells)
+
+            def grow(k, record):
+                # the text did not fit the buffer the chunk was formatted against: nothing was formatted
+                if record[TEXT_LEN] <= formatted_cap[k]:
+                    return False
+                reserve(k, max(record[TEXT_LEN], 2 * formatted_cap[k]))
+                return True
+
+            def copies(k, cells, record):
+                size = record[SIZE] if compress else record[TEXT_LEN]
+                if stage_host[k].numel() < size:
+                    stage_host[k] = torch.empty(size, dtype=torch.uint8).pin_memory()
+                return [((packed if compress else text)[k][:size], stage_host[k][:size])]
+
+            def deliver(dsts, lo, hi, record):
+                consume(lo, hi, dsts[0].numpy(), record[CRC] & 0xFFFFFFFF if compress else 0, record[TEXT_LEN])
+
+            return step, grow, encode, copies, deliver
+
+        # the text of a chunk and, with compress, its compressed form, bounded by about as many bytes again, and the
+        # tokens
+        return ((2 + tokens) if compress else 1) * cell_text, empty, start
 
     def _dense_chunks(self, rows, scaling32, seed, cell0, tdt, chunk_cells, overflow_cap, host_out=None,
                       consume=None):

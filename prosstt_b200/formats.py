@@ -29,6 +29,10 @@ added, both readable without this package:
   plus the cells' parameters.  The GPU formats each chunk as text (pst_mtx_format) and compresses it
   (pst_deflate_blocks), so only compressed text crosses PCIe and reaches the disk.  The call returns an
   `MtxRecord`.
+* the reference's own `_simulation.txt` (`TsvWriter`, written by `out="tsv", path=...`): the dense tab-separated
+  table of `tree_utils.save_matrices`, byte for byte, that `pd.read_csv(path, sep="\t", index_col=0)` reads;
+  with `compress=True` one gzip member of it.  The GPU formats each chunk's rows (pst_tsv_format) and, for the
+  gzipped file, compresses them, so only the file's bytes cross PCIe.  The call returns a `TsvRecord`.
 """
 import collections
 import concurrent.futures
@@ -694,6 +698,128 @@ class MtxWriter(object):
         if self._small is not None:
             concurrent.futures.wait([self._small])      # it writes into the directory removed below
         shutil.rmtree(self._dir, ignore_errors=True)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, exc, tb):
+        if exc_type is None:
+            self.close()
+        else:
+            self.abort()
+        return False
+
+
+_STORED_MAX = 65535                                           # bytes of one stored DEFLATE block
+
+
+def _stored_blocks(raw):
+    """`raw` as non-final stored DEFLATE blocks (RFC 1951 3.2.4), at most _STORED_MAX bytes each."""
+    out = []
+    for at in range(0, len(raw), _STORED_MAX):
+        piece = raw[at:at + _STORED_MAX]
+        out.append(struct.pack("<BHH", 0, len(piece), len(piece) ^ 0xFFFF) + piece)
+    return b"".join(out)
+
+
+def tsv_header(G):
+    """The header line of the reference's _simulation.txt: "\tgene_0\tgene_1 ... \n"; pandas writes '""' for a
+    frame without columns."""
+    if G == 0:
+        return b'""\n'
+    return ("".join("\tgene_%d" % j for j in range(G)) + "\n").encode("ascii")
+
+
+class TsvRecord(collections.namedtuple("TsvRecord", "path shape nbytes compressed")):
+    """The X of an out="tsv" call: the reference's _simulation.txt on disk, gzipped when `compressed`.  shape is
+    (cells, genes); nbytes is the file's size; load() reads it back as the reference's readers do, a
+    pandas.DataFrame indexed by the cell names."""
+    __slots__ = ()
+
+    def load(self):
+        import pandas as pd
+        return pd.read_csv(self.path, sep="\t", index_col=0, compression="gzip" if self.compressed else None)
+
+
+class TsvWriter(object):
+    """Writer of one dense tab-separated count table (the reference's _simulation.txt), appended chunk by chunk:
+    the header line "\tgene_0 ... \tgene_<G-1>", then one line "cell_<i>\t<count> ... \t<count>" per cell, i the
+    global cell index (first + local index).  With compress=True the file is one gzip member with MTIME 0, XFL 0
+    and OS 255: the header line as stored blocks, the appended blocks, the final block 03 00, then the CRC-32 (the
+    header's combined with the appended text's) and ISIZE.
+
+    append(rows, data, crc, raw_len) takes the text of the next `rows` cells, raw_len bytes: the text itself
+    (crc is not used), or with compress=True raw DEFLATE blocks that are not final and end on a byte boundary
+    (pst_deflate_blocks' output over pst_tsv_format's text, or sync_deflate's) with the CRC-32 of the text.  As
+    CsrShardWriter: everything goes to `<path>.partial`, renamed to `<path>` only by a complete close(); an
+    exception inside `with` or abort() leaves nothing behind; an existing `<path>` raises FileExistsError.  The
+    same appends give the same bytes."""
+
+    def __init__(self, path, shape, first=0, compress=False):
+        self.path = os.fspath(path)
+        if os.path.lexists(self.path):
+            raise FileExistsError(errno.EEXIST, "the count table exists already", self.path)
+        n, G = (int(v) for v in shape)
+        self.shape, self.first, self.compress = (n, G), int(first), bool(compress)
+        self.rows = 0
+        self._partial = self.path + ".partial"
+        self._fh = None
+        if os.path.lexists(self._partial):              # left behind by an interrupted writer
+            os.remove(self._partial)
+        try:
+            self._fh = open(self._partial, "wb")
+            header = tsv_header(G)
+            if self.compress:
+                self._fh.write(_GZIP_HEADER + _stored_blocks(header))
+                self._crc, self._raw = zlib.crc32(header), len(header)
+            else:
+                self._fh.write(header)
+        except BaseException:
+            self.abort()
+            raise
+
+    def append(self, rows, data, crc, raw_len):
+        """The text of the next `rows` cells, raw_len bytes: plain, or as non-final DEFLATE blocks."""
+        if self.rows + int(rows) > self.shape[0]:
+            raise ValueError("more rows than announced (%d)" % self.shape[0])
+        data = memoryview(data).cast("B")
+        if not self.compress and len(data) != int(raw_len):
+            raise ValueError("%d bytes of text, %d announced" % (len(data), raw_len))
+        self._fh.write(data)
+        if self.compress:
+            self._crc = int(nat.load().pst_host_crc32_combine(self._crc, int(crc) & 0xFFFFFFFF, int(raw_len)))
+            self._raw += int(raw_len)
+        self.rows += int(rows)
+
+    def close(self):
+        """Finish the file and move it to `path`; raises (and leaves nothing) when rows are missing."""
+        if self._fh is None:
+            return
+        try:
+            if self.rows != self.shape[0]:
+                raise ValueError("%s: %d of %d rows written" % (self.path, self.rows, self.shape[0]))
+            if self.compress:
+                self._fh.write(_FINAL_BLOCK + struct.pack("<II", self._crc, self._raw & 0xFFFFFFFF))
+            self._fh.close()
+            self._fh = None
+            os.rename(self._partial, self.path)
+        except BaseException:
+            self.abort()
+            raise
+
+    def record(self):
+        """The TsvRecord of the closed file."""
+        return TsvRecord(self.path, self.shape, os.path.getsize(self.path), self.compress)
+
+    def abort(self):
+        """Drop everything written so far."""
+        if self._fh is not None:
+            self._fh.close()
+        self._fh = None
+        try:
+            os.remove(self._partial)
+        except OSError:
+            pass
 
     def __enter__(self):
         return self

@@ -31,6 +31,13 @@ Extra keyword-only arguments (never required):
            and compresses every chunk, so only gzipped text crosses PCIe and reaches the disk.  X is then a
            formats.MtxRecord (path, shape, nnz, nbytes, load()); the counts are those of out="csr".  The file is
            always gzipped (compress=True is an error), and dtype must be int64 or int32 as for "csr"
+           out="tsv" with path: write the reference's own counts file at `path`, the dense tab-separated table of
+           tree_utils.save_matrices' `<job>_simulation.txt`, byte for byte (formats.TsvWriter: header line
+           "\tgene_0\tgene_1...", rows "cell_<global index>\t<count>..."), read by
+           pd.read_csv(path, sep="\t", index_col=0); with compress=True one gzip member of those bytes.  The GPU
+           formats (and compresses) every chunk, so only the file's bytes cross PCIe.  X is then a
+           formats.TsvRecord (path, shape, nbytes, compressed, load()); dtype must be int64 or int32 and does not
+           change the text.  Under shard=, each rank writes a complete file with its own header line
   compression  "huffman" (default) or "lz77", where the GPU compresses (compress=True, out="mtx"): "lz77" adds
            LZ77 matches within each 32 KiB DEFLATE block (pst_deflate_lz_blocks), so the same content is written
            in a smaller file; "huffman" writes Huffman-only blocks.  Both files decompress to the same bytes
@@ -57,7 +64,7 @@ from prosstt_b200 import count_model as cm
 from prosstt_b200 import hostpool
 from prosstt_b200 import sim_utils as sut
 from prosstt_b200.device import CountEngine, TreeTables, choice_cdf, raise_flags, tree_tables
-from prosstt_b200.formats import CsrNpzWriter, CsrShardWriter, MtxWriter, _csr_matrix, load_csr_shard
+from prosstt_b200.formats import CsrNpzWriter, CsrShardWriter, MtxWriter, TsvWriter, _csr_matrix, load_csr_shard
 from prosstt_b200.sharding import shard_range
 
 DEFAULT_SAMPLER = "hybrid"
@@ -435,9 +442,20 @@ def _shard_range(n, shard):
 def _check_csr_request(out, dtype, host_out=None, path=None, compress=False, compression="huffman"):
     """out="csr" takes int64 (default) or int32 data and no preallocated host_out; path needs out="csr";
     compress needs both.  out="mtx" needs path, takes int64 or int32 and neither host_out nor compress.
+    out="tsv" needs path, takes int64 or int32, compress and no host_out.
     compression is "huffman" or "lz77"; "lz77" only where the GPU compresses (compress=True or out="mtx")."""
     if compression not in ("huffman", "lz77"):
         raise ValueError("compression must be 'huffman' or 'lz77', not %r" % (compression,))
+    if out == "tsv":
+        if path is None:
+            raise ValueError("out='tsv' writes the reference's _simulation.txt: it needs path=")
+        if host_out is not None:
+            raise ValueError("host_out cannot be combined with out='tsv'")
+        if np.dtype(dtype) not in (np.dtype(np.int64), np.dtype(np.int32)):
+            raise ValueError("out='tsv' takes dtype int64 or int32, not %s" % np.dtype(dtype))
+        if compression == "lz77" and not compress:
+            raise ValueError("compression='lz77' applies where the GPU compresses: out='tsv' needs compress=True")
+        return
     if compression == "lz77" and out != "mtx" and not compress:
         raise ValueError("compression='lz77' applies where the GPU compresses: out='csr', path=, compress=True "
                          "or out='mtx', path=")
@@ -475,8 +493,11 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
     shard's memory-mapped matrix is returned; with `compress`, into one compressed file (formats.CsrNpzWriter,
     stream_csr(compress=True)), and its formats.CompressedCsr record is returned.
     out="mtx": the chunks go to a 10x directory at path (stream_csr(mtx=True) into a formats.MtxWriter, whose
-    barcodes count from the global cell index `first`), and its formats.MtxRecord is returned.  `compression`
-    picks the device compressor of both compressed forms (stream_csr)."""
+    barcodes count from the global cell index `first`), and its formats.MtxRecord is returned.
+    out="tsv": the chunks go to the reference's _simulation.txt at path, gzipped with `compress`
+    (stream_csr(tsv=True) into a formats.TsvWriter, whose rows are named from the global cell index `first`), and
+    its formats.TsvRecord is returned.  `compression` picks the device compressor of the compressed forms
+    (stream_csr)."""
     if out == "torch":
         X = engine.draw(rows, s32, seed, first)
         engine.check()
@@ -486,6 +507,12 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
         with MtxWriter(path, (int(rows.numel()), engine.G), *cells, first=first) as w:
             engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *text: w.append(hi - lo, text[3], *text[:3]),
                               mtx=True, compression=compression)
+        return w.record()
+    if out == "tsv":
+        _check_csr_request(out, dtype, path=path, compress=compress, compression=compression)
+        with TsvWriter(path, (int(rows.numel()), engine.G), first=first, compress=compress) as w:
+            engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *text: w.append(hi - lo, *text), tsv=True,
+                              compress=compress, compression=compression)
         return w.record()
     if out == "csr":
         _check_csr_request(out, dtype)
@@ -572,8 +599,9 @@ def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, s
     host_transport ("direct", "i32", "u16", "u8"; with host_out): the format in which the counts cross
     PCIe; the narrow ones are expanded into the int32 / int64 host matrix by `host_threads` host threads
     (0 = all) together with their exact overflow list - the caller receives the same counts either way.
-    out="csr" / "mtx", path, compress, compression: the sparse and on-disk forms of the module docstring; out="mtx",
-    path="counts_10x" writes a 10x directory and returns its formats.MtxRecord."""
+    out="csr" / "mtx" / "tsv", path, compress, compression: the sparse and on-disk forms of the module docstring;
+    out="mtx", path="counts_10x" writes a 10x directory and returns its formats.MtxRecord; out="tsv",
+    path="job_simulation.txt" writes the reference's counts file and returns its formats.TsvRecord."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
@@ -748,7 +776,9 @@ def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, de
     variance = alpha_g mean^2 + beta_g mean).  out="csr", path=p writes the CSR shard with the
     pseudotime, branches and scalings given here and returns its memory-mapped matrix; with compress=True the
     compressed file, and its formats.CompressedCsr record.  out="mtx", path=p writes the 10x directory with
-    them (barcodes cell_<first + i>) and returns its formats.MtxRecord.  compression="lz77": see sample_density."""
+    them (barcodes cell_<first + i>) and returns its formats.MtxRecord.  out="tsv", path=p writes the reference's
+    _simulation.txt (rows cell_<first + i>) and returns its formats.TsvRecord.  compression="lz77": see
+    sample_density."""
     dev = nat.device(device)
     _check_csr_request(out, dtype, path=path, compress=compress, compression=compression)
     seed = nat.split_seed(seed)
