@@ -327,6 +327,20 @@ int pst_delta_write(const void *values, int32_t value_bits, const int64_t *count
  * chunk's local row pointer (indptr[0] = 0). */
 int pst_csr_row_ids(const int64_t *indptr, int64_t n, int64_t first, int64_t *out, void *stream);
 
+/* ---- the chunk grid of a Zarr array (out="zarr", pst_zarr.cu) --------------------------------------------
+ * One array of the store is cut into chunks of chunk_bytes while the engine delivers its values chunk by chunk;
+ * in place of writing each engine chunk's values at a host-known offset.  The carry is the tail that does not fill
+ * a chunk yet: prev_state[0] / prev_state[1] (device int64) are its byte offset in prev and its length.
+ * pst_zarr_cut writes seg = carry || src, src being (*count) * scale bytes (count a device int64, clamped to max_src;
+ * NULL: max_src bytes), then *nchunks = the whole chunks in seg and state = {nchunks * chunk_bytes, the rest}: the
+ * carry for the next call, which passes this seg as its prev.  With `final` the rest is zero-padded to one more
+ * chunk and the carry is empty.  prev and seg are distinct buffers; lengths are multiples of 4 bytes; seg holds
+ * pst_zarr_seg_bytes(max_src, chunk_bytes) bytes. */
+int64_t pst_zarr_seg_bytes(int64_t max_src, int64_t chunk_bytes);
+int pst_zarr_cut(const void *prev, const int64_t *prev_state, const void *src, const int64_t *count, int64_t scale,
+                 int64_t max_src, int64_t chunk_bytes, int32_t final, void *seg, int64_t seg_bytes, int64_t *state,
+                 int64_t *nchunks, void *stream);
+
 /* ---- raw DEFLATE (RFC 1951) on the device: the compressed CSR file (pst_deflate.cu) ---------------
  * The input is cut into blocks of `block` bytes (a multiple of 1024, at most 32768).  Each block becomes
  * one dynamic-Huffman block over the literals 0-255 and end-of-block (no length or distance codes; the
@@ -357,6 +371,19 @@ int64_t pst_deflate_lz_workspace_bytes(int64_t n, int32_t block);
 int pst_deflate_lz_blocks(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes, int32_t block,
                           void *out, int64_t *out_bytes, uint32_t *crc, void *work, int64_t work_bytes,
                           void *stream);
+/* The zlib chunks of a Zarr store (out="zarr"): pst_deflate_blocks / pst_deflate_lz_blocks with the input cut
+ * into segments of seg_blocks blocks, in place of their CRC-32.  Same blocks, bound, workspace and out / out_bytes;
+ * in addition, for nseg = ceil(ceil(max_bytes / block) / seg_blocks), seg_offsets[s] (device int64, nseg + 1
+ * entries) is the offset in out of segment s's first block (seg_offsets[nseg] = *out_bytes), and seg_adler[s]
+ * (device uint32, nseg entries) the Adler-32 (zlib.adler32) of its input bytes.  Segments past the input length
+ * are empty.  So 78 01, out[seg_offsets[s] .. seg_offsets[s+1]), 03 00 and the big-endian seg_adler[s] are one
+ * zlib stream (RFC 1950) of segment s. */
+int pst_deflate_segments(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes, int32_t block,
+                         int64_t seg_blocks, void *out, int64_t *out_bytes, int64_t *seg_offsets, uint32_t *seg_adler,
+                         void *work, int64_t work_bytes, void *stream);
+int pst_deflate_lz_segments(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes, int32_t block,
+                            int64_t seg_blocks, void *out, int64_t *out_bytes, int64_t *seg_offsets,
+                            uint32_t *seg_adler, void *work, int64_t work_bytes, void *stream);
 /* *crc = CRC-32 (zlib.crc32) of the n device bytes at in; crc is a device word. */
 int pst_crc32(const void *in, int64_t n, uint32_t *crc, void *stream);
 

@@ -8,7 +8,8 @@ import sys
 PKG = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG, "csrc")
 LIB = os.path.join(PKG, "libprosstt_b200.so")
-SOURCES = ["pst_index.cu", "pst_lineage.cu", "pst_counts.cu", "pst_epilogue.cu", "pst_deflate.cu", "pst_parquet.cu"]
+SOURCES = ["pst_index.cu", "pst_lineage.cu", "pst_counts.cu", "pst_epilogue.cu", "pst_deflate.cu", "pst_parquet.cu",
+           "pst_zarr.cu"]
 HOST_SOURCES = ["pst_host.cpp"]          # host side of the device->host path (threads, no CUDA)
 HOST_FLAGS = ["-O3", "-std=c++17", "-fPIC", "-fvisibility=hidden", "-pthread", "-Wall", "-Wextra"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",

@@ -14,6 +14,11 @@
 // code lengths.  Then the blocks' sizes are scanned and the blocks compacted into one output.  The
 // CRC-32 of the input is built from per-thread CRCs moved to their place by the GF(2) shift
 // x^(8 * bytes following them) mod P and XOR-ed together: the same word whatever the launch order.
+//
+// Segments (pst_deflate_segments, the zlib chunks of a Zarr store): the same blocks, and per segment of
+// seg_blocks blocks its compressed offset (from the scan of the block sizes) and the Adler-32 of its input.
+// The block kernel then sums its staged block instead of taking its CRC (ADLER), and a small kernel combines
+// the blocks' sums of each segment as zlib's adler32_combine does.
 #include <algorithm>
 #include "pst_common.cuh"
 
@@ -24,7 +29,9 @@ constexpr int kDefThreads = 256;         // one thread per byte value in the his
 constexpr int kMaxBlock = 32768;          // largest block: its stored form must stay below 65 535 bytes
 constexpr int kStoredOverhead = 5;        // stored block header: 1 byte of BFINAL/BTYPE + padding, LEN, NLEN
 constexpr int64_t kSlotPad = 16;          // per-block slot in the workspace: B + 16 bytes
+constexpr int64_t kSumsAt = 8;            // a block's output is at most B + 5 bytes: its Adler sums at B + 8
 constexpr uint32_t kCrcPoly = 0xEDB88320u;
+constexpr uint32_t kAdlerMod = 65521;
 
 // ---------------------------------------------------------------------------------------------
 // CRC-32 (zlib's): table-driven per byte; multmodp / x2nmodp are zlib's GF(2) product and x^(2^k) powers
@@ -118,6 +125,36 @@ __device__ uint32_t block_crc(const uint32_t *s, int len, int seg, const uint32_
   uint32_t all = 0;
   if (threadIdx.x == 0)
     for (int w = 0; w < (int)(blockDim.x >> 5); ++w) all ^= red[w];
+  __syncthreads();
+  return all;
+}
+
+// Adler-32 sums of the staged block (len bytes), valid in thread 0: x = sum b_i and y = sum (len - i) b_i, both
+// mod 65521, so that adler32 = (1 + x) | ((len + y) << 16).  A thread's segment sums stay below 2^22 (at most 128
+// bytes); each is moved to the block's end and reduced before the warps add them up.  `red` holds two words per warp.
+__device__ uint2 block_adler(const uint32_t *s, int len, int seg, uint32_t *red) {
+  int lo, hi;
+  segment(len, seg, lo, hi);
+  uint32_t x = 0, y = 0;                                           // y = sum (hi - i) b_i over the segment
+  for (int i = lo; i < hi; i += 4) {
+    const uint32_t w = staged_word(s, i >> 2);
+    const int k = min(4, hi - i);
+    for (int j = 0; j < k; ++j) { x += (w >> (8 * j)) & 0xFF; y += x; }
+  }
+  y = (uint32_t)(((uint64_t)y + (uint64_t)(len - hi) * x) % kAdlerMod);
+  x %= kAdlerMod;
+  for (int d = 16; d; d >>= 1) {
+    x += __shfl_xor_sync(0xffffffffu, x, d);
+    y += __shfl_xor_sync(0xffffffffu, y, d);
+  }
+  if ((threadIdx.x & 31) == 0) { red[2 * (threadIdx.x >> 5)] = x; red[2 * (threadIdx.x >> 5) + 1] = y; }
+  __syncthreads();
+  uint2 all = make_uint2(0, 0);
+  if (threadIdx.x == 0) {
+    for (int w = 0; w < (int)(blockDim.x >> 5); ++w) { all.x += red[2 * w]; all.y += red[2 * w + 1]; }
+    all.x %= kAdlerMod;
+    all.y %= kAdlerMod;
+  }
   __syncthreads();
   return all;
 }
@@ -309,7 +346,7 @@ struct HuffShared {
   uint32_t crc_table[256];
   uint32_t x2n[32];
   int count[33], next[16];
-  uint32_t red[kDefThreads / 32];
+  uint32_t red[2 * (kDefThreads / 32)];
   long long scan[kDefThreads / 32];
   int header_bits, stored;
   long long total_bits;
@@ -317,8 +354,10 @@ struct HuffShared {
 
 // ---------------------------------------------------------------------------------------------
 // one CTA per block b: block bytes in[b*B, min((b+1)*B, n)), written to slot b of the workspace
-// (B + 16 bytes), its size to sizes[b]; its CRC, shifted past the rest of the input, XOR-ed into *crc
+// (B + 16 bytes), its size to sizes[b]; its CRC, shifted past the rest of the input, XOR-ed into *crc, or with
+// ADLER its Adler sums (block_adler) at byte B + 8 of the slot
 // ---------------------------------------------------------------------------------------------
+template <bool ADLER>
 __global__ void __launch_bounds__(kDefThreads)
 deflate_block_kernel(const uint8_t *__restrict__ in, const int64_t *__restrict__ count, int64_t scale,
                      int64_t max_bytes, int block, uint8_t *__restrict__ slots, int32_t *__restrict__ sizes,
@@ -340,7 +379,7 @@ deflate_block_kernel(const uint8_t *__restrict__ in, const int64_t *__restrict__
   stage_block(in + start, len, staged);
   for (int i = tid; i < bit_words; i += blockDim.x) bits[i] = 0;
   for (int i = tid; i < (kDefThreads / 32) * 257; i += blockDim.x) (&sh.hist[0][0])[i] = 0;
-  crc_tables(sh.crc_table, sh.x2n);
+  if (!ADLER) crc_tables(sh.crc_table, sh.x2n);
   __syncthreads();
 
   // ---- histogram: word w of the block per thread and round, its four bytes aggregated over the warp
@@ -356,7 +395,10 @@ deflate_block_kernel(const uint8_t *__restrict__ in, const int64_t *__restrict__
       __syncwarp();
     }
   }
-  const uint32_t crc = block_crc(staged, len, seg, sh.crc_table, sh.x2n, sh.red);   // synchronises
+  uint32_t crc = 0;
+  uint2 sums = make_uint2(0, 0);
+  if (ADLER) sums = block_adler(staged, len, seg, sh.red);                           // synchronises
+  else crc = block_crc(staged, len, seg, sh.crc_table, sh.x2n, sh.red);              // synchronises
   for (int s = tid; s < 257; s += blockDim.x) {
     uint32_t f = (s == 256) ? 1u : 0u;                             // end-of-block
     if (s < 256)
@@ -456,7 +498,10 @@ deflate_block_kernel(const uint8_t *__restrict__ in, const int64_t *__restrict__
     const int nbytes = sizes[blockIdx.x];
     for (int w = tid; w < (nbytes + 3) / 4; w += blockDim.x) reinterpret_cast<uint32_t *>(slot)[w] = bits[w];
   }
-  if (tid == 0) atomicXor(crc_out, crc_shift(crc, n - start - len, sh.x2n));
+  if (tid == 0) {
+    if (ADLER) *reinterpret_cast<uint2 *>(slot + block + kSumsAt) = sums;
+    else atomicXor(crc_out, crc_shift(crc, n - start - len, sh.x2n));
+  }
 }
 
 // ---------------------------------------------------------------------------------------------
@@ -538,7 +583,7 @@ struct LzShared {
   uint32_t crc_table[256];
   uint32_t x2n[32];
   int count[33], next[16];
-  uint32_t red[kLzWarps];
+  uint32_t red[2 * kLzWarps];
   long long scan[kLzWarps];
   int ntok[kMaxBlock / kLzSeg];           // tokens of each segment
   int header_bits, stored;
@@ -551,6 +596,7 @@ inline size_t lz_scratch_bytes(int32_t block) {
 }
 
 // one CTA per block b, as deflate_block_kernel; tokens: the block's slot of `block` uint16 entries
+template <bool ADLER>
 __global__ void __launch_bounds__(kLzThreads)
 deflate_lz_block_kernel(const uint8_t *__restrict__ in, const int64_t *__restrict__ count, int64_t scale,
                         int64_t max_bytes, int block, uint8_t *__restrict__ slots, int32_t *__restrict__ sizes,
@@ -572,7 +618,7 @@ deflate_lz_block_kernel(const uint8_t *__restrict__ in, const int64_t *__restric
   if (tid == 0) staged[padded_word((len + 3) >> 2)] = 0;           // the word past the block's last one
   for (int i = tid; i < (kLzWarps << kHashBits); i += blockDim.x) scratch[i] = kNone;
   for (int s = tid; s < kLitSyms + kDistSyms; s += blockDim.x) { sh.freq[s] = (s == 256); sh.len[s] = 0; }
-  crc_tables(sh.crc_table, sh.x2n);
+  if (!ADLER) crc_tables(sh.crc_table, sh.x2n);
   __syncthreads();
 
   // ---- 1. hash chains: warp w over its region, then the first positions of each region
@@ -762,8 +808,14 @@ deflate_lz_block_kernel(const uint8_t *__restrict__ in, const int64_t *__restric
     const int nbytes = sizes[blockIdx.x];
     for (int w = tid; w < (nbytes + 3) / 4; w += blockDim.x) reinterpret_cast<uint32_t *>(slot)[w] = bits[w];
   }
-  const uint32_t crc = block_crc(staged, len, ((block / kLzThreads) + 3) & ~3, sh.crc_table, sh.x2n, sh.red);
-  if (tid == 0) atomicXor(crc_out, crc_shift(crc, n - start - len, sh.x2n));
+  const int seg = ((block / kLzThreads) + 3) & ~3;
+  if (ADLER) {
+    const uint2 sums = block_adler(staged, len, seg, sh.red);
+    if (tid == 0) *reinterpret_cast<uint2 *>(slot + block + kSumsAt) = sums;
+  } else {
+    const uint32_t crc = block_crc(staged, len, seg, sh.crc_table, sh.x2n, sh.red);
+    if (tid == 0) atomicXor(crc_out, crc_shift(crc, n - start - len, sh.x2n));
+  }
 }
 
 // CRC-32 only: one CTA per block, as in deflate_block_kernel
@@ -794,6 +846,31 @@ deflate_compact_kernel(const uint8_t *__restrict__ slots, const int32_t *__restr
   }
 }
 
+// segment s = blocks [s*seg_blocks, (s+1)*seg_blocks): seg_offsets[s] = offsets of its first block (the total for
+// s = nseg), seg_adler[s] = Adler-32 of its input, its blocks' sums combined as zlib's adler32_combine: for A || B,
+// x = x_A + x_B and y = y_A + |B| x_A + y_B.  Blocks past the input length n are empty.
+__global__ void __launch_bounds__(kDefThreads)
+adler_segments_kernel(const uint8_t *__restrict__ slots, const int64_t *__restrict__ offsets,
+                      const int64_t *__restrict__ count, int64_t scale, int64_t max_bytes, int block, int64_t nb,
+                      int64_t seg_blocks, int64_t nseg, int64_t *__restrict__ seg_offsets,
+                      uint32_t *__restrict__ seg_adler) {
+  const int64_t n = count ? min(max_bytes, count[0] * scale) : max_bytes;
+  for (int64_t s = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; s <= nseg; s += (int64_t)gridDim.x * blockDim.x) {
+    const int64_t b0 = min(s * seg_blocks, nb);
+    seg_offsets[s] = offsets[b0];
+    if (s == nseg) continue;
+    uint64_t x = 0, y = 0, total = 0;
+    for (int64_t b = b0; b < min(nb, b0 + seg_blocks) && b * block < n; ++b) {
+      const int64_t len = min((int64_t)block, n - b * block);
+      const uint2 sums = *reinterpret_cast<const uint2 *>(slots + b * (block + kSlotPad) + block + kSumsAt);
+      y = (y + (uint64_t)len * x + sums.y) % kAdlerMod;
+      x = (x + sums.x) % kAdlerMod;
+      total += (uint64_t)len;
+    }
+    seg_adler[s] = (uint32_t)((1 + x) % kAdlerMod) | ((uint32_t)((total + y) % kAdlerMod) << 16);
+  }
+}
+
 inline int64_t n_blocks(int64_t n, int32_t block) { return (n + block - 1) / block; }
 inline int64_t align16(int64_t v) { return (v + 15) / 16 * 16; }
 inline size_t staged_bytes(int32_t block) { return (size_t)(block / 4 + block / 128 + 4) * 4; }
@@ -819,20 +896,38 @@ extern "C" int64_t pst_deflate_lz_workspace_bytes(int64_t n, int32_t block) {
   return pst_deflate_workspace_bytes(n, block) + n_blocks(n, block) * 2 * block;
 }
 
+// the dynamic shared memory limit of one kernel, raised once per device and thread
+template <bool LZ, bool ADLER, typename K>
+static void allow_smem(K kernel, size_t bytes) {
+  static thread_local int configured_dev = -1;
+  int dev = 0;
+  cudaGetDevice(&dev);
+  if (configured_dev != dev) {
+    cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)bytes);
+    configured_dev = dev;
+  }
+}
+
 // pst_deflate_blocks (lz false) and pst_deflate_lz_blocks (lz true): the block kernel, the scan of the
-// block sizes and the compaction; the LZ workspace has the token slots after the output slots
+// block sizes and the compaction; the LZ workspace has the token slots after the output slots.  With seg_offsets
+// (pst_deflate_segments, pst_deflate_lz_segments) the block kernel takes Adler sums instead of the CRC, and
+// adler_segments_kernel writes the segments' offsets and Adler-32s after the scan.
 static int deflate_launch(const char *fn, bool lz, const void *in, const int64_t *count, int64_t scale,
                           int64_t max_bytes, int32_t block, void *out, int64_t *out_bytes, uint32_t *crc, void *work,
-                          int64_t work_bytes, void *stream) {
+                          int64_t work_bytes, void *stream, int64_t seg_blocks = 0, int64_t *seg_offsets = nullptr,
+                          uint32_t *seg_adler = nullptr) {
+  const bool adler = seg_offsets != nullptr;
   PST_REQUIRE(max_bytes >= 0 && scale >= 0, fn, "need max_bytes, scale >= 0");
   PST_REQUIRE(block >= 1024 && block <= kMaxBlock && block % 1024 == 0, fn,
               "block must be a multiple of 1024 between 1024 and 32768");
-  PST_REQUIRE(out_bytes && crc, fn, "null pointer");
+  PST_REQUIRE(out_bytes && (adler ? seg_adler != nullptr : crc != nullptr), fn, "null pointer");
+  PST_REQUIRE(!adler || seg_blocks >= 1, fn, "need seg_blocks >= 1");
   cudaStream_t st = (cudaStream_t)stream;
   const int64_t nb = n_blocks(max_bytes, block);
-  if (cudaMemsetAsync(crc, 0, sizeof(uint32_t), st) != cudaSuccess) return check_launch(fn);
+  if (!adler && cudaMemsetAsync(crc, 0, sizeof(uint32_t), st) != cudaSuccess) return check_launch(fn);
   if (nb == 0) {
     if (cudaMemsetAsync(out_bytes, 0, sizeof(int64_t), st) != cudaSuccess) return check_launch(fn);
+    if (adler && cudaMemsetAsync(seg_offsets, 0, sizeof(int64_t), st) != cudaSuccess) return check_launch(fn);
     return 0;
   }
   PST_REQUIRE(in && out && work, fn, "null pointer");
@@ -846,29 +941,32 @@ static int deflate_launch(const char *fn, bool lz, const void *in, const int64_t
   int32_t *sizes = reinterpret_cast<int32_t *>(work);
   int64_t *offsets = reinterpret_cast<int64_t *>(static_cast<uint8_t *>(work) + align16(4 * nb));
   uint8_t *slots = static_cast<uint8_t *>(work) + align16(4 * nb) + align16(8 * (nb + 1));
-  int dev = 0;
-  cudaGetDevice(&dev);
+  const uint8_t *src = static_cast<const uint8_t *>(in);
   if (lz) {
-    static thread_local int configured_dev = -1;
-    if (configured_dev != dev) {
-      cudaFuncSetAttribute(deflate_lz_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)(staged_bytes(kMaxBlock) + 2 * kMaxBlock + lz_scratch_bytes(kMaxBlock)));
-      configured_dev = dev;
-    }
+    const size_t most = staged_bytes(kMaxBlock) + 2 * kMaxBlock + lz_scratch_bytes(kMaxBlock);
     uint16_t *tokens = reinterpret_cast<uint16_t *>(slots + nb * (block + kSlotPad));
     const size_t smem = staged_bytes(block) + 2 * (size_t)block + lz_scratch_bytes(block);
-    deflate_lz_block_kernel<<<(unsigned)nb, kLzThreads, smem, st>>>(static_cast<const uint8_t *>(in), count, scale,
-                                                                    max_bytes, block, slots, sizes, crc, tokens);
-  } else {
-    static thread_local int configured_dev = -1;
-    if (configured_dev != dev) {
-      cudaFuncSetAttribute(deflate_block_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                           (int)(staged_bytes(kMaxBlock) + (kMaxBlock / 4 + 8) * 4));
-      configured_dev = dev;
+    if (adler) {
+      allow_smem<true, true>(deflate_lz_block_kernel<true>, most);
+      deflate_lz_block_kernel<true><<<(unsigned)nb, kLzThreads, smem, st>>>(src, count, scale, max_bytes, block, slots,
+                                                                            sizes, nullptr, tokens);
+    } else {
+      allow_smem<true, false>(deflate_lz_block_kernel<false>, most);
+      deflate_lz_block_kernel<false><<<(unsigned)nb, kLzThreads, smem, st>>>(src, count, scale, max_bytes, block, slots,
+                                                                             sizes, crc, tokens);
     }
+  } else {
+    const size_t most = staged_bytes(kMaxBlock) + (kMaxBlock / 4 + 8) * 4;
     const size_t smem = staged_bytes(block) + (size_t)(block / 4 + 8) * 4;
-    deflate_block_kernel<<<(unsigned)nb, kDefThreads, smem, st>>>(static_cast<const uint8_t *>(in), count, scale,
-                                                                  max_bytes, block, slots, sizes, crc);
+    if (adler) {
+      allow_smem<false, true>(deflate_block_kernel<true>, most);
+      deflate_block_kernel<true><<<(unsigned)nb, kDefThreads, smem, st>>>(src, count, scale, max_bytes, block, slots,
+                                                                          sizes, nullptr);
+    } else {
+      allow_smem<false, false>(deflate_block_kernel<false>, most);
+      deflate_block_kernel<false><<<(unsigned)nb, kDefThreads, smem, st>>>(src, count, scale, max_bytes, block, slots,
+                                                                           sizes, crc);
+    }
   }
   int rc = check_launch(fn);
   if (rc) return rc;
@@ -877,6 +975,12 @@ static int deflate_launch(const char *fn, bool lz, const void *in, const int64_t
   const unsigned grid = (unsigned)std::min<int64_t>(nb, (int64_t)num_sm() * 8);
   deflate_compact_kernel<<<grid, kDefThreads, 0, st>>>(slots, sizes, offsets, nb, block,
                                                        static_cast<uint8_t *>(out), out_bytes);
+  if (adler) {
+    const int64_t nseg = (nb + seg_blocks - 1) / seg_blocks;
+    const unsigned sgrid = (unsigned)std::min<int64_t>((nseg + kDefThreads) / kDefThreads, (int64_t)num_sm() * 8);
+    adler_segments_kernel<<<sgrid, kDefThreads, 0, st>>>(slots, offsets, count, scale, max_bytes, block, nb, seg_blocks,
+                                                         nseg, seg_offsets, seg_adler);
+  }
   return check_launch(fn);
 }
 
@@ -892,6 +996,26 @@ extern "C" int pst_deflate_lz_blocks(const void *in, const int64_t *count, int64
                                      int64_t work_bytes, void *stream) {
   return deflate_launch("pst_deflate_lz_blocks", true, in, count, scale, max_bytes, block, out, out_bytes, crc,
                         work, work_bytes, stream);
+}
+
+extern "C" int pst_deflate_segments(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes,
+                                    int32_t block, int64_t seg_blocks, void *out, int64_t *out_bytes,
+                                    int64_t *seg_offsets, uint32_t *seg_adler, void *work, int64_t work_bytes,
+                                    void *stream) {
+  const char *fn = "pst_deflate_segments";
+  PST_REQUIRE(seg_offsets, fn, "null pointer");
+  return deflate_launch(fn, false, in, count, scale, max_bytes, block, out, out_bytes, nullptr, work, work_bytes,
+                        stream, seg_blocks, seg_offsets, seg_adler);
+}
+
+extern "C" int pst_deflate_lz_segments(const void *in, const int64_t *count, int64_t scale, int64_t max_bytes,
+                                       int32_t block, int64_t seg_blocks, void *out, int64_t *out_bytes,
+                                       int64_t *seg_offsets, uint32_t *seg_adler, void *work, int64_t work_bytes,
+                                       void *stream) {
+  const char *fn = "pst_deflate_lz_segments";
+  PST_REQUIRE(seg_offsets, fn, "null pointer");
+  return deflate_launch(fn, true, in, count, scale, max_bytes, block, out, out_bytes, nullptr, work, work_bytes,
+                        stream, seg_blocks, seg_offsets, seg_adler);
 }
 
 extern "C" int pst_crc32(const void *in, int64_t n, uint32_t *crc, void *stream) {

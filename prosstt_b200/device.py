@@ -12,7 +12,8 @@ import torch
 
 from prosstt_b200 import _native as nat
 from prosstt_b200 import hostpool
-from prosstt_b200.formats import sync_deflate
+from prosstt_b200 import formats
+from prosstt_b200.formats import sync_deflate, zarr_chunks
 
 
 def tree_tables(tree, dev):
@@ -222,6 +223,8 @@ _DEFLATE_BLOCK = 32768                        # bytes per DEFLATE block of the c
 # stream_csr's `compression`: the device compressor, its workspace size and the workspace's token bytes per input byte
 _DEFLATE = {"huffman": ("pst_deflate_blocks", "pst_deflate_workspace_bytes", 0),
             "lz77": ("pst_deflate_lz_blocks", "pst_deflate_lz_workspace_bytes", 2)}
+# the same compressors cutting their input into zlib streams, one per Zarr chunk (stream_csr(zarr=True))
+_DEFLATE_SEGMENTS = {"huffman": "pst_deflate_segments", "lz77": "pst_deflate_lz_segments"}
 # stream_csr's per-chunk record of int64 slots, read by the host one chunk late: those of every format, then its own
 _REC_SAT, _REC_NNZ, _REC_STATUS, _REC_OWN = range(4)
 _REC_SLOTS = _REC_OWN + 15                    # Parquet has the most slots of its own: 5 for each of its 3 pages
@@ -617,7 +620,7 @@ class CountEngine(object):
 
     def stream_csr(self, rows, scaling32, seed, cell0, consume, index_dtype=np.int64, data_dtype=np.int64,
                    chunk_cells=None, threads=0, overflow_cap=None, compress=False, mtx=False, compression="huffman",
-                   tsv=False, parquet=False):
+                   tsv=False, parquet=False, zarr=False):
         """Sample the cells in chunks and hand each one as CSR to consume(lo, hi, indptr, indices, data), on a
         worker thread, once per chunk, in cell order.  indptr is chunk-local int64 (hi - lo + 1 entries from 0);
         indices and data are the chunk's nonzeros in `index_dtype` / `data_dtype` (int32 or int64), columns
@@ -653,6 +656,13 @@ class CountEngine(object):
         that decompresses to them, whose CRC-32 is crc.  min and max are those of the column's values.  index_dtype
         does not apply.
 
+        zarr=True: consume(lo, hi, nnz, parts) receives the Zarr chunks of formats.ZARR_CHUNK elements that the chunk
+        completes in the arrays indptr (int64, the leading 0 first, then the row ends after the nonzeros before the
+        chunk), indices (int32) and data (data_dtype) of the csr_matrix, parts = [indptr chunks, indices chunks, data
+        chunks] (formats.ZarrWriter.append): a chunk is its raw bytes, or with compress=True (raw DEFLATE blocks that
+        decompress to them, their Adler-32, their length); the last chunk of the call pads each array to a whole
+        chunk with zeros.  Chunks are views of reused host buffers.  index_dtype does not apply.
+
         compression ("huffman" or "lz77", with compress=True or mtx=True): the device compressor,
         pst_deflate_blocks (Huffman-only) or pst_deflate_lz_blocks (LZ77 matches within each 32 KiB block,
         smaller output, a larger workspace).  Both write the same framing, so the consumer is the same."""
@@ -670,6 +680,7 @@ class CountEngine(object):
         cell_bytes, empty, start = (
             self._mtx_encoder(n, consume, compression) if mtx else
             self._parquet_encoder(n, consume, data_dtype, compress, compression, cell0) if parquet else
+            self._zarr_encoder(n, consume, data_dtype, compress, compression) if zarr else
             self._tsv_encoder(n, consume, compress, compression, cell0) if tsv else
             self._npz_encoder(n, consume, index_dtype, data_dtype, compression) if compress else
             self._shard_encoder(n, consume, index_dtype, data_dtype, threads, overflow_cap))
@@ -1053,6 +1064,108 @@ class CountEngine(object):
         # tokens of the largest page; at most _PARQUET_PAGE_VALUES values per chunk
         cell_bytes = (2 * (12 + dsz) + tokens * 8) * G
         return max(cell_bytes, -(-_STAGE_BYTES // max(1, _PARQUET_PAGE_VALUES // max(1, G)))), empty, start
+
+    def _zarr_encoder(self, n, consume, data_dtype, compress, compression):
+        """stream_csr(zarr=True): pst_csr_pack writes the int32 indices and data_dtype data and pst_csr_indptr_bytes the
+        int64 row ends after a running nnz kept on the device, all shared by both k.  For each array pst_zarr_cut then
+        writes `carry || new values` into segment buffer k: the carry is the tail of chunk i - 1's segment buffer
+        that did not fill a Zarr chunk (at first indptr's leading 0), its place on the device.  The whole chunks of
+        segment buffer k are copied as they are or, with compress, pst_deflate_segments compresses them into one zlib
+        stream each (their blocks, offsets and Adler-32s cross PCIe).  The host follows the carries from the records
+        and checks the chunk counts of the device against them; a chunk is never encoded again.  Record: per array
+        the whole chunks, then the compressed sizes."""
+        G, dev, st, lib, block = self.G, self.dev, nat.stream_ptr(self.dev), nat.load(), _DEFLATE_BLOCK
+        deflate_work, tokens = _DEFLATE[compression][1:]
+        chunk_values = int(formats.ZARR_CHUNK)
+        if chunk_values <= 0 or chunk_values % 8192:
+            raise ValueError("formats.ZARR_CHUNK must be a positive multiple of 8192, not %d" % chunk_values)
+        dsz = data_dtype.itemsize
+        esz = (8, 4, dsz)                                               # indptr, indices, data
+        cb = [chunk_values * e for e in esz]                            # bytes of one Zarr chunk of each array
+        NSEG, SIZE = _REC_OWN, _REC_OWN + 3
+
+        def empty():                                    # G == 0: indptr n + 1 zeros, no nonzeros
+            consume(0, n, 0, [zarr_chunks(bytes(8 * (n + 1)), cb[0], compress), [], []])
+
+        def start(chunk, work, indptr, info, pack_flags):
+            most = (chunk * 8, chunk * G * 4, chunk * G * dsz)
+            wide = [torch.empty(max(1, m), dtype=torch.uint8, device=dev) for m in most]
+            seg_bytes = [int(lib.pst_zarr_seg_bytes(m, c)) for m, c in zip(most, cb)]
+            seg = [[torch.empty(b, dtype=torch.uint8, device=dev) for b in seg_bytes] for _ in range(2)]
+            state = torch.zeros((2, 3, 2), dtype=torch.int64, device=dev)      # carry: byte offset, bytes
+            first = torch.tensor([[0, 8], [0, 0], [0, 0]], dtype=torch.int64).to(dev)
+            zero = torch.zeros(16, dtype=torch.uint8, device=dev)               # indptr's leading 0
+            running = torch.zeros(1, dtype=torch.int64, device=dev)
+            nseg = [b // c for b, c in zip(seg_bytes, cb)]
+            if compress:
+                packed = [[torch.empty(int(lib.pst_deflate_bound(b, block)), dtype=torch.uint8, device=dev)
+                           for b in seg_bytes] for _ in range(2)]
+                offsets = [[torch.empty(s + 1, dtype=torch.int64, device=dev) for s in nseg] for _ in range(2)]
+                adler = [[torch.empty(s, dtype=torch.int32, device=dev) for s in nseg] for _ in range(2)]
+                dwork_bytes = max(int(getattr(lib, deflate_work)(b, block)) for b in seg_bytes)
+                dwork = torch.empty(dwork_bytes, dtype=torch.uint8, device=dev)
+                # per array its blocks, nseg + 1 offsets and nseg Adler-32s, each copy starting on 64 bytes
+                host_bytes = sum(p.numel() + 12 * s + 8 + 3 * 64 for p, s in zip(packed[0], nseg))
+            else:
+                host_bytes = sum(seg_bytes) + 3 * 64
+            stage_host = _pinned_staging(dev, host_bytes)
+            carry, rows = [1, 0, 0], [0]                # the host's view of the carries, in values: indptr's 0
+
+            def step(k, lo, cells):
+                nat.call("pst_csr_pack", work[k].data_ptr(), cells, G, G, indptr[k], 0, wide[1], 32, wide[2], 8 * dsz,
+                         None, None, 0, None, pack_flags, st)
+                nat.call("pst_csr_indptr_bytes", indptr[k], cells, running, wide[0], 64, st)
+                nnz = indptr[k][cells:cells + 1]
+                final = int(lo + cells == n)
+                for j, (count, scale, m) in enumerate(((None, 0, cells * 8), (nnz, 4, cells * G * 4),
+                                                       (nnz, dsz, cells * G * dsz))):
+                    prev, prev_state = (zero, first[j]) if lo == 0 else (seg[k ^ 1][j], state[k ^ 1, j])
+                    nat.call("pst_zarr_cut", prev, prev_state, wide[j], count, scale, m, cb[j], final, seg[k][j],
+                             seg_bytes[j], state[k, j], info[k, NSEG + j], st)
+                    if compress:
+                        nat.call(_DEFLATE_SEGMENTS[compression], seg[k][j], info[k, NSEG + j], cb[j], seg_bytes[j],
+                                 block, cb[j] // block, packed[k][j], info[k, SIZE + j], offsets[k][j], adler[k][j],
+                                 dwork, dwork_bytes, st)
+
+            def copies(k, cells, record):
+                rows[0] += cells
+                final = rows[0] == n
+                pairs, at = [], 0
+                for j, new in enumerate((cells, record[_REC_NNZ], record[_REC_NNZ])):
+                    carry[j] += new
+                    whole = -(-carry[j] // chunk_values) if final else carry[j] // chunk_values
+                    carry[j] = 0 if final else carry[j] - whole * chunk_values
+                    if record[NSEG + j] != whole:
+                        raise RuntimeError("X/%s: the device cut %d Zarr chunks, the host expects %d"
+                                           % (("indptr", "indices", "data")[j], record[NSEG + j], whole))
+                    if compress:
+                        srcs = [packed[k][j][:record[SIZE + j]], offsets[k][j][:whole + 1].view(torch.uint8),
+                                adler[k][j][:whole].view(torch.uint8)]
+                    else:
+                        srcs = [seg[k][j][:whole * cb[j]]]
+                    for src in srcs:
+                        pairs.append((src, stage_host[k][at:at + src.numel()]))
+                        at = (at + src.numel() + 63) // 64 * 64
+                return pairs
+
+            def deliver(dsts, lo, hi, record):
+                parts = []
+                for j in range(3):
+                    if compress:
+                        blocks, offs, adl = dsts[3 * j].numpy(), dsts[3 * j + 1].numpy().view(np.int64), \
+                            dsts[3 * j + 2].numpy().view(np.uint32)
+                        parts.append([(blocks[offs[s]:offs[s + 1]], int(adl[s]), cb[j]) for s in range(len(adl))])
+                    else:
+                        raw = dsts[j].numpy()
+                        parts.append([raw[s * cb[j]:(s + 1) * cb[j]] for s in range(len(raw) // cb[j])])
+                consume(lo, hi, record[_REC_NNZ], parts)
+
+            return step, (lambda k, record: False), None, copies, deliver
+
+        # per cell: the packed values and one segment buffer and, with compress, its compressed form and the workspace's
+        # tokens (the device buffers of one k beside the shared ones; the pinned staging of k holds at most the segment
+        # buffer or its compressed form)
+        return (2 + (1 + tokens) * compress) * (4 + dsz) * G, empty, start
 
     def _dense_chunks(self, rows, scaling32, seed, cell0, tdt, chunk_cells, overflow_cap, host_out=None,
                       consume=None):

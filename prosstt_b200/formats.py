@@ -38,11 +38,17 @@ added, both readable without this package:
   encodes each chunk's columns as DELTA_BINARY_PACKED pages (pst_delta_sizes, pst_delta_write) and, with
   compress=True, gzips them, so only the pages cross PCIe.  The writer serializes the Parquet metadata itself (no
   pyarrow).  The call returns a `ParquetRecord`.
+* AnnData Zarr stores (`ZarrWriter`, written by `out="zarr", path=...`): a Zarr v2 directory in AnnData's on-disk
+  layout, X as a csr_matrix group and obs as the reference's _cellparams.txt, that `anndata.read_zarr`, zarr-python,
+  dask and AnnData's lazy readers open.  The GPU cuts each array into Zarr chunks of `ZARR_CHUNK` elements
+  (pst_zarr_cut) and, with compress=True, compresses every chunk into one zlib stream (pst_deflate_segments), so
+  only the chunks' bytes cross PCIe.  The call returns a `ZarrRecord`.
 """
 import collections
 import concurrent.futures
 import errno
 import io
+import json
 import os
 import shutil
 import struct
@@ -1082,6 +1088,256 @@ class ParquetWriter(object):
         if self._fh is not None:
             self._fh.close()
         self._fh = None
+        shutil.rmtree(self._dir, ignore_errors=True)
+
+    def __enter__(self):
+        return self
+
+    def __exit__(self, exc_type, exc, tb):
+        if exc_type is None:
+            self.close()
+        else:
+            self.abort()
+        return False
+
+
+# ---------------------------------------------------------------------------------------------- AnnData Zarr store
+ZARR_CHUNK = 1 << 20            # elements per chunk of every array of a store: 4 or 8 MiB, whole 32 KiB DEFLATE blocks
+_ZLIB_HEADER = b"\x78\x01"      # CM 8 (DEFLATE), 32 KiB window, FLEVEL 0, no dictionary
+_ZARR_COMPRESSOR = {"id": "zlib", "level": 1}
+_ZARR_X = (("indptr", np.dtype("<i8")), ("indices", np.dtype("<i4")), ("data", None))
+_ZARR_DICTS = ("obsm", "varm", "obsp", "varp", "layers", "uns")
+
+
+def _zarr_json(obj):
+    return json.dumps(obj, indent=4, sort_keys=True, ensure_ascii=True).encode("ascii")
+
+
+def zarr_chunks(raw, chunk_bytes, compress):
+    """The chunks of an array's raw bytes as ZarrWriter.append takes them, the last zero-padded to chunk_bytes: raw
+    bytes, or with compress (raw DEFLATE blocks that are not final, Adler-32, chunk_bytes) made by zlib."""
+    raw = bytes(raw)
+    out = []
+    for at in range(0, len(raw), chunk_bytes):
+        piece = raw[at:at + chunk_bytes].ljust(chunk_bytes, b"\0")
+        if compress:
+            c = zlib.compressobj(1, zlib.DEFLATED, -15)
+            piece = (c.compress(piece) + c.flush(zlib.Z_SYNC_FLUSH), zlib.adler32(piece), chunk_bytes)
+        out.append(piece)
+    return out
+
+
+def _vlen_utf8(items, size):
+    """numcodecs' VLenUTF8 encoding of `items` padded with empty strings to `size` items: the item count, then each
+    item's byte length and UTF-8 bytes (little-endian uint32s).  Assembled with NumPy: a chunk holds 2^20 items."""
+    coded = [v.encode("utf-8") for v in items]
+    lens = np.fromiter(map(len, coded), np.int64, len(coded))
+    before = np.cumsum(lens) - lens                          # payload bytes of the items before each one
+    out = np.zeros(4 + 4 * size + int(lens.sum()), np.uint8)  # the padding items are zero lengths
+    out[:4] = np.frombuffer(struct.pack("<I", size), np.uint8)
+    at = 4 + 4 * np.arange(len(coded)) + before              # each item's length field
+    for k in range(4):
+        out[at + k] = (lens >> (8 * k)) & 0xFF
+    out[np.repeat(at + 4 - before, lens) + np.arange(int(lens.sum()))] = np.frombuffer(b"".join(coded), np.uint8)
+    return out.tobytes()
+
+
+def _codes_dtype(categories):
+    """pandas' rule for the codes of a categorical: the smallest signed integer type below whose maximum the number
+    of categories stays."""
+    for dt in (np.int8, np.int16, np.int32):
+        if categories < np.iinfo(dt).max:
+            return np.dtype(dt)
+    return np.dtype(np.int64)
+
+
+class ZarrRecord(collections.namedtuple("ZarrRecord", "path shape nnz nbytes compressed")):
+    """The X of an out="zarr" call: an AnnData Zarr store on disk.  shape is (cells, genes) of the call; nbytes is
+    the size of the chunk files of X; load() reads X back as the cells x genes csr_matrix with json, zlib and NumPy
+    (anndata.read_zarr(path) reads the whole AnnData)."""
+    __slots__ = ()
+
+    def load(self):
+        def array(name):
+            folder = os.path.join(self.path, "X", name)
+            with open(os.path.join(folder, ".zarray")) as fh:
+                meta = json.load(fh)
+            (length,), (chunk,), dt = meta["shape"], meta["chunks"], np.dtype(meta["dtype"])
+            out = np.empty(length, dt)
+            for c, at in enumerate(range(0, length, chunk)):
+                with open(os.path.join(folder, str(c)), "rb") as fh:
+                    raw = fh.read()
+                if meta["compressor"] is not None:
+                    raw = zlib.decompress(raw)
+                piece = np.frombuffer(raw, dt)
+                out[at:at + chunk] = piece[:min(chunk, length - at)]
+            return out
+
+        indptr, indices, data = (array(name) for name, _ in _ZARR_X)
+        idx = np.int32 if len(indices) < (1 << 31) else np.int64
+        return _csr_matrix(indptr.astype(idx), indices.astype(idx), data, tuple(self.shape))
+
+
+class ZarrWriter(object):
+    """Writer of one AnnData store in Zarr v2 format (anndata's on-disk specification), X appended chunk by chunk:
+      X         csr_matrix group (shape [cells, genes]): indptr int64 (cells + 1 values from 0), indices int32 (genes
+                ascending in a cell) and data (`dtype`, int64 or int32);
+      obs       dataframe of the reference's _cellparams.txt (tree_utils.cell_params_frame): index cell_<first + i>,
+                pseudotime int64, branches categorical (categories the sorted names, codes pandas' smallest type),
+                scalings float64;
+      var       dataframe with index gene_<j> and no columns;
+      obsm, varm, obsp, varp, layers, uns   empty dicts;
+      .zmetadata  the consolidated metadata: every .zgroup, .zattrs and .zarray by its key.
+    Every array has chunks of ZARR_CHUNK elements (as it was when the writer was made) named 0, 1, ...; the last one
+    is stored at full size, zero-padded (empty strings for string arrays).  compress=True gives every array the zlib
+    compressor: each chunk file is one zlib stream.  The host writes obs, var and the metadata.
+
+    append(rows, nnz, parts) takes the next `rows` cells and their `nnz` nonzeros as the complete chunks they fill
+    (the tail that does not fill a chunk comes with a later append; the last append pads it to a whole chunk), parts =
+    [indptr chunks, indices chunks, data chunks]: each chunk is its raw bytes, or with compress=True a tuple (raw
+    DEFLATE blocks that are not final and end on a byte boundary, Adler-32 of the raw chunk, raw length), as
+    pst_deflate_segments or zarr_chunks make them.  As ParquetWriter: everything goes to `<path>.partial`, renamed to
+    `<path>` only by a complete close(), which checks that every array has ceil(length / chunk) chunks; an exception
+    inside `with` or abort() leaves nothing behind; an existing `<path>` raises FileExistsError; the same appends
+    give the same bytes."""
+
+    def __init__(self, path, shape, pseudotime, branches, scalings, first=0, dtype=np.int64, compress=False):
+        self.path = os.fspath(path)
+        if os.path.lexists(self.path):
+            raise FileExistsError(errno.EEXIST, "the Zarr store exists already", self.path)
+        n, G = (int(v) for v in shape)
+        self.shape, self.first, self.compress = (n, G), int(first), bool(compress)
+        self.dtype = np.dtype(dtype)
+        if self.dtype not in (np.dtype(np.int32), np.dtype(np.int64)):
+            raise ValueError("X/data is int32 or int64, not %s" % self.dtype)
+        self.chunk = int(ZARR_CHUNK)
+        self.cells = _csr_cells(n, pseudotime, branches, scalings)
+        self.dtypes = [dt or self.dtype.newbyteorder("<") for _, dt in _ZARR_X]
+        self.rows, self.nnz, self.chunks = 0, 0, [0, 0, 0]
+        self.meta = {}
+        self._dir = self.path + ".partial"
+        self._open = True
+        if os.path.lexists(self._dir):                  # left behind by an interrupted writer
+            shutil.rmtree(self._dir)
+        try:
+            for name, _ in _ZARR_X:
+                os.makedirs(os.path.join(self._dir, "X", name))
+            if n == 0:                                   # no chunk of cells comes: indptr is [0]
+                self.append(0, 0, [zarr_chunks(bytes(8), 8 * self.chunk, self.compress), [], []])
+        except BaseException:
+            self.abort()
+            raise
+
+    def append(self, rows, nnz, parts):
+        """The next `rows` cells with their `nnz` nonzeros, as the complete chunks of indptr, indices and data."""
+        if self.rows + int(rows) > self.shape[0]:
+            raise ValueError("more rows than announced (%d)" % self.shape[0])
+        if len(parts) != 3:
+            raise ValueError("a chunk needs the chunk lists of indptr, indices and data")
+        for j, chunks in enumerate(parts):
+            want = self.chunk * self.dtypes[j].itemsize
+            for piece in chunks:
+                if self.compress:
+                    blocks, adler, raw_len = piece
+                    if int(raw_len) != want:
+                        raise ValueError("a chunk of %d bytes, %d expected" % (raw_len, want))
+                    pieces = [_ZLIB_HEADER, blocks, _FINAL_BLOCK, struct.pack(">I", int(adler) & 0xFFFFFFFF)]
+                else:
+                    if len(memoryview(piece).cast("B")) != want:
+                        raise ValueError("a chunk of %d bytes, %d expected" % (len(memoryview(piece).cast("B")), want))
+                    pieces = [piece]
+                with open(os.path.join(self._dir, "X", _ZARR_X[j][0], str(self.chunks[j])), "wb") as fh:
+                    for p in pieces:
+                        fh.write(p)
+                self.chunks[j] += 1
+        self.rows += int(rows)
+        self.nnz += int(nnz)
+
+    def _group(self, key, attrs):
+        self.meta[key + ".zgroup"] = {"zarr_format": 2}
+        self.meta[key + ".zattrs"] = attrs
+
+    def _array(self, key, length, dtype, attrs=None, strings=False):
+        self.meta[key + "/.zarray"] = {
+            "chunks": [self.chunk], "compressor": _ZARR_COMPRESSOR if self.compress else None,
+            "dtype": "|O" if strings else dtype.str, "fill_value": None if strings else (0.0 if dtype.kind == "f" else 0),
+            "filters": [{"id": "vlen-utf8"}] if strings else None, "order": "C", "shape": [int(length)],
+            "zarr_format": 2}
+        if attrs is not None:
+            self.meta[key + "/.zattrs"] = attrs
+
+    def _host_array(self, key, values, attrs):
+        """A small array the host writes whole: a numeric NumPy array or a list of strings."""
+        strings = isinstance(values, list)
+        dtype = None if strings else values.dtype.newbyteorder("<")
+        self._array(key, len(values), dtype, attrs, strings)
+        os.makedirs(os.path.join(self._dir, key), exist_ok=True)
+        for c, at in enumerate(range(0, len(values), self.chunk)):
+            if strings:
+                raw = _vlen_utf8(values[at:at + self.chunk], self.chunk)
+            else:
+                raw = zarr_chunks(values[at:at + self.chunk].astype(dtype).tobytes(), self.chunk * dtype.itemsize,
+                                  False)[0]
+            with open(os.path.join(self._dir, key, str(c)), "wb") as fh:
+                fh.write(zlib.compress(raw, 1) if self.compress else raw)
+
+    def close(self):
+        """Write obs, var and the metadata and move the store to `path`; raises (and leaves nothing) when rows or
+        chunks are missing."""
+        if not self._open:
+            return
+        try:
+            n, G = self.shape
+            if self.rows != n:
+                raise ValueError("%s: %d of %d rows written" % (self.path, self.rows, n))
+            for j, length in enumerate((n + 1, self.nnz, self.nnz)):
+                if self.chunks[j] != -(-length // self.chunk):
+                    raise ValueError("%s: X/%s has %d chunks, %d values need %d" % (
+                        self.path, _ZARR_X[j][0], self.chunks[j], length, -(-length // self.chunk)))
+            array, string_array = ({"encoding-type": e, "encoding-version": "0.2.0"} for e in ("array", "string-array"))
+            self._group("", {"encoding-type": "anndata", "encoding-version": "0.1.0"})
+            self._group("X/", {"encoding-type": "csr_matrix", "encoding-version": "0.1.0", "shape": [n, G]})
+            for j, length in enumerate((n + 1, self.nnz, self.nnz)):
+                self._array("X/" + _ZARR_X[j][0], length, self.dtypes[j])
+            cells = self.cells
+            self._group("obs/", {"_index": "_index", "column-order": ["pseudotime", "branches", "scalings"],
+                                 "encoding-type": "dataframe", "encoding-version": "0.2.0"})
+            self._host_array("obs/_index", ["cell_%d" % i for i in range(self.first, self.first + n)], string_array)
+            self._host_array("obs/pseudotime", cells["pseudotime"], array)
+            categories, codes = np.unique(np.asarray(cells["branches"]).astype(str), return_inverse=True)
+            self._group("obs/branches/", {"encoding-type": "categorical", "encoding-version": "0.2.0",
+                                          "ordered": False})
+            self._host_array("obs/branches/categories", [str(c) for c in categories], string_array)
+            self._host_array("obs/branches/codes", codes.reshape(-1).astype(_codes_dtype(len(categories))), array)
+            self._host_array("obs/scalings", cells["scalings"], array)
+            self._group("var/", {"_index": "_index", "column-order": [], "encoding-type": "dataframe",
+                                 "encoding-version": "0.2.0"})
+            self._host_array("var/_index", ["gene_%d" % j for j in range(G)], string_array)
+            for name in _ZARR_DICTS:
+                self._group(name + "/", {"encoding-type": "dict", "encoding-version": "0.1.0"})
+            for key, value in self.meta.items():
+                os.makedirs(os.path.dirname(os.path.join(self._dir, key)), exist_ok=True)
+                with open(os.path.join(self._dir, key), "wb") as fh:
+                    fh.write(_zarr_json(value))
+            with open(os.path.join(self._dir, ".zmetadata"), "wb") as fh:
+                fh.write(_zarr_json({"metadata": self.meta, "zarr_consolidated_format": 1}))
+            self._open = False
+            os.rename(self._dir, self.path)
+        except BaseException:
+            self.abort()
+            raise
+
+    def record(self):
+        """The ZarrRecord of the closed store."""
+        nbytes = 0
+        for name, _ in _ZARR_X:
+            folder = os.path.join(self.path, "X", name)
+            nbytes += sum(os.path.getsize(os.path.join(folder, f)) for f in os.listdir(folder) if f[0] != ".")
+        return ZarrRecord(self.path, self.shape, self.nnz, nbytes, self.compress)
+
+    def abort(self):
+        """Drop everything written so far."""
+        self._open = False
         shutil.rmtree(self._dir, ignore_errors=True)
 
     def __enter__(self):

@@ -45,6 +45,13 @@ Extra keyword-only arguments (never required):
            gzips them, so only the pages cross PCIe.  X is then a formats.ParquetRecord (path, shape, nnz, nbytes,
            compressed, load()); the counts are those of out="csr", and dtype (int64 or int32) is the type of the
            count column.  Under shard=, each rank writes a complete directory
+           out="zarr" with path: write an AnnData store in Zarr v2 format at `path` (formats.ZarrWriter): X the
+           cells x genes csr_matrix (indptr int64, indices int32, data of `dtype`, int64 or int32), obs the cells'
+           pseudotime, branches (categorical) and scalings indexed by cell_<global index>, var indexed by gene_<j>,
+           and consolidated metadata, so anndata.read_zarr(path), zarr-python, dask and AnnData's lazy readers open
+           it.  The GPU cuts X into Zarr chunks and, with compress=True, compresses each into one zlib stream, so only
+           the chunks cross PCIe.  X is then a formats.ZarrRecord (path, shape, nnz, nbytes, compressed, load()); the
+           counts are those of out="csr".  Under shard=, each rank writes a complete store of its own cells
   compression  "huffman" (default) or "lz77", where the GPU compresses (compress=True, out="mtx"): "lz77" adds
            LZ77 matches within each 32 KiB DEFLATE block (pst_deflate_lz_blocks), so the same content is written
            in a smaller file; "huffman" writes Huffman-only blocks.  Both files decompress to the same bytes
@@ -71,8 +78,8 @@ from prosstt_b200 import count_model as cm
 from prosstt_b200 import hostpool
 from prosstt_b200 import sim_utils as sut
 from prosstt_b200.device import CountEngine, TreeTables, choice_cdf, raise_flags, tree_tables
-from prosstt_b200.formats import (CsrNpzWriter, CsrShardWriter, MtxWriter, ParquetWriter, TsvWriter, _csr_matrix,
-                                   load_csr_shard)
+from prosstt_b200.formats import (CsrNpzWriter, CsrShardWriter, MtxWriter, ParquetWriter, TsvWriter, ZarrWriter,
+                                   _csr_matrix, load_csr_shard)
 from prosstt_b200.sharding import shard_range
 
 DEFAULT_SAMPLER = "hybrid"
@@ -450,14 +457,15 @@ def _shard_range(n, shard):
 def _check_csr_request(out, dtype, host_out=None, path=None, compress=False, compression="huffman"):
     """out="csr" takes int64 (default) or int32 data and no preallocated host_out; path needs out="csr";
     compress needs both.  out="mtx" needs path, takes int64 or int32 and neither host_out nor compress.
-    out="tsv" and out="parquet" need path, take int64 or int32, compress and no host_out.
+    out="tsv", out="parquet" and out="zarr" need path, take int64 or int32, compress and no host_out.
     compression is "huffman" or "lz77"; "lz77" only where the GPU compresses (compress=True or out="mtx")."""
     if compression not in ("huffman", "lz77"):
         raise ValueError("compression must be 'huffman' or 'lz77', not %r" % (compression,))
-    if out in ("tsv", "parquet"):
+    if out in ("tsv", "parquet", "zarr"):
         if path is None:
-            raise ValueError("out='tsv' writes the reference's _simulation.txt: it needs path=" if out == "tsv" else
-                             "out='parquet' writes a directory of Parquet files: it needs path=")
+            raise ValueError({"tsv": "out='tsv' writes the reference's _simulation.txt: it needs path=",
+                              "parquet": "out='parquet' writes a directory of Parquet files: it needs path=",
+                              "zarr": "out='zarr' writes an AnnData Zarr store: it needs path="}[out])
         if host_out is not None:
             raise ValueError("host_out cannot be combined with out=%r" % out)
         if np.dtype(dtype) not in (np.dtype(np.int64), np.dtype(np.int32)):
@@ -508,8 +516,10 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
     its formats.TsvRecord is returned.
     out="parquet": the chunks go to a Parquet directory at path, gzipped with `compress` (stream_csr(parquet=True)
     into a formats.ParquetWriter, whose cell column counts from the global cell index `first`), and its
-    formats.ParquetRecord is returned.  `compression` picks the device compressor of the compressed forms
-    (stream_csr)."""
+    formats.ParquetRecord is returned.
+    out="zarr": the chunks go to an AnnData Zarr store at path, zlib-compressed with `compress` (stream_csr(zarr=True)
+    into a formats.ZarrWriter, whose obs names count from the global cell index `first`), and its formats.ZarrRecord
+    is returned.  `compression` picks the device compressor of the compressed forms (stream_csr)."""
     if out == "torch":
         X = engine.draw(rows, s32, seed, first)
         engine.check()
@@ -532,6 +542,12 @@ def _sample_counts(engine, rows, s32, seed, first, dtype, out, path=None, cells=
                            compress=compress) as w:
             engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *chunk: w.append(hi - lo, *chunk),
                               data_dtype=dtype, parquet=True, compress=compress, compression=compression)
+        return w.record()
+    if out == "zarr":
+        _check_csr_request(out, dtype, path=path, compress=compress, compression=compression)
+        with ZarrWriter(path, (int(rows.numel()), engine.G), *cells, first=first, dtype=dtype, compress=compress) as w:
+            engine.stream_csr(rows, s32, seed, first, lambda lo, hi, *chunk: w.append(hi - lo, *chunk),
+                              data_dtype=dtype, zarr=True, compress=compress, compression=compression)
         return w.record()
     if out == "csr":
         _check_csr_request(out, dtype)
@@ -618,10 +634,11 @@ def sample_density(tree, no_cells, alpha=0.3, beta=2, scale=True, scale_v=0.7, s
     host_transport ("direct", "i32", "u16", "u8"; with host_out): the format in which the counts cross
     PCIe; the narrow ones are expanded into the int32 / int64 host matrix by `host_threads` host threads
     (0 = all) together with their exact overflow list - the caller receives the same counts either way.
-    out="csr" / "mtx" / "tsv" / "parquet", path, compress, compression: the sparse and on-disk forms of the module
-    docstring; out="mtx", path="counts_10x" writes a 10x directory and returns its formats.MtxRecord; out="tsv",
+    out="csr" / "mtx" / "tsv" / "parquet" / "zarr", path, compress, compression: the sparse and on-disk forms of the
+    module docstring; out="mtx", path="counts_10x" writes a 10x directory and returns its formats.MtxRecord; out="tsv",
     path="job_simulation.txt" writes the reference's counts file and returns its formats.TsvRecord; out="parquet",
-    path="counts_pq" writes counts.parquet and cells.parquet there and returns its formats.ParquetRecord."""
+    path="counts_pq" writes counts.parquet and cells.parquet there and returns its formats.ParquetRecord; out="zarr",
+    path="cells.zarr" writes an AnnData store that anndata.read_zarr opens and returns its formats.ZarrRecord."""
     dev = nat.device(device)
     seed = nat.split_seed(seed)
     tables = tree_tables(tree, dev)
@@ -798,7 +815,8 @@ def draw_counts(tree, pseudotime, branches, scalings, alpha, beta, seed=None, de
     compressed file, and its formats.CompressedCsr record.  out="mtx", path=p writes the 10x directory with
     them (barcodes cell_<first + i>) and returns its formats.MtxRecord.  out="tsv", path=p writes the reference's
     _simulation.txt (rows cell_<first + i>) and returns its formats.TsvRecord.  out="parquet", path=p writes the
-    Parquet directory (cell column first + i) and returns its formats.ParquetRecord.  compression="lz77": see
+    Parquet directory (cell column first + i) and returns its formats.ParquetRecord.  out="zarr", path=p writes the
+    AnnData Zarr store (obs names cell_<first + i>) and returns its formats.ZarrRecord.  compression="lz77": see
     sample_density."""
     dev = nat.device(device)
     _check_csr_request(out, dtype, path=path, compress=compress, compression=compression)
